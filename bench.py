@@ -1,6 +1,6 @@
 """bench.py -- headline benchmark of the B200-native MSDeformAttn engine for Snipper.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -97,9 +97,23 @@ def synthetic_snippets(n, seed):
     return [torch.rand(1, 3 * T, H, W, generator=g) for _ in range(n)]  # frames are /255 floats in [0,1]
 
 
+HEADS = ("pred_logits", "pred_kpts2d", "pred_depth")
+
+
 def pack_result(out):
     """The step's result a caller reads back: final-layer predictions."""
-    return torch.cat([out["pred_logits"].flatten(), out["pred_kpts2d"].flatten(), out["pred_depth"].flatten()])
+    return torch.cat([out[k].flatten() for k in HEADS])
+
+
+def dump_outputs(out_dir, packed, head_shapes):
+    """Write one step's packed predictions back out as DIR/<head>.npy (float32), one file per prediction head."""
+    import numpy as np
+    flat = packed.detach().cpu().float().numpy()
+    sizes = [int(np.prod(s)) for s in head_shapes]
+    assert flat.size == sum(sizes), (flat.size, head_shapes)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, shape, part in zip(HEADS, head_shapes, np.split(flat, np.cumsum(sizes)[:-1])):
+        np.save(os.path.join(out_dir, name + ".npy"), part.reshape(shape))
 
 
 def fused_layer_gathered_bytes(dims, n_frame, e=4):
@@ -387,7 +401,9 @@ def train_run(dev, rank, world, local_rank, steps=8, warmup=3, batch=2):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline loops (resident and end to end) and of the per-kernel event loop; "
+                         "the train and gpu_baseline entries always time 8 steps of their own")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-graph", action="store_true", help="time eager launches instead of CUDA-graph replay")
@@ -398,8 +414,16 @@ def main():
     ap.add_argument("--precision", default="fp32", choices=["fp32", "tf32", "bf16"],
                     help="NOT the headline: 'tf32' lets cuBLAS use TF32 tensor cores for the stock Linear layers, "
                          "'bf16' runs the network under torch.autocast(bfloat16) (bf16 GEMMs, bf16 MSDA gathers). "
-                         "The default and the number the driver records is fp32.")
+                         "The default and the headline number is fp32.")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the predictions of the last timed step as DIR/<head>.npy (float32; "
+                         "rank 0); inputs and weights are seeded, so two builds can be compared output for output. "
+                         "--impl ours only: the CPU reference arm runs other inputs, so its outputs are not comparable")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -448,7 +472,10 @@ def main():
         return pack_result(out).float()
 
     with torch.no_grad(), autocast():
-        result = forward_packed(resident[0])
+        first, _ = model(resident[0])
+        result = pack_result(first).float()
+    head_shapes = [tuple(first[k].shape) for k in HEADS]
+    del first
     d2h_bytes = result.numel() * result.element_size()
     host_out = torch.empty(result.shape, dtype=result.dtype).pin_memory()
     runner, launches_per_step = None, None
@@ -505,6 +532,9 @@ def main():
     eager_launches = ops.STATS.launches
     ms_e2e_total = timed(step_e2e, args.steps, args.warmup)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # host_out holds the last timed step's result; both timed loops feed step warmup + steps - 1 the same input
+        dump_outputs(args.dump_outputs, host_out, head_shapes)
     if launches_per_step is None:
         launches_per_step = eager_launches // (args.steps + args.warmup)
 

@@ -8,7 +8,7 @@ import ref_loader
 from conftest import rel_err
 from oracle import torch_ref
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
+pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="original Snipper source tree not found (set SNIPPER_REFERENCE to it)")
 
 
 @pytest.mark.parametrize("num_future", [0, 2])

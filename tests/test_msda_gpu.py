@@ -291,7 +291,8 @@ def test_matches_vendored_cuda_op(full_case):
     from oracle.build_ref import load_ref
     ref = load_ref()
     if ref is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
+        pytest.skip("the original's CUDA op is not built: build() compiles it into oracle/_ref when SNIPPER_REFERENCE "
+                    "names the original Snipper source tree")
     dev = "cuda:0"
     c = {k: v.to(dev) for k, v in full_case.items()}
     out_ref = ref.ms_deform_attn_forward(c["value"], c["shapes"], c["lsi"], c["loc"], c["attn"], 64)

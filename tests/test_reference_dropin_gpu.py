@@ -20,7 +20,7 @@ import torch
 import ref_loader
 from conftest import rel_err
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")]
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ref_loader.available(), reason="original Snipper source tree not found (set SNIPPER_REFERENCE to it)")]
 DEV = "cuda:0"
 KW = dict(hidden_dim=384, nheads=8, num_feature_levels=3, enc_n_points=4, dec_n_points=4, num_frames=4,
           num_future_frames=2, enc_layers=2, dec_layers=2, num_queries=9, dim_feedforward=256, dropout=0.0)
