@@ -40,7 +40,14 @@ int check_im2col_step(int batch, int im2col_step)
     return (batch % step == 0) ? MSDA_OK : MSDA_ERR_IM2COL_STEP;
 }
 
-bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+// false for NULL: optional pointers pass; required ones are checked for NULL separately
+bool misaligned(const void *p, uintptr_t bytes) { return reinterpret_cast<uintptr_t>(p) % bytes != 0; }
+
+// the planar slot layout exists for float32 heads of 48 channels (msda_planar.cu)
+bool planar_ok(int spatial_size, int num_heads, int channels, int dtype)
+{
+    return dtype == MSDA_DTYPE_F32 && msda::planar_slot_bytes(spatial_size, num_heads, channels, 4) != 0;
+}
 
 }  // namespace
 
@@ -87,7 +94,7 @@ int msda_forward(const void *value, const int64_t *spatial_shapes, const int64_t
     }
     switch (dtype) {
         case MSDA_DTYPE_F32:
-            if (msda::fast_path_ok(d) && aligned16(value) && aligned16(output))
+            if (msda::fast_path_ok(d) && !misaligned(value, 16) && !misaligned(output, 16))
                 return cuda_status(msda::launch_forward_fast_f32(
                     (const float *)value, spatial_shapes, level_start_index, (const float *)sampling_loc,
                     (const float *)attn_weight, (float *)output, d, s));
@@ -100,7 +107,7 @@ int msda_forward(const void *value, const int64_t *spatial_shapes, const int64_t
                 (const double *)attn_weight, (double *)output, d, s));
         case MSDA_DTYPE_BF16:
             // vectorised path only: D % 16 == 0 (16-byte lanes of 8 channels, an even number of lanes)
-            if (!(msda::fast_path_ok(d, 2) && aligned16(value) && aligned16(output))) return MSDA_ERR_UNSUPPORTED_DTYPE;
+            if (!(msda::fast_path_ok(d, 2) && !misaligned(value, 16) && !misaligned(output, 16))) return MSDA_ERR_UNSUPPORTED_DTYPE;
             return cuda_status(msda::launch_forward_fast_bf16(
                 value, spatial_shapes, level_start_index, (const float *)sampling_loc,
                 (const float *)attn_weight, output, d, s));
@@ -163,7 +170,7 @@ int msda_backward(const void *value, const int64_t *spatial_shapes, const int64_
     }
     if (dtype == MSDA_DTYPE_BF16) {
         if (flags & MSDA_FLAG_DETERMINISTIC) return MSDA_ERR_UNSUPPORTED_DTYPE;
-        if (!(msda::fast_path_ok(d, 2) && aligned16(value) && aligned16(grad_output) && aligned16(grad_value)))
+        if (!(msda::fast_path_ok(d, 2) && !misaligned(value, 16) && !misaligned(grad_output, 16) && !misaligned(grad_value, 16)))
             return MSDA_ERR_UNSUPPORTED_DTYPE;
         return cuda_status(msda::launch_backward_fast_bf16(
             value, spatial_shapes, level_start_index, (const float *)sampling_loc,
@@ -172,7 +179,7 @@ int msda_backward(const void *value, const int64_t *spatial_shapes, const int64_
     }
     if (flags & MSDA_FLAG_DETERMINISTIC) {
         const size_t need = msda::deterministic_workspace_bytes(d);
-        if (workspace == nullptr || workspace_bytes < need || (reinterpret_cast<uintptr_t>(workspace) & 255u))
+        if (workspace == nullptr || workspace_bytes < need || misaligned(workspace, 256))
             return MSDA_ERR_WORKSPACE;
         return cuda_status(msda::launch_backward_deterministic_f32(
             (const float *)value, spatial_shapes, level_start_index, (const float *)sampling_loc,
@@ -180,7 +187,7 @@ int msda_backward(const void *value, const int64_t *spatial_shapes, const int64_
             (float *)grad_sampling_loc, (float *)grad_attn_weight, d, workspace, s,
             (flags & MSDA_FLAG_ACCUMULATE_VALUE) != 0));
     }
-    if (msda::fast_path_ok(d) && aligned16(value) && aligned16(grad_output) && aligned16(grad_value))
+    if (msda::fast_path_ok(d) && !misaligned(value, 16) && !misaligned(grad_output, 16) && !misaligned(grad_value, 16))
         return cuda_status(msda::launch_backward_fast_f32(
             (const float *)value, spatial_shapes, level_start_index, (const float *)sampling_loc,
             (const float *)attn_weight, (const float *)grad_output, (float *)grad_value,
@@ -204,12 +211,19 @@ static msda::OpDims snippet_det_dims(int batch, int n_query_frames, int n_frame,
     return od;
 }
 
+// the deterministic workspace starts with the sampling locations (2 floats per sample) and attention weights (1),
+// each block 256-byte aligned; the two-pass state of msda_backward follows
+static size_t det_sample_bytes(const msda::OpDims &od, int floats)
+{
+    return align256(sizeof(float) * floats * (size_t)od.N * od.Lq * od.M * od.L * od.P);
+}
+
 static int check_mask(const unsigned char *mask, int64_t row_stride, int col_stride)
 {
     if (mask == nullptr) return MSDA_OK;
     if (row_stride < 0 || (col_stride != 0 && col_stride != 1)) return MSDA_ERR_INVALID_ARGUMENT;
     // per-channel masks are read as 32-bit words
-    if (col_stride == 1 && ((reinterpret_cast<uintptr_t>(mask) & 3u) || (row_stride & 3))) return MSDA_ERR_INVALID_ARGUMENT;
+    if (col_stride == 1 && (misaligned(mask, 4) || (row_stride & 3))) return MSDA_ERR_INVALID_ARGUMENT;
     return MSDA_OK;
 }
 
@@ -253,13 +267,41 @@ static int snippet_dims(msda::SnippetDims &d, int batch, int n_src_frames, int n
     return MSDA_OK;
 }
 
+// flag combinations of the snippet entries: planar slots and the deterministic mode both ride on the pre-summed
+// path, and they exclude each other (the deterministic mode walks cell-major float32 slots)
+static int snippet_flags_ok(unsigned flags, unsigned allowed, int dtype, int spatial_size, int num_heads, int channels)
+{
+    const bool presummed = (flags & MSDA_FLAG_PRESUMMED) != 0, deterministic = (flags & MSDA_FLAG_DETERMINISTIC) != 0,
+               planar = (flags & MSDA_FLAG_PLANAR) != 0;
+    if ((flags & ~allowed) || ((planar || deterministic) && !presummed) || (planar && deterministic))
+        return MSDA_ERR_INVALID_ARGUMENT;
+    if ((planar && !planar_ok(spatial_size, num_heads, channels, dtype)) || (deterministic && dtype != MSDA_DTYPE_F32))
+        return MSDA_ERR_UNSUPPORTED_DTYPE;
+    return MSDA_OK;
+}
+
+// the pointers a snippet launch dereferences, checked when there is work to do: none NULL, each aligned for its widest
+// access.  `out`: the forward's output or the backward's grad_output; `grads`: the backward's three outputs or NULL.
+static bool snippet_pointers_ok(const msda::SnippetDims &d, const void *value, const int64_t *spatial_shapes,
+                                const int64_t *level_start_index, const void *offsets, const void *logits,
+                                const void *reference_points, const void *out, bool planar, void *const *grads)
+{
+    const uintptr_t slot_align = planar ? 128 : 16;
+    if (grads && (!grads[0] || !grads[1] || !grads[2] || misaligned(grads[0], slot_align) || misaligned(grads[1], 8) ||
+                  misaligned(grads[2], 4)))
+        return false;
+    return value && spatial_shapes && level_start_index && offsets && logits && (reference_points || d.valid_ratios) &&
+           out && !misaligned(value, slot_align) && !misaligned(out, 16) && !misaligned(offsets, 8) &&
+           !misaligned(logits, 4) && !misaligned(d.off_bias, 8);
+}
+
 int msda_masked_zero(void *data, const unsigned char *mask, int64_t n_elements, int dtype, void *stream)
 {
     if (n_elements < 0) return MSDA_ERR_INVALID_ARGUMENT;
     if (n_elements == 0) return MSDA_OK;
     if (!data || !mask) return MSDA_ERR_INVALID_ARGUMENT;
     if (dtype != MSDA_DTYPE_F32 && dtype != MSDA_DTYPE_BF16) return MSDA_ERR_UNSUPPORTED_DTYPE;
-    if (!aligned16(mask)) return MSDA_ERR_INVALID_ARGUMENT;
+    if (misaligned(mask, 16)) return MSDA_ERR_INVALID_ARGUMENT;
     return cuda_status(msda::launch_masked_zero(data, mask, n_elements, dtype == MSDA_DTYPE_BF16 ? 2 : 4,
                                                 static_cast<cudaStream_t>(stream)));
 }
@@ -277,39 +319,53 @@ int msda_snippet_forward(const void *value, const int64_t *spatial_shapes,
                          const unsigned char *value_mask, int64_t mask_row_stride, int mask_col_stride,
                          int dtype, unsigned flags, void *stream)
 {
-    if (flags & ~(MSDA_FLAG_PRESUMMED | MSDA_FLAG_PLANAR)) return MSDA_ERR_INVALID_ARGUMENT;
+    int st = snippet_flags_ok(flags, MSDA_FLAG_PRESUMMED | MSDA_FLAG_PLANAR, dtype, spatial_size, num_heads, channels);
+    if (st != MSDA_OK) return st;
     const bool planar = (flags & MSDA_FLAG_PLANAR) != 0;
-    if (planar && !(flags & MSDA_FLAG_PRESUMMED)) return MSDA_ERR_INVALID_ARGUMENT;
-    if (planar && (dtype != MSDA_DTYPE_F32 || msda::planar_slot_bytes(spatial_size, num_heads, channels, 4) == 0))
-        return MSDA_ERR_UNSUPPORTED_DTYPE;
     msda::SnippetDims d;
-    int st = snippet_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, num_heads,
-                          channels, num_levels, num_query, num_point, value_stride_n,
-                          value_stride_t, ref_stride_n, ref_stride_t, offsets_row_stride, logits_row_stride,
-                          offsets_bias, logits_bias, encoder_valid_ratios, value_mask, mask_row_stride, mask_col_stride,
-                          dtype, flags);
+    st = snippet_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, num_heads,
+                      channels, num_levels, num_query, num_point, value_stride_n,
+                      value_stride_t, ref_stride_n, ref_stride_t, offsets_row_stride, logits_row_stride,
+                      offsets_bias, logits_bias, encoder_valid_ratios, value_mask, mask_row_stride, mask_col_stride,
+                      dtype, flags);
     if (st != MSDA_OK) return st;
     if (batch == 0 || num_query == 0) return MSDA_OK;
-    if (!value || !spatial_shapes || !level_start_index || !offsets || !logits ||
-        (!reference_points && !encoder_valid_ratios) || !output)
+    if (!snippet_pointers_ok(d, value, spatial_shapes, level_start_index, offsets, logits, reference_points, output, planar,
+                             nullptr))
         return MSDA_ERR_INVALID_ARGUMENT;
-    if (!aligned16(value) || !aligned16(output) || (reinterpret_cast<uintptr_t>(offsets) & 7u) ||
-        (reinterpret_cast<uintptr_t>(logits) & 3u) || (reinterpret_cast<uintptr_t>(offsets_bias) & 7u))
-        return MSDA_ERR_INVALID_ARGUMENT;
-    if (planar) {
-        if (reinterpret_cast<uintptr_t>(value) & 127u) return MSDA_ERR_INVALID_ARGUMENT;
-        return cuda_status(msda::launch_planar_forward_f32(
-            value, spatial_shapes, level_start_index, (const float *)offsets, (const float *)logits,
-            (const float *)reference_points, (float *)output, d, static_cast<cudaStream_t>(stream)));
-    }
+    const float *off = (const float *)offsets, *lg = (const float *)logits, *ref = (const float *)reference_points;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (planar)
+        return cuda_status(msda::launch_planar_forward_f32(value, spatial_shapes, level_start_index, off, lg, ref,
+                                                           (float *)output, d, s));
     if (dtype == MSDA_DTYPE_BF16)
-        return cuda_status(msda::launch_snippet_forward_bf16(
-            value, spatial_shapes, level_start_index, (const float *)offsets, (const float *)logits,
-            (const float *)reference_points, output, d, static_cast<cudaStream_t>(stream)));
-    return cuda_status(msda::launch_snippet_forward_f32(
-        (const float *)value, spatial_shapes, level_start_index, (const float *)offsets,
-        (const float *)logits, (const float *)reference_points, (float *)output, d,
-        static_cast<cudaStream_t>(stream)));
+        return cuda_status(msda::launch_snippet_forward_bf16(value, spatial_shapes, level_start_index, off, lg, ref,
+                                                             output, d, s));
+    return cuda_status(msda::launch_snippet_forward_f32((const float *)value, spatial_shapes, level_start_index, off,
+                                                        lg, ref, (float *)output, d, s));
+}
+
+// bit-reproducible backward (MSDA_FLAG_DETERMINISTIC, pre-summed float32 slots, validated): the fused kernel with
+// its scatter compiled out for grad_offsets / grad_logits, then msda_backward's two-pass grad_value over the slots
+static int snippet_backward_deterministic(const msda::SnippetDims &d, const float *value, const int64_t *spatial_shapes,
+                                          const int64_t *level_start_index, const float *offsets, const float *logits,
+                                          const float *reference_points, const float *grad_output, float *grad_value,
+                                          float *grad_offsets, float *grad_logits, bool accumulate, void *workspace,
+                                          cudaStream_t s)
+{
+    const msda::OpDims od = snippet_det_dims(d.N, d.T1, d.n_frame, d.S, d.M, d.D, d.L, d.Lq, d.P);
+    unsigned char *ws = static_cast<unsigned char *>(workspace);
+    float *loc = reinterpret_cast<float *>(ws), *attn = reinterpret_cast<float *>(ws + det_sample_bytes(od, 2));
+    int st = cuda_status(msda::launch_snippet_backward_noscatter_f32(
+        value, spatial_shapes, level_start_index, offsets, logits, reference_points, grad_output, grad_offsets,
+        grad_logits, d, s));
+    if (st != MSDA_OK) return st;
+    st = cuda_status(msda::launch_snippet_loc_attn(spatial_shapes, level_start_index, offsets, logits, reference_points,
+                                                   loc, attn, d, s));
+    if (st != MSDA_OK) return st;
+    // grad_value: count / scan / fill / ordered reduce; every slot cell is written exactly once
+    return cuda_status(msda::launch_deterministic_grad_value_f32(spatial_shapes, level_start_index, loc, attn, grad_output,
+        grad_value, od, ws + det_sample_bytes(od, 2) + det_sample_bytes(od, 1), s, accumulate));
 }
 
 int msda_snippet_backward(const void *value, const int64_t *spatial_shapes,
@@ -326,97 +382,62 @@ int msda_snippet_backward(const void *value, const int64_t *spatial_shapes,
                           const unsigned char *value_mask, int64_t mask_row_stride, int mask_col_stride,
                           int dtype, unsigned flags, void *workspace, size_t workspace_bytes, void *stream)
 {
-    if (flags & ~(MSDA_FLAG_PRESUMMED | MSDA_FLAG_ACCUMULATE_VALUE | MSDA_FLAG_DETERMINISTIC | MSDA_FLAG_PLANAR))
-        return MSDA_ERR_INVALID_ARGUMENT;
-    const bool deterministic = (flags & MSDA_FLAG_DETERMINISTIC) != 0;
-    const bool planar = (flags & MSDA_FLAG_PLANAR) != 0;
-    if (planar && (deterministic || !(flags & MSDA_FLAG_PRESUMMED))) return MSDA_ERR_INVALID_ARGUMENT;
-    if (planar && (dtype != MSDA_DTYPE_F32 || msda::planar_slot_bytes(spatial_size, num_heads, channels, 4) == 0))
-        return MSDA_ERR_UNSUPPORTED_DTYPE;
-    // deterministic mode: two-pass grad_value over the pre-summed slots, float32
-    if (deterministic && !(flags & MSDA_FLAG_PRESUMMED)) return MSDA_ERR_INVALID_ARGUMENT;
-    if (deterministic && dtype != MSDA_DTYPE_F32) return MSDA_ERR_UNSUPPORTED_DTYPE;
-    msda::SnippetDims d;
-    int st = snippet_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, num_heads,
-                          channels, num_levels, num_query, num_point, value_stride_n,
-                          value_stride_t, ref_stride_n, ref_stride_t, offsets_row_stride, logits_row_stride,
-                          offsets_bias, logits_bias, encoder_valid_ratios, value_mask, mask_row_stride, mask_col_stride,
-                          dtype, flags);
+    int st = snippet_flags_ok(flags, MSDA_FLAG_PRESUMMED | MSDA_FLAG_ACCUMULATE_VALUE | MSDA_FLAG_DETERMINISTIC |
+                              MSDA_FLAG_PLANAR, dtype, spatial_size, num_heads, channels);
     if (st != MSDA_OK) return st;
-    if (!reference_points && encoder_valid_ratios) reference_points = encoder_valid_ratios;  // never dereferenced; passes the null checks
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    msda::SnippetDims d;
+    st = snippet_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, num_heads,
+                      channels, num_levels, num_query, num_point, value_stride_n,
+                      value_stride_t, ref_stride_n, ref_stride_t, offsets_row_stride, logits_row_stride,
+                      offsets_bias, logits_bias, encoder_valid_ratios, value_mask, mask_row_stride, mask_col_stride,
+                      dtype, flags);
+    if (st != MSDA_OK) return st;
+    const bool planar = (flags & MSDA_FLAG_PLANAR) != 0, accumulate = (flags & MSDA_FLAG_ACCUMULATE_VALUE) != 0,
+               deterministic = (flags & MSDA_FLAG_DETERMINISTIC) != 0, work = batch > 0 && num_query > 0;
     const int gframes = (flags & MSDA_FLAG_PRESUMMED) ? msda::snippet_num_slots(n_query_frames, n_frame) : n_src_frames;
-    const size_t value_elems = planar ? (size_t)batch * gframes * (msda::planar_slot_bytes(spatial_size, num_heads, channels, 4) / 4)
-                                      : (size_t)batch * gframes * spatial_size * num_heads * channels;
     if (deterministic) {
-        // 32-bit corner / cell ids (checked before anything is enqueued)
-        const int64_t samples = (int64_t)batch * n_query_frames * num_query * num_heads * num_levels * num_point;
-        if (samples * 4 >= (int64_t)INT32_MAX || (int64_t)batch * gframes * spatial_size * num_heads >= (int64_t)INT32_MAX)
+        // 32-bit corner / cell ids
+        if ((int64_t)batch * n_query_frames * num_query * num_heads * num_levels * num_point * 4 >= (int64_t)INT32_MAX ||
+            (int64_t)batch * gframes * spatial_size * num_heads >= (int64_t)INT32_MAX)
             return MSDA_ERR_TOO_LARGE;
-        const msda::OpDims od = snippet_det_dims(batch, n_query_frames, n_frame, spatial_size, num_heads, channels,
-                                                 num_levels, num_query, num_point);
-        const size_t loc_bytes = align256(sizeof(float) * 2 * (size_t)samples), attn_bytes = align256(sizeof(float) * (size_t)samples);
-        const size_t need = loc_bytes + attn_bytes + msda::deterministic_workspace_bytes(od);
-        if (batch > 0 && num_query > 0 &&
-            (workspace == nullptr || workspace_bytes < need || (reinterpret_cast<uintptr_t>(workspace) & 255u)))
+        const size_t need = msda_snippet_backward_workspace_bytes(batch, n_query_frames, n_frame, spatial_size, num_heads,
+                                                                  channels, num_levels, num_query, num_point, dtype, flags);
+        if (work && (workspace == nullptr || workspace_bytes < need || misaligned(workspace, 256)))
             return MSDA_ERR_WORKSPACE;
-        if (batch == 0) return MSDA_OK;
-        if (!grad_value || !aligned16(grad_value)) return MSDA_ERR_INVALID_ARGUMENT;
-        if (num_query == 0) {
-            if (flags & MSDA_FLAG_ACCUMULATE_VALUE) return MSDA_OK;
-            return cuda_status(cudaMemsetAsync(grad_value, 0, sizeof(float) * value_elems, s));
-        }
-        if (!value || !spatial_shapes || !level_start_index || !offsets || !logits || !reference_points ||
-            !grad_output || !grad_offsets || !grad_logits)
-            return MSDA_ERR_INVALID_ARGUMENT;
-        if (!aligned16(value) || !aligned16(grad_output) || (reinterpret_cast<uintptr_t>(offsets) & 7u) ||
-            (reinterpret_cast<uintptr_t>(grad_offsets) & 7u) || (reinterpret_cast<uintptr_t>(offsets_bias) & 7u))
-            return MSDA_ERR_INVALID_ARGUMENT;
-        unsigned char *ws = static_cast<unsigned char *>(workspace);
-        float *loc = reinterpret_cast<float *>(ws), *attn = reinterpret_cast<float *>(ws + loc_bytes);
-        // everything but grad_value: the fused backward kernel with its scatter compiled out
-        st = cuda_status(msda::launch_snippet_backward_noscatter_f32(
-            (const float *)value, spatial_shapes, level_start_index, (const float *)offsets, (const float *)logits,
-            (const float *)reference_points, (const float *)grad_output, (float *)grad_offsets, (float *)grad_logits, d, s));
-        if (st != MSDA_OK) return st;
-        st = cuda_status(msda::launch_snippet_loc_attn(spatial_shapes, level_start_index, (const float *)offsets,
-                                                       (const float *)logits, (const float *)reference_points, loc, attn, d, s));
-        if (st != MSDA_OK) return st;
-        // grad_value: count / scan / fill / ordered reduce; every slot cell is written exactly once
-        return cuda_status(msda::launch_deterministic_grad_value_f32(
-            spatial_shapes, level_start_index, loc, attn, (const float *)grad_output, (float *)grad_value, od,
-            ws + loc_bytes + attn_bytes, s, (flags & MSDA_FLAG_ACCUMULATE_VALUE) != 0));
     }
-    if (!(flags & MSDA_FLAG_ACCUMULATE_VALUE) && value_elems > 0) {
-        if (!grad_value) return MSDA_ERR_INVALID_ARGUMENT;
-        st = cuda_status(cudaMemsetAsync(grad_value, 0, sizeof(float) * value_elems, s));
-        if (st != MSDA_OK) return st;
-    }
-    if (batch == 0 || num_query == 0) return MSDA_OK;
-    if (!value || !spatial_shapes || !level_start_index || !offsets || !logits || !reference_points ||
-        !grad_output || !grad_value || !grad_offsets || !grad_logits)
+    if (batch == 0) return MSDA_OK;
+    // grad_value is zero-filled unless accumulated into or written in full by the deterministic ordered reduce
+    const bool zero_fill = !accumulate && !(deterministic && work);
+    if (((zero_fill || deterministic) && !grad_value) || (deterministic && misaligned(grad_value, 16)))
         return MSDA_ERR_INVALID_ARGUMENT;
-    if (!aligned16(value) || !aligned16(grad_output) || !aligned16(grad_value) ||
-        (reinterpret_cast<uintptr_t>(offsets) & 7u) || (reinterpret_cast<uintptr_t>(grad_offsets) & 7u) ||
-        (reinterpret_cast<uintptr_t>(offsets_bias) & 7u))
+    void *const grads[] = {grad_value, grad_offsets, grad_logits};
+    if (work && !snippet_pointers_ok(d, value, spatial_shapes, level_start_index, offsets, logits, reference_points,
+                                     grad_output, planar, grads))
         return MSDA_ERR_INVALID_ARGUMENT;
-    if (planar) {
-        if ((reinterpret_cast<uintptr_t>(value) & 127u) || (reinterpret_cast<uintptr_t>(grad_value) & 127u))
-            return MSDA_ERR_INVALID_ARGUMENT;
-        return cuda_status(msda::launch_planar_backward_f32(
-            value, spatial_shapes, level_start_index, (const float *)offsets, (const float *)logits,
-            (const float *)reference_points, (const float *)grad_output, grad_value, (float *)grad_offsets,
-            (float *)grad_logits, d, s));
+    // everything is validated: from here on work is enqueued
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (zero_fill) {
+        const size_t slot_elems = planar ? msda::planar_slot_bytes(spatial_size, num_heads, channels, 4) / 4
+                                         : (size_t)spatial_size * num_heads * channels;
+        st = cuda_status(cudaMemsetAsync(grad_value, 0, sizeof(float) * batch * gframes * slot_elems, s));
+        if (st != MSDA_OK) return st;
     }
+    if (!work) return MSDA_OK;
+    const float *off = (const float *)offsets, *lg = (const float *)logits, *ref = (const float *)reference_points;
+    float *goff = (float *)grad_offsets, *glg = (float *)grad_logits;
+    if (deterministic)
+        return snippet_backward_deterministic(d, (const float *)value, spatial_shapes, level_start_index, off, lg, ref,
+                                              (const float *)grad_output, (float *)grad_value, goff, glg, accumulate,
+                                              workspace, s);
+    if (planar)
+        return cuda_status(msda::launch_planar_backward_f32(value, spatial_shapes, level_start_index, off, lg, ref,
+                                                            (const float *)grad_output, grad_value, goff, glg, d, s));
     if (dtype == MSDA_DTYPE_BF16)
-        return cuda_status(msda::launch_snippet_backward_bf16(
-            value, spatial_shapes, level_start_index, (const float *)offsets, (const float *)logits,
-            (const float *)reference_points, grad_output, (float *)grad_value, (float *)grad_offsets,
-            (float *)grad_logits, d, s));
-    return cuda_status(msda::launch_snippet_backward_f32(
-        (const float *)value, spatial_shapes, level_start_index, (const float *)offsets,
-        (const float *)logits, (const float *)reference_points, (const float *)grad_output,
-        (float *)grad_value, (float *)grad_offsets, (float *)grad_logits, d, s));
+        return cuda_status(msda::launch_snippet_backward_bf16(value, spatial_shapes, level_start_index, off, lg, ref,
+                                                              grad_output, (float *)grad_value, goff, glg, d, s));
+    return cuda_status(msda::launch_snippet_backward_f32((const float *)value, spatial_shapes, level_start_index, off,
+                                                         lg, ref, (const float *)grad_output, (float *)grad_value, goff,
+                                                         glg, d, s));
 }
 
 size_t msda_snippet_backward_workspace_bytes(int batch, int n_query_frames, int n_frame, int spatial_size,
@@ -425,10 +446,9 @@ size_t msda_snippet_backward_workspace_bytes(int batch, int n_query_frames, int 
 {
     if (!(flags & MSDA_FLAG_DETERMINISTIC) || dtype != MSDA_DTYPE_F32) return 0;
     if (batch <= 0 || n_query_frames <= 0 || n_frame <= 0 || num_query <= 0) return 0;
-    const size_t samples = (size_t)batch * n_query_frames * num_query * num_heads * num_levels * num_point;
     const msda::OpDims od = snippet_det_dims(batch, n_query_frames, n_frame, spatial_size, num_heads, channels,
                                              num_levels, num_query, num_point);
-    return align256(sizeof(float) * 2 * samples) + align256(sizeof(float) * samples) + msda::deterministic_workspace_bytes(od);
+    return det_sample_bytes(od, 2) + det_sample_bytes(od, 1) + msda::deterministic_workspace_bytes(od);
 }
 
 int msda_snippet_num_slots(int n_query_frames, int n_frame)
@@ -461,7 +481,7 @@ int msda_snippet_prefers_presum(int n_src_frames, int n_query_frames, int n_fram
 
 static int frame_dims(msda::FrameDims &d, int batch, int n_src_frames, int n_query_frames, int n_frame,
                       int spatial_size, int row_elems, int64_t value_stride_n, int64_t value_stride_t,
-                      const unsigned char *mask, int64_t mask_row_stride, int mask_col_stride, int dtype)
+                      const unsigned char *mask, int64_t mask_row_stride, int mask_col_stride, int dtype, int esize)
 {
     if (dtype != MSDA_DTYPE_F32 && dtype != MSDA_DTYPE_BF16) return MSDA_ERR_UNSUPPORTED_DTYPE;
     if (batch < 0 || n_src_frames <= 0 || n_query_frames <= 0 || n_frame <= 0 || n_frame > n_src_frames ||
@@ -474,7 +494,7 @@ static int frame_dims(msda::FrameDims &d, int batch, int n_src_frames, int n_que
     if (value_stride_n < 0 || value_stride_t < 0) return MSDA_ERR_INVALID_ARGUMENT;
     d = msda::FrameDims{batch, n_src_frames, n_query_frames, n_frame, spatial_size, row_elems, value_stride_n,
                         value_stride_t, mask ? mask_row_stride : 0, mask ? mask_col_stride : 0};
-    return MSDA_OK;
+    return msda::frame_dims_ok(d, esize) ? MSDA_OK : MSDA_ERR_INVALID_ARGUMENT;
 }
 
 int msda_frame_sum(const void *value, const unsigned char *value_mask, void *vsum,
@@ -483,13 +503,12 @@ int msda_frame_sum(const void *value, const unsigned char *value_mask, void *vsu
                    int64_t mask_row_stride, int mask_col_stride, int dtype, void *stream)
 {
     msda::FrameDims d;
-    int st = frame_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, row_elems, value_stride_n,
-                        value_stride_t, value_mask, mask_row_stride, mask_col_stride, dtype);
-    if (st != MSDA_OK) return st;
     const int esize = dtype == MSDA_DTYPE_BF16 ? 2 : 4;
-    if (!msda::frame_dims_ok(d, esize)) return MSDA_ERR_INVALID_ARGUMENT;
+    int st = frame_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, row_elems, value_stride_n,
+                        value_stride_t, value_mask, mask_row_stride, mask_col_stride, dtype, esize);
+    if (st != MSDA_OK) return st;
     if (batch == 0) return MSDA_OK;
-    if (!value || !vsum || !aligned16(value) || !aligned16(vsum)) return MSDA_ERR_INVALID_ARGUMENT;
+    if (!value || !vsum || misaligned(value, 16) || misaligned(vsum, 16)) return MSDA_ERR_INVALID_ARGUMENT;
     return cuda_status(msda::launch_frame_sum(value, value_mask, vsum, d, esize, static_cast<cudaStream_t>(stream)));
 }
 
@@ -500,13 +519,12 @@ int msda_frame_unsum(const void *grad_vsum, const unsigned char *value_mask, voi
 {
     msda::FrameDims d;
     int st = frame_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, row_elems, 0, 0,
-                        value_mask, mask_row_stride, mask_col_stride, dtype);
+                        value_mask, mask_row_stride, mask_col_stride, dtype, 4);   // one thread per 4 fp32 channels
     if (st != MSDA_OK) return st;
-    if (!msda::frame_dims_ok(d, 4)) return MSDA_ERR_INVALID_ARGUMENT;   // one thread per 4 fp32 channels
     if (batch == 0) return MSDA_OK;
-    if (!grad_vsum || !grad_value || !aligned16(grad_vsum) || (reinterpret_cast<uintptr_t>(grad_value) & 7u))
+    // each thread stores 4 channels: 16 bytes of float32, 8 of bfloat16
+    if (!grad_vsum || !grad_value || misaligned(grad_vsum, 16) || misaligned(grad_value, dtype == MSDA_DTYPE_F32 ? 16 : 8))
         return MSDA_ERR_INVALID_ARGUMENT;
-    if (dtype == MSDA_DTYPE_F32 && !aligned16(grad_value)) return MSDA_ERR_INVALID_ARGUMENT;
     return cuda_status(msda::launch_frame_unsum(static_cast<const float *>(grad_vsum), value_mask, grad_value, d,
                                                 dtype == MSDA_DTYPE_BF16 ? 2 : 4, static_cast<cudaStream_t>(stream)));
 }
@@ -522,16 +540,13 @@ int msda_frame_sum_planar(const void *value, const unsigned char *value_mask, vo
                           int spatial_size, int num_heads, int channels, int64_t value_stride_n, int64_t value_stride_t,
                           int64_t mask_row_stride, int mask_col_stride, int dtype, void *stream)
 {
-    if (dtype != MSDA_DTYPE_F32 || num_heads <= 0 || channels <= 0 ||
-        msda::planar_slot_bytes(spatial_size, num_heads, channels, 4) == 0)
-        return MSDA_ERR_UNSUPPORTED_DTYPE;
+    if (!planar_ok(spatial_size, num_heads, channels, dtype)) return MSDA_ERR_UNSUPPORTED_DTYPE;
     msda::FrameDims d;
     int st = frame_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, num_heads * channels,
-                        value_stride_n, value_stride_t, value_mask, mask_row_stride, mask_col_stride, dtype);
+                        value_stride_n, value_stride_t, value_mask, mask_row_stride, mask_col_stride, dtype, 4);
     if (st != MSDA_OK) return st;
-    if (!msda::frame_dims_ok(d, 4)) return MSDA_ERR_INVALID_ARGUMENT;
     if (batch == 0) return MSDA_OK;
-    if (!value || !vsum_planar || !aligned16(value) || (reinterpret_cast<uintptr_t>(vsum_planar) & 127u))
+    if (!value || !vsum_planar || misaligned(value, 16) || misaligned(vsum_planar, 128))
         return MSDA_ERR_INVALID_ARGUMENT;
     return cuda_status(msda::launch_frame_sum_planar(static_cast<const float *>(value), value_mask, vsum_planar, d,
                                                      num_heads, static_cast<cudaStream_t>(stream)));
@@ -542,16 +557,13 @@ int msda_frame_unsum_planar(const void *grad_vsum_planar, const unsigned char *v
                             int spatial_size, int num_heads, int channels, int64_t mask_row_stride, int mask_col_stride,
                             int dtype, void *stream)
 {
-    if (dtype != MSDA_DTYPE_F32 || num_heads <= 0 || channels <= 0 ||
-        msda::planar_slot_bytes(spatial_size, num_heads, channels, 4) == 0)
-        return MSDA_ERR_UNSUPPORTED_DTYPE;
+    if (!planar_ok(spatial_size, num_heads, channels, dtype)) return MSDA_ERR_UNSUPPORTED_DTYPE;
     msda::FrameDims d;
     int st = frame_dims(d, batch, n_src_frames, n_query_frames, n_frame, spatial_size, num_heads * channels, 0, 0,
-                        value_mask, mask_row_stride, mask_col_stride, dtype);
+                        value_mask, mask_row_stride, mask_col_stride, dtype, 4);
     if (st != MSDA_OK) return st;
-    if (!msda::frame_dims_ok(d, 4)) return MSDA_ERR_INVALID_ARGUMENT;
     if (batch == 0) return MSDA_OK;
-    if (!grad_vsum_planar || !grad_value || (reinterpret_cast<uintptr_t>(grad_vsum_planar) & 127u) || !aligned16(grad_value))
+    if (!grad_vsum_planar || !grad_value || misaligned(grad_vsum_planar, 128) || misaligned(grad_value, 16))
         return MSDA_ERR_INVALID_ARGUMENT;
     return cuda_status(msda::launch_frame_unsum_planar(grad_vsum_planar, value_mask, static_cast<float *>(grad_value), d,
                                                        num_heads, static_cast<cudaStream_t>(stream)));
@@ -567,8 +579,8 @@ int msda_layer_tail(const void *y, const void *bias, const void *residual, const
     if (rows == 0) return MSDA_OK;
     const void *ptrs[] = {y, residual, gamma, beta, out};
     for (const void *p : ptrs)
-        if (p == nullptr || !aligned16(p)) return MSDA_ERR_INVALID_ARGUMENT;
-    if (!aligned16(bias) || !aligned16(pos) || !aligned16(out_plus_pos)) return MSDA_ERR_INVALID_ARGUMENT;
+        if (p == nullptr || misaligned(p, 16)) return MSDA_ERR_INVALID_ARGUMENT;
+    if (misaligned(bias, 16) || misaligned(pos, 16) || misaligned(out_plus_pos, 16)) return MSDA_ERR_INVALID_ARGUMENT;
     return cuda_status(msda::launch_layer_tail((const float *)y, (const float *)bias, (const float *)residual,
                                                (const float *)gamma, (const float *)beta, (const float *)pos,
                                                (float *)out, (float *)out_plus_pos, rows, cols, eps,

@@ -11,7 +11,7 @@ What differs is the execution:
 
 * fused path (default): offsets and logits are computed ONCE for all query frames, by ONE GEMM
   over the stacked weights (the reference recomputes the same two GEMMs for every (t1,t2) pair
-  -- 20 GEMMs per layer at T=4, only 2 distinct), then ONE kernel launch per layer (``snipper_b200::snippet_forward``) does the
+  -- 20 GEMMs per layer at T=4, only 2 distinct), then ONE kernel launch per layer (``snipper_b200::snippet_attn``) does the
   offset normalisation, the softmax over levels x points x neighbour frames and the gather from
   all neighbour frames.  No ``.contiguous()`` copies, no stack+sum, no host sync (the
   reference's shape assert at :112 synchronises the stream every call).

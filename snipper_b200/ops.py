@@ -5,11 +5,15 @@ in the hand-written kernels.  Ops (namespace ``snipper_b200``):
 
   msda_forward / msda_backward          per-call op, the reference's extension functions
                                         (models/ops/src/vision.cpp:13-16)
-  snippet_forward / snippet_backward    fused per-layer Snipper attention
+  snippet_forward / snippet_backward    fused per-layer Snipper attention on separate offsets / logits
                                         (models/ops/modules/ms_deform_attn.py:126-225)
+  snippet_attn / snippet_attn_backward  the same layer on the packed [offsets | logits] projection, with in-kernel
+                                        biases, padding mask and encoder reference points; what the module runs
+  masked_zero_                          in-place masked zero-fill of value (ms_deform_attn.py:116-117)
+  layer_tail                            bias + residual + LayerNorm (+ pos) after a block, inference only
 
-Both forwards carry ``register_autograd`` formulas, so they compose with autograd / DDP as plain
-nodes (no host sync, no unused parameters).
+The three forwards (msda_forward, snippet_forward, snippet_attn) carry ``register_autograd`` formulas, so they
+compose with autograd / DDP as plain nodes (no host sync, no unused parameters).
 """
 from typing import Optional, Tuple
 
@@ -47,10 +51,6 @@ def is_deterministic() -> bool:
     return _deterministic
 
 
-def _stream(device) -> int:
-    return torch.cuda.current_stream(device).cuda_stream
-
-
 class LaunchStats:
     """Counts kernel launches issued through the C ABI and, when ``timing`` is on, brackets each
     launch with CUDA events on the launching stream (bench.py's roofline measurement)."""
@@ -75,25 +75,26 @@ class LaunchStats:
 STATS = LaunchStats()
 
 
-class _Launch:
-    """with _Launch(tag, dims, device, n_kernels): <C call>"""
-
-    def __init__(self, tag, dims, device, n_kernels=1):
-        self.tag, self.dims, self.device, self.n = tag, dims, device, n_kernels
-
-    def __enter__(self):
+def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None, im2col_step=None):
+    """Call the C entry point ``entry`` with ``args`` and ``device``'s current stream (every launching entry point takes
+    the stream last), count its ``n_kernels`` kernels in STATS under ``tag`` / ``dims`` and raise on a failed status."""
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device)
         if STATS.timing:
-            self.s = torch.cuda.Event(enable_timing=True)
-            self.e = torch.cuda.Event(enable_timing=True)
-            self.s.record(torch.cuda.current_stream(self.device))
-        return self
-
-    def __exit__(self, *exc):
-        STATS.launches += self.n
+            start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            start.record(stream)
+        status = getattr(capi.lib(), entry)(*args, stream.cuda_stream)
+        STATS.launches += n_kernels
         if STATS.timing:
-            self.e.record(torch.cuda.current_stream(self.device))
-            STATS.events.append((self.tag, self.dims, self.s, self.e))
-        return False
+            end.record(stream)
+            STATS.events.append((tag, dims, start, end))
+    capi.check(status, what or entry, batch, im2col_step)
+
+
+def _workspace(nbytes, device):
+    """-> (tensor to keep alive, 256-byte aligned pointer to ``nbytes`` bytes of it)"""
+    ws = torch.empty(nbytes + 256, dtype=torch.uint8, device=device)
+    return ws, (ws.data_ptr() + 255) // 256 * 256
 
 
 def _require_cuda(t: Tensor, name: str) -> None:
@@ -155,12 +156,11 @@ def msda_forward(value: Tensor, spatial_shapes: Tensor, level_start_index: Tenso
     N, S, M, D, L, Lq, P = _check_percall(value, spatial_shapes, level_start_index, sampling_loc, attn_weight)
     vbs = _value_batch_stride(value)
     out = torch.empty((N, Lq, M * D), dtype=value.dtype, device=value.device)
-    with torch.cuda.device(value.device), _Launch("msda_forward", (N, S, M, D, L, Lq, P), value.device):
-        st = capi.lib().msda_forward(
+    _launch("msda_forward", "msda_forward", (N, S, M, D, L, Lq, P), value.device,
             value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
             sampling_loc.data_ptr(), attn_weight.data_ptr(), out.data_ptr(),
-            N, S, M, D, L, Lq, P, vbs, int(im2col_step), _DTYPES[value.dtype], _stream(value.device))
-    capi.check(st, "ms_deform_attn_forward", N, im2col_step)
+            N, S, M, D, L, Lq, P, vbs, int(im2col_step), _DTYPES[value.dtype],
+            what="ms_deform_attn_forward", batch=N, im2col_step=im2col_step)
     return out
 
 
@@ -189,22 +189,18 @@ def msda_backward(value: Tensor, spatial_shapes: Tensor, level_start_index: Tens
     grad_attn = torch.empty_like(attn_weight)
     flags = capi.MSDA_FLAG_DETERMINISTIC if deterministic else 0
     dt = _DTYPES[value.dtype]
-    ws, ws_bytes = None, 0
-    with torch.cuda.device(value.device):
-        if deterministic:
-            ws_bytes = capi.lib().msda_backward_workspace_bytes(N, S, M, D, L, Lq, P, dt, flags)
-            ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=value.device)
-        ws_ptr = 0 if ws is None else (ws.data_ptr() + 255) // 256 * 256
-        # deterministic: no-scatter kernel, memset, count, 3 scan kernels, fill, reduce, long-list reduce
-        with _Launch("msda_backward_deterministic" if deterministic else "msda_backward", (N, S, M, D, L, Lq, P),
-                     value.device, 9 if deterministic else 2):
-            st = capi.lib().msda_backward(
-                value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-                sampling_loc.data_ptr(), attn_weight.data_ptr(), grad_output.data_ptr(),
-                grad_value.data_ptr(), grad_loc.data_ptr(), grad_attn.data_ptr(),
-                N, S, M, D, L, Lq, P, vbs, int(im2col_step), dt, flags, ws_ptr, ws_bytes,
-                _stream(value.device))
-    capi.check(st, "ms_deform_attn_backward", N, im2col_step)
+    ws, ws_ptr, ws_bytes = None, 0, 0
+    if deterministic:
+        ws_bytes = capi.lib().msda_backward_workspace_bytes(N, S, M, D, L, Lq, P, dt, flags)
+        ws, ws_ptr = _workspace(ws_bytes, value.device)
+    # deterministic: no-scatter kernel, memset, count, 3 scan kernels, fill, reduce, long-list reduce
+    _launch("msda_backward", "msda_backward_deterministic" if deterministic else "msda_backward",
+            (N, S, M, D, L, Lq, P), value.device,
+            value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
+            sampling_loc.data_ptr(), attn_weight.data_ptr(), grad_output.data_ptr(),
+            grad_value.data_ptr(), grad_loc.data_ptr(), grad_attn.data_ptr(),
+            N, S, M, D, L, Lq, P, vbs, int(im2col_step), dt, flags, ws_ptr, ws_bytes,
+            n_kernels=9 if deterministic else 2, what="ms_deform_attn_backward", batch=N, im2col_step=im2col_step)
     if bf16:
         grad_value = grad_value.to(torch.bfloat16)
     return grad_value, grad_loc, grad_attn
@@ -244,10 +240,8 @@ def masked_zero_(data: Tensor, mask: Tensor) -> None:
         raise RuntimeError("masked_zero_: data and mask must be contiguous tensors of one shape")
     if mask.dtype != torch.bool or data.dtype not in (torch.float32, torch.bfloat16):
         raise RuntimeError("masked_zero_: data must be float32 / bfloat16 and mask bool")
-    with torch.cuda.device(data.device), _Launch("masked_zero", (data.numel(),), data.device):
-        st = capi.lib().msda_masked_zero(data.data_ptr(), mask.data_ptr(), data.numel(), _DTYPES[data.dtype],
-                                         _stream(data.device))
-    capi.check(st, "msda_masked_zero")
+    _launch("msda_masked_zero", "masked_zero", (data.numel(),), data.device,
+            data.data_ptr(), mask.data_ptr(), data.numel(), _DTYPES[data.dtype])
 
 
 def masked_zero_supported(data: Tensor, mask: Tensor) -> bool:
@@ -272,29 +266,68 @@ def snippet_supported(n_heads: int, d_head: int, n_levels: int, n_points: int, d
             batch_frames <= 65535)                                           # gridDim.z
 
 
-def _check_snippet(value, spatial_shapes, level_start_index, offsets, logits, ref, n_frame):
-    for t, name in ((value, "value"), (spatial_shapes, "spatial_shapes"), (level_start_index, "level_start_index"),
-                    (offsets, "offsets"), (logits, "logits"), (ref, "reference_points")):
-        _require_cuda(t, name)
-    if value.dim() != 5 or offsets.dim() != 7 or logits.dim() != 6 or ref.dim() != 5:
-        raise RuntimeError("expected value (N,T2,S,M,D), offsets (N,T1,Lq,M,L,P,2), logits (N,T1,Lq,M,L,P), "
-                           "reference_points (N,T1,Lq,L,2)")
-    N, T2, S, M, D = value.shape
-    No, T1, Lq, Mo, L, P, two = offsets.shape
-    if (No, Mo, two) != (N, M, 2) or tuple(logits.shape) != (N, T1, Lq, M, L, P):
-        raise RuntimeError("offsets / logits shapes do not match value")
-    if tuple(ref.shape) != (N, T1, Lq, L, 2) or tuple(spatial_shapes.shape) != (L, 2):
-        raise RuntimeError("reference_points must be (N,T1,Lq,L,2) and spatial_shapes (L,2)")
-    if not snippet_supported(M, D, L, P, value.dtype):
+def _check_fused(value, spatial_shapes, level_start_index, reference_points, n_frame, *, offsets=None, logits=None,
+                 proj=None, biases=(None, None), valid_ratios=None, presummed=False, T2=None, planar_dims=None):
+    """Validate one fused call -> (N, T2, T1, S, M, D, L, Lq, P).
+
+    The queries' sampling offsets and logits come as separate ``offsets`` (N,T1,Lq,M,L,P,2) and ``logits``
+    (N,T1,Lq,M,L,P), or as the packed projection ``proj`` (N,T1,Lq,3*M*L*P) with optional ``biases``.  ``value`` is
+    (N,T2,S,M,D), or the (N,slots,S,M,D) pre-summed slots when ``presummed`` (``T2`` then gives the source frames);
+    ``planar_dims`` = (S, M, D) marks it as a planar carry (N, slots, planar_slot_elems) -- see snippet_attn."""
+    ref = reference_points
+    rows = (("proj", proj),) if proj is not None else (("offsets", offsets), ("logits", logits))
+    for name, t in (("value", value), ("spatial_shapes", spatial_shapes), ("level_start_index", level_start_index),
+                    *rows, ("reference_points", ref)):
+        if t is not None:
+            _require_cuda(t, name)
+    if planar_dims is not None:
+        if (value.dim() != 3 or value.dtype != torch.float32 or not value.is_contiguous() or
+                value.shape[2] != planar_slot_elems(*planar_dims, value.dtype) or value.data_ptr() % 128 != 0):
+            raise RuntimeError("planar carry must be a contiguous float32 (N, slots, planar_slot_elems) tensor, 128-byte aligned")
+        vshape = (value.shape[0], value.shape[1], *planar_dims)
+    else:
+        vshape = tuple(value.shape)
+    if len(vshape) != 5 or (ref is not None and ref.dim() != 5):
+        raise RuntimeError("expected value (N,T2,S,M,D) and reference_points (N,T1,Lq,L,2)")
+    if (ref is None) == (valid_ratios is None):
+        raise RuntimeError("pass either reference_points or (encoder self-attention) valid_ratios")
+    N, F, S, M, D = vshape
+    if proj is not None:
+        L = spatial_shapes.shape[0]
+        if proj.dim() != 4 or proj.shape[0] != N or proj.shape[3] % (3 * M * L) != 0:
+            raise RuntimeError("proj must be (N,T1,Lq,3*M*L*P): [offsets (M,L,P,2) | logits (M,L,P)] per query")
+        _, T1, Lq, W = proj.shape
+        P = W // (3 * M * L)
+    else:
+        if offsets.dim() != 7 or logits.dim() != 6:
+            raise RuntimeError("expected offsets (N,T1,Lq,M,L,P,2) and logits (N,T1,Lq,M,L,P)")
+        No, T1, Lq, Mo, L, P, two = offsets.shape
+        if (No, Mo, two) != (N, M, 2) or tuple(logits.shape) != (N, T1, Lq, M, L, P):
+            raise RuntimeError("offsets / logits shapes do not match value")
+    if tuple(spatial_shapes.shape) != (L, 2) or level_start_index.numel() != L:
+        raise RuntimeError("spatial_shapes must be (L,2) and level_start_index (L,)")
+    if ref is not None and (tuple(ref.shape) != (N, T1, Lq, L, 2) or ref.dtype != torch.float32):
+        raise RuntimeError("reference_points must be float32 (N,T1,Lq,L,2)")
+    if valid_ratios is not None:
+        if (not valid_ratios.is_cuda or valid_ratios.dtype != torch.float32 or tuple(valid_ratios.shape) != (N, L, 2)
+                or not valid_ratios.is_contiguous() or Lq != S):
+            raise RuntimeError("valid_ratios must be contiguous float32 (N,L,2) and the queries the S pixels of the pyramid")
+    if not snippet_supported(M, D, L, P, value.dtype, S, N * T1):
         raise RuntimeError("fused snippet attention needs float32 / bfloat16 value, D % 16 == 0, D <= 128, L*P <= 32")
-    if any(t.dtype != torch.float32 for t in (offsets, logits, ref)):
-        raise RuntimeError("offsets, logits and reference_points must be float32")
+    if any(t.dtype != torch.float32 for _, t in rows):
+        raise RuntimeError("offsets and logits (or proj) must be float32")
+    for b, n in zip(biases, (2 * M * L * P, M * L * P)):
+        if b is not None and (not b.is_cuda or b.dtype != torch.float32 or b.numel() != n or not b.is_contiguous()):
+            raise RuntimeError("biases must be contiguous float32 CUDA tensors of 2*M*L*P / M*L*P elements")
+    if presummed:
+        if F != num_slots(T1, n_frame) or not value.is_contiguous():
+            raise RuntimeError("presummed value must be a contiguous (N, slots, S, M, D) tensor (or a planar carry)")
+    else:
+        T2 = F
     if not (0 < n_frame <= T2):
         raise RuntimeError("n_frame must be in (0, T2]")
-    _require_contiguous(offsets, "offsets")
-    _require_contiguous(logits, "logits")
-    _require_contiguous(spatial_shapes, "spatial_shapes")
-    _require_contiguous(level_start_index, "level_start_index")
+    for name, t in (*rows, ("spatial_shapes", spatial_shapes), ("level_start_index", level_start_index)):
+        _require_contiguous(t, name)
     return N, T2, T1, S, M, D, L, Lq, P
 
 
@@ -315,22 +348,61 @@ def _ref_strides(ref):
     return ref, (ref.stride(0) if N > 1 else 0), (ref.stride(1) if T1 > 1 else 0)
 
 
+def _ptr(t):
+    return None if t is None else t.data_ptr()
+
+
+# The two builders below are the only callers of the fused entry points: they put the named pieces of a call into the
+# ABI's positional order (include/msda_b200.h).  ``value_strides`` are (batch, frame) element strides of value or the
+# slots, 0 = dense; ``offsets`` / ``logits`` are (pointer, row stride in floats), 0 = dense rows; either
+# ``reference_points`` or the encoder's ``valid_ratios`` is given; ``mask`` is (tensor or None, row stride, col stride)
+# as mask_layout returns it.
+def _issue_snippet_forward(tag, dims, n_frame, value, spatial_shapes, level_start_index, out, *, offsets, logits,
+                           value_strides=(0, 0), reference_points=None, valid_ratios=None, biases=(None, None),
+                           mask=(None, 0, 0), flags=0):
+    N, T2, T1, S, M, D, L, Lq, P = dims
+    ref, rsn, rst = _ref_strides(reference_points) if reference_points is not None else (None, 0, 0)
+    _launch("msda_snippet_forward", tag, dims, value.device,
+            value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(), offsets[0], logits[0], _ptr(ref),
+            out.data_ptr(), N, T2, T1, int(n_frame), S, M, D, L, Lq, P, *value_strides, rsn, rst, offsets[1], logits[1],
+            _ptr(biases[0]), _ptr(biases[1]), _ptr(valid_ratios), _ptr(mask[0]), mask[1], mask[2],
+            _DTYPES[value.dtype], flags)
+
+
+def _issue_snippet_backward(tag, n_kernels, dims, n_frame, value, spatial_shapes, level_start_index, grad_output,
+                            grad_value, *, offsets, logits, grad_offsets, grad_logits, value_strides=(0, 0),
+                            reference_points=None, valid_ratios=None, biases=(None, None), mask=(None, 0, 0), flags=0,
+                            workspace=(None, 0)):
+    """``grad_offsets`` / ``grad_logits`` are pointers with the row strides of ``offsets`` / ``logits``; ``workspace``
+    is (pointer, bytes)."""
+    N, T2, T1, S, M, D, L, Lq, P = dims
+    ref, rsn, rst = _ref_strides(reference_points) if reference_points is not None else (None, 0, 0)
+    _launch("msda_snippet_backward", tag, dims, value.device,
+            value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(), offsets[0], logits[0], _ptr(ref),
+            grad_output.data_ptr(), grad_value.data_ptr(), grad_offsets, grad_logits,
+            N, T2, T1, int(n_frame), S, M, D, L, Lq, P, *value_strides, rsn, rst, offsets[1], logits[1],
+            _ptr(biases[0]), _ptr(biases[1]), _ptr(valid_ratios), _ptr(mask[0]), mask[1], mask[2],
+            _DTYPES[value.dtype], flags, *workspace, n_kernels=n_kernels)
+
+
+def _grad_ref(grad_offsets, spatial_shapes):
+    """grad_offsets (N,T1,Lq,M,L,P,2) -> the gradient of reference_points (N,T1,Lq,L,2):
+    loc = ref + off/(W,H)  =>  dL/dref = sum_{m,p} dL/dloc = sum_{m,p} dL/doff * (W,H)"""
+    wh = torch.stack([spatial_shapes[:, 1], spatial_shapes[:, 0]], -1).to(grad_offsets.dtype)
+    return (grad_offsets * wh[None, None, None, None, :, None, :]).sum(dim=(3, 5))
+
+
 @torch.library.custom_op("snipper_b200::snippet_forward", mutates_args=())
 def snippet_forward(value: Tensor, spatial_shapes: Tensor, level_start_index: Tensor,
                     offsets: Tensor, logits: Tensor, reference_points: Tensor, n_frame: int) -> Tensor:
     """Fused layer attention on separate offsets / logits tensors, neighbour frames gathered directly."""
-    N, T2, T1, S, M, D, L, Lq, P = _check_snippet(value, spatial_shapes, level_start_index, offsets,
-                                                  logits, reference_points, n_frame)
-    sn, st = _value_strides5(value)
-    ref, rsn, rst = _ref_strides(reference_points)
+    dims = _check_fused(value, spatial_shapes, level_start_index, reference_points, n_frame, offsets=offsets,
+                        logits=logits)
+    N, T2, T1, S, M, D, L, Lq, P = dims
     out = torch.empty((N, T1, Lq, M * D), dtype=value.dtype, device=value.device)
-    with torch.cuda.device(value.device), _Launch("snippet_forward", (N, T2, T1, S, M, D, L, Lq, P), value.device):
-        status = capi.lib().msda_snippet_forward(
-            value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-            offsets.data_ptr(), logits.data_ptr(), ref.data_ptr(), out.data_ptr(),
-            N, T2, T1, int(n_frame), S, M, D, L, Lq, P, sn, st, rsn, rst, 0, 0, None, None, None, None, 0, 0,
-            _DTYPES[value.dtype], 0, _stream(value.device))
-    capi.check(status, "msda_snippet_forward")
+    _issue_snippet_forward("snippet_forward", dims, n_frame, value, spatial_shapes, level_start_index, out,
+                           offsets=(offsets.data_ptr(), 0), logits=(logits.data_ptr(), 0),
+                           value_strides=_value_strides5(value), reference_points=reference_points)
     return out
 
 
@@ -344,23 +416,18 @@ def _(value, spatial_shapes, level_start_index, offsets, logits, reference_point
 def snippet_backward(value: Tensor, spatial_shapes: Tensor, level_start_index: Tensor,
                      offsets: Tensor, logits: Tensor, reference_points: Tensor, grad_output: Tensor,
                      n_frame: int) -> Tuple[Tensor, Tensor, Tensor]:
-    N, T2, T1, S, M, D, L, Lq, P = _check_snippet(value, spatial_shapes, level_start_index, offsets,
-                                                  logits, reference_points, n_frame)
+    dims = _check_fused(value, spatial_shapes, level_start_index, reference_points, n_frame, offsets=offsets,
+                        logits=logits)
+    N, T2, T1, S, M, D, L, Lq, P = dims
     _require_cuda(grad_output, "grad_output")
     _require_contiguous(grad_output, "grad_output")
-    sn, st = _value_strides5(value)
-    ref, rsn, rst = _ref_strides(reference_points)
     grad_value = torch.empty((N, T2, S, M, D), dtype=torch.float32, device=value.device)  # fp32 accumulation
     grad_offsets = torch.empty_like(offsets)
     grad_logits = torch.empty_like(logits)
-    with torch.cuda.device(value.device), _Launch("snippet_backward", (N, T2, T1, S, M, D, L, Lq, P), value.device):
-        status = capi.lib().msda_snippet_backward(
-            value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-            offsets.data_ptr(), logits.data_ptr(), ref.data_ptr(), grad_output.data_ptr(),
-            grad_value.data_ptr(), grad_offsets.data_ptr(), grad_logits.data_ptr(),
-            N, T2, T1, int(n_frame), S, M, D, L, Lq, P, sn, st, rsn, rst, 0, 0, None, None, None, None, 0, 0,
-            _DTYPES[value.dtype], 0, None, 0, _stream(value.device))
-    capi.check(status, "msda_snippet_backward")
+    _issue_snippet_backward("snippet_backward", 2, dims, n_frame, value, spatial_shapes, level_start_index, grad_output,
+                            grad_value, offsets=(offsets.data_ptr(), 0), logits=(logits.data_ptr(), 0),
+                            grad_offsets=grad_offsets.data_ptr(), grad_logits=grad_logits.data_ptr(),
+                            value_strides=_value_strides5(value), reference_points=reference_points)
     if value.dtype != torch.float32:
         grad_value = grad_value.to(value.dtype)
     return grad_value, grad_offsets, grad_logits
@@ -381,11 +448,7 @@ def _snippet_backward_formula(ctx, grad_output):
     value, spatial_shapes, level_start_index, offsets, logits, ref = ctx.saved_tensors
     gv, goff, glog = torch.ops.snipper_b200.snippet_backward(
         value, spatial_shapes, level_start_index, offsets, logits, ref, grad_output.contiguous(), ctx.n_frame)
-    gref = None
-    if ctx.needs_input_grad[5]:
-        # loc = ref + off/(W,H)  =>  dL/dref = sum_{m,p} dL/dloc = sum_{m,p} dL/doff * (W,H)
-        wh = torch.stack([spatial_shapes[:, 1], spatial_shapes[:, 0]], -1).to(goff.dtype)
-        gref = (goff * wh[None, None, None, None, :, None, :]).sum(dim=(3, 5))
+    gref = _grad_ref(goff, spatial_shapes) if ctx.needs_input_grad[5] else None
     return gv, None, None, goff, glog, gref, None
 
 
@@ -437,91 +500,34 @@ def planar_slot_elems(S: int, M: int, D: int, dtype) -> int:
     return capi.lib().msda_planar_slot_bytes(S, M, D, capi.MSDA_DTYPE_F32) // 4
 
 
-def _check_packed(value, spatial_shapes, level_start_index, proj, offsets_bias, logits_bias, ref, n_frame,
-                  presummed=False, T2=None, valid_ratios=None, planar_dims=None):
-    """``planar_dims`` = (S, M, D): ``value`` is then a planar carry (N, slots, planar_slot_elems) -- see snippet_attn."""
-    if planar_dims is not None:
-        S_, M_, D_ = planar_dims
-        if (value.dim() != 3 or value.dtype != torch.float32 or not value.is_contiguous() or
-                value.shape[2] != planar_slot_elems(S_, M_, D_, value.dtype) or value.data_ptr() % 128 != 0):
-            raise RuntimeError("planar carry must be a contiguous float32 (N, slots, planar_slot_elems) tensor, 128-byte aligned")
-        vshape = (value.shape[0], value.shape[1], S_, M_, D_)
-    else:
-        vshape = tuple(value.shape)
-    return _check_packed_impl(value, vshape, spatial_shapes, level_start_index, proj, offsets_bias, logits_bias, ref,
-                              n_frame, presummed, T2, valid_ratios, planar_dims is not None)
-
-
-def _check_packed_impl(value, vshape, spatial_shapes, level_start_index, proj, offsets_bias, logits_bias, ref, n_frame,
-                       presummed, T2, valid_ratios, planar):
-    for t, name in ((value, "value"), (spatial_shapes, "spatial_shapes"), (level_start_index, "level_start_index"),
-                    (proj, "proj")) + (((ref, "reference_points"),) if ref is not None else ()):
-        _require_cuda(t, name)
-    if len(vshape) != 5 or proj.dim() != 4 or (ref is not None and ref.dim() != 5):
-        raise RuntimeError("expected value (N,T2,S,M,D), proj (N,T1,Lq,3*M*L*P), reference_points (N,T1,Lq,L,2)")
-    if (ref is None) == (valid_ratios is None):
-        raise RuntimeError("pass either reference_points or (encoder self-attention) valid_ratios")
-    N, F, S, M, D = vshape
-    L = spatial_shapes.shape[0]
-    Np, T1, Lq, W = proj.shape
-    if Np != N or W % (3 * M * L) != 0:
-        raise RuntimeError("proj must be (N,T1,Lq,3*M*L*P): [offsets (M,L,P,2) | logits (M,L,P)] per query")
-    P = W // (3 * M * L)
-    if tuple(spatial_shapes.shape) != (L, 2) or level_start_index.numel() != L:
-        raise RuntimeError("spatial_shapes must be (L,2) and level_start_index (L,)")
-    if ref is not None and (tuple(ref.shape) != (N, T1, Lq, L, 2) or ref.dtype != torch.float32):
-        raise RuntimeError("reference_points must be float32 (N,T1,Lq,L,2)")
-    if valid_ratios is not None:
-        if (not valid_ratios.is_cuda or valid_ratios.dtype != torch.float32 or tuple(valid_ratios.shape) != (N, L, 2)
-                or not valid_ratios.is_contiguous() or Lq != S):
-            raise RuntimeError("valid_ratios must be contiguous float32 (N,L,2) and the queries the S pixels of the pyramid")
-    if not snippet_supported(M, D, L, P, value.dtype, S, N * T1):
-        raise RuntimeError("fused snippet attention needs float32 / bfloat16 value, D % 16 == 0, D <= 128, L*P <= 32")
-    if proj.dtype != torch.float32:
-        raise RuntimeError("proj must be float32")
-    for b, n in ((offsets_bias, 2 * M * L * P), (logits_bias, M * L * P)):
-        if b is not None and (not b.is_cuda or b.dtype != torch.float32 or b.numel() != n or not b.is_contiguous()):
-            raise RuntimeError("biases must be contiguous float32 CUDA tensors of 2*M*L*P / M*L*P elements")
-    if presummed:
-        if F != num_slots(T1, n_frame) or not value.is_contiguous():
-            raise RuntimeError("presummed value must be a contiguous (N, slots, S, M, D) tensor (or a planar carry)")
-    else:
-        T2 = F
-    if not (0 < n_frame <= T2):
-        raise RuntimeError("n_frame must be in (0, T2]")
-    _require_contiguous(proj, "proj")
-    _require_contiguous(spatial_shapes, "spatial_shapes")
-    _require_contiguous(level_start_index, "level_start_index")
-    return N, T2, T1, S, M, D, L, Lq, P
-
-
-def _ptr(t):
-    return None if t is None else t.data_ptr()
-
-
-def _frame_sum(value, mask, mrs, mcs, T1, n_frame):
-    """(N,T2,S,M,D) -> (N,slots,S,M,D): masked neighbour-frame sums, one slot per query frame."""
+def _frame_sum(value, mask, T1, n_frame, planar):
+    """(N,T2,S,M,D) -> masked neighbour-frame sums, one slot per query frame: (N,slots,S,M,D) in value's dtype, or the
+    same sums in the planar fp32 layout (N, slots, planar_slot_elems) laid out for the gather."""
     N, T2, S, M, D = value.shape
     sn, st = _value_strides5(value)
-    vsum = torch.empty((N, num_slots(T1, n_frame), S, M, D), dtype=value.dtype, device=value.device)
-    with torch.cuda.device(value.device), _Launch("frame_sum", (N, T2, T1, S, M * D), value.device):
-        status = capi.lib().msda_frame_sum(value.data_ptr(), _ptr(mask), vsum.data_ptr(), N, T2, T1, int(n_frame), S,
-                                           M * D, sn, st, mrs, mcs, _DTYPES[value.dtype], _stream(value.device))
-    capi.check(status, "msda_frame_sum")
+    slots = num_slots(T1, n_frame)
+    if planar:
+        vsum = torch.empty((N, slots, planar_slot_elems(S, M, D, value.dtype)), dtype=torch.float32, device=value.device)
+        entry, tag, row = "msda_frame_sum_planar", "frame_sum_planar", (S, M, D)
+    else:
+        vsum = torch.empty((N, slots, S, M, D), dtype=value.dtype, device=value.device)
+        entry, tag, row = "msda_frame_sum", "frame_sum", (S, M * D)
+    _launch(entry, tag, (N, T2, T1, S, M * D), value.device, value.data_ptr(), _ptr(mask[0]), vsum.data_ptr(),
+            N, T2, T1, int(n_frame), *row, sn, st, mask[1], mask[2], _DTYPES[value.dtype])
     return vsum
 
 
-def _frame_sum_planar(value, mask, mrs, mcs, T1, n_frame):
-    """(N,T2,S,M,D) -> planar slots (N, slots, planar_slot_elems): the same sums, laid out for the gather."""
-    N, T2, S, M, D = value.shape
-    sn, st = _value_strides5(value)
-    vsum = torch.empty((N, num_slots(T1, n_frame), planar_slot_elems(S, M, D, value.dtype)), dtype=torch.float32,
-                       device=value.device)
-    with torch.cuda.device(value.device), _Launch("frame_sum_planar", (N, T2, T1, S, M * D), value.device):
-        status = capi.lib().msda_frame_sum_planar(value.data_ptr(), _ptr(mask), vsum.data_ptr(), N, T2, T1, int(n_frame),
-                                                  S, M, D, sn, st, mrs, mcs, _DTYPES[value.dtype], _stream(value.device))
-    capi.check(status, "msda_frame_sum_planar")
-    return vsum
+def _frame_unsum(grad_slots, mask, dims, n_frame, dtype, planar):
+    """The adjoint of _frame_sum: fp32 slot gradients -> grad_value (N,T2,S,M,D) in ``dtype``, masked alike."""
+    N, T2, T1, S, M, D = dims[:6]
+    grad_value = torch.empty((N, T2, S, M, D), dtype=dtype, device=grad_slots.device)
+    if planar:
+        entry, tag, row = "msda_frame_unsum_planar", "frame_unsum_planar", (S, M, D)
+    else:
+        entry, tag, row = "msda_frame_unsum", "frame_unsum", (S, M * D)
+    _launch(entry, tag, (N, T2, T1, S, M * D), grad_slots.device, grad_slots.data_ptr(), _ptr(mask[0]),
+            grad_value.data_ptr(), N, T2, T1, int(n_frame), *row, mask[1], mask[2], _DTYPES[dtype])
+    return grad_value
 
 
 def use_planar(S: int, M: int, D: int, dtype) -> bool:
@@ -532,12 +538,9 @@ def use_planar(S: int, M: int, D: int, dtype) -> bool:
     return planar_slot_elems(S, M, D, dtype) > 0 and not (_deterministic and torch.is_grad_enabled())
 
 
-def _ref_args(reference_points, valid_ratios):
-    """-> (tensor to keep alive, ref pointer, batch stride, frame stride, valid-ratio pointer)"""
-    if reference_points is None:
-        return None, None, 0, 0, valid_ratios.data_ptr()
-    ref, rsn, rst = _ref_strides(reference_points)
-    return ref, ref.data_ptr(), rsn, rst, None
+def _proj_columns(proj, mlp):
+    """[offsets (M,L,P,2) | logits (M,L,P)] column blocks of a packed projection row -> two (pointer, row stride)"""
+    return (proj.data_ptr(), 3 * mlp), (proj.data_ptr() + 4 * 2 * mlp, 3 * mlp)
 
 
 @torch.library.custom_op("snipper_b200::snippet_attn", mutates_args=())
@@ -554,34 +557,26 @@ def snippet_attn(value: Tensor, value_mask: Optional[Tensor], spatial_shapes: Te
     Returns (out (N,T1,Lq,M*D), carry): carry is the presummed value when ``presum`` -- the only form of value the
     backward needs: (N,slots,S,M,D), or the library's planar slots (N,slots,planar_slot_elems) when ``planar`` (only
     with ``presum``; ``use_planar`` says where the layout applies) -- and an empty tensor otherwise."""
-    N, T2, T1, S, M, D, L, Lq, P = _check_packed(value, spatial_shapes, level_start_index, proj, offsets_bias,
-                                                 logits_bias, reference_points, n_frame, valid_ratios=valid_ratios)
-    mask, mrs, mcs = mask_layout(value_mask, N, T2, S, M * D)
-    ref, ref_ptr, rsn, rst, vr_ptr = _ref_args(reference_points, valid_ratios)
-    mlp = M * L * P
+    dims = _check_fused(value, spatial_shapes, level_start_index, reference_points, n_frame, proj=proj,
+                        biases=(offsets_bias, logits_bias), valid_ratios=valid_ratios)
+    N, T2, T1, S, M, D, L, Lq, P = dims
+    mask = mask_layout(value_mask, N, T2, S, M * D)
     out = torch.empty((N, T1, Lq, M * D), dtype=value.dtype, device=value.device)
-    dims = (N, T2, T1, S, M, D, L, Lq, P)
     if planar and not (presum and planar_slot_elems(S, M, D, value.dtype) > 0):
         raise RuntimeError("planar slots need presum=True, float32 value and 48 channels per head")
-    if planar:
-        carry = _frame_sum_planar(value, mask, mrs, mcs, T1, n_frame)
-        src, sn, st, kmask, tag = carry, 0, 0, None, "snippet_forward_planar"
-        flags = capi.MSDA_FLAG_PRESUMMED | capi.MSDA_FLAG_PLANAR
-    elif presum:
-        carry = _frame_sum(value, mask, mrs, mcs, T1, n_frame)
-        src, sn, st, kmask, flags, tag = carry, 0, 0, None, capi.MSDA_FLAG_PRESUMMED, "snippet_forward_presummed"
+    if presum:
+        # the mask was applied by the frame sums; the kernel gets its strides without the pointer
+        carry = _frame_sum(value, mask, T1, n_frame, planar)
+        src, strides, kmask = carry, (0, 0), (None,) + mask[1:]
+        flags = capi.MSDA_FLAG_PRESUMMED | (capi.MSDA_FLAG_PLANAR if planar else 0)
+        tag = "snippet_forward_planar" if planar else "snippet_forward_presummed"
     else:
         carry = value.new_empty((0,))
-        sn, st = _value_strides5(value)
-        src, kmask, flags, tag = value, mask, 0, "snippet_forward"
-    with torch.cuda.device(value.device), _Launch(tag, dims, value.device):
-        status = capi.lib().msda_snippet_forward(
-            src.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-            proj.data_ptr(), proj.data_ptr() + 4 * 2 * mlp, ref_ptr, out.data_ptr(),
-            N, T2, T1, int(n_frame), S, M, D, L, Lq, P, sn, st, rsn, rst, 3 * mlp, 3 * mlp,
-            _ptr(offsets_bias), _ptr(logits_bias), vr_ptr, _ptr(kmask), mrs, mcs,
-            _DTYPES[value.dtype], flags, _stream(value.device))
-    capi.check(status, "msda_snippet_forward")
+        src, strides, kmask, flags, tag = value, _value_strides5(value), mask, 0, "snippet_forward"
+    offsets, logits = _proj_columns(proj, M * L * P)
+    _issue_snippet_forward(tag, dims, n_frame, src, spatial_shapes, level_start_index, out, offsets=offsets,
+                           logits=logits, value_strides=strides, reference_points=reference_points,
+                           valid_ratios=valid_ratios, biases=(offsets_bias, logits_bias), mask=kmask, flags=flags)
     return out, carry
 
 
@@ -610,80 +605,48 @@ def snippet_attn_backward(value_or_vsum: Tensor, value_mask: Optional[Tensor], s
     planar = value_dims is not None
     if planar and not presum:
         raise RuntimeError("planar slots exist on the pre-summed path only")
-    N, T2, T1, S, M, D, L, Lq, P = _check_packed(value_or_vsum, spatial_shapes, level_start_index, proj,
-                                                 offsets_bias, logits_bias, reference_points, n_frame,
-                                                 presummed=presum, T2=n_src_frames, valid_ratios=valid_ratios,
-                                                 planar_dims=tuple(value_dims) if planar else None)
+    dims = _check_fused(value_or_vsum, spatial_shapes, level_start_index, reference_points, n_frame, proj=proj,
+                        biases=(offsets_bias, logits_bias), valid_ratios=valid_ratios, presummed=presum,
+                        T2=n_src_frames, planar_dims=tuple(value_dims) if planar else None)
+    N, T2, T1, S, M, D, L, Lq, P = dims
     _require_cuda(grad_output, "grad_output")
     _require_contiguous(grad_output, "grad_output")
     if grad_output.dtype != value_or_vsum.dtype or grad_output.numel() != N * T1 * Lq * M * D:
         raise RuntimeError("grad_output must be (N,T1,Lq,M*D) in value's dtype")
     dev, dt = value_or_vsum.device, value_or_vsum.dtype
-    mask, mrs, mcs = mask_layout(value_mask, N, T2, S, M * D)
-    ref, ref_ptr, rsn, rst, vr_ptr = _ref_args(reference_points, valid_ratios)
-    mlp = M * L * P
+    mask = mask_layout(value_mask, N, T2, S, M * D)
     grad_proj = torch.empty_like(proj)
-    dims = (N, T2, T1, S, M, D, L, Lq, P)
-    L_ = capi.lib()
     if deterministic and not (presum and dt == torch.float32 and not planar):
         raise RuntimeError("the deterministic fused backward runs on the pre-summed (cell-major) float32 path")
+    ws, workspace = None, (None, 0)
     if planar:
-        slots = value_or_vsum.shape[1]
-        gsum = torch.empty_like(value_or_vsum)                                       # planar fp32 slots, zero-filled by the call
-        flags = capi.MSDA_FLAG_PRESUMMED | capi.MSDA_FLAG_PLANAR
-        with torch.cuda.device(dev), _Launch("snippet_backward_planar", dims, dev, 2):
-            status = L_.msda_snippet_backward(
-                value_or_vsum.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-                proj.data_ptr(), proj.data_ptr() + 4 * 2 * mlp, ref_ptr, grad_output.data_ptr(),
-                gsum.data_ptr(), grad_proj.data_ptr(), grad_proj.data_ptr() + 4 * 2 * mlp,
-                N, T2, T1, int(n_frame), S, M, D, L, Lq, P, 0, 0, rsn, rst, 3 * mlp, 3 * mlp,
-                _ptr(offsets_bias), _ptr(logits_bias), vr_ptr, None, 0, 0, _DTYPES[dt], flags, None, 0, _stream(dev))
-        capi.check(status, "msda_snippet_backward")
-        grad_value = torch.empty((N, T2, S, M, D), dtype=dt, device=dev)
-        with torch.cuda.device(dev), _Launch("frame_unsum_planar", (N, T2, T1, S, M * D), dev):
-            status = L_.msda_frame_unsum_planar(gsum.data_ptr(), _ptr(mask), grad_value.data_ptr(), N, T2, T1, int(n_frame),
-                                                S, M, D, mrs, mcs, _DTYPES[dt], _stream(dev))
-        capi.check(status, "msda_frame_unsum_planar")
-        return grad_value, grad_proj
-    if presum:
-        slots = value_or_vsum.shape[1]
-        gsum = torch.empty((N, slots, S, M, D), dtype=torch.float32, device=dev)   # fp32 accumulation
-        flags, ws_ptr, ws_bytes, ws, tag, n_kernels = capi.MSDA_FLAG_PRESUMMED, None, 0, None, "snippet_backward_presummed", 2
+        grad_src = torch.empty_like(value_or_vsum)                                  # planar fp32 slots, zero-filled by the call
+        flags, tag, n_kernels = capi.MSDA_FLAG_PRESUMMED | capi.MSDA_FLAG_PLANAR, "snippet_backward_planar", 2
+    elif presum:
+        grad_src = torch.empty((N, value_or_vsum.shape[1], S, M, D), dtype=torch.float32, device=dev)  # fp32 accumulation
+        flags, tag, n_kernels = capi.MSDA_FLAG_PRESUMMED, "snippet_backward_presummed", 2
         if deterministic:
             # bit-reproducible: no-scatter kernel + two-pass ordered grad_value over the slots (include/msda_b200.h)
             flags |= capi.MSDA_FLAG_DETERMINISTIC
-            ws_bytes = L_.msda_snippet_backward_workspace_bytes(N, T1, int(n_frame), S, M, D, L, Lq, P, _DTYPES[dt], flags)
-            ws = torch.empty(ws_bytes + 256, dtype=torch.uint8, device=dev)
-            ws_ptr = (ws.data_ptr() + 255) // 256 * 256
+            ws_bytes = capi.lib().msda_snippet_backward_workspace_bytes(N, T1, int(n_frame), S, M, D, L, Lq, P,
+                                                                        _DTYPES[dt], flags)
+            ws, ws_ptr = _workspace(ws_bytes, dev)
+            workspace = (ws_ptr, ws_bytes)
             tag, n_kernels = "snippet_backward_deterministic", 10
-        with torch.cuda.device(dev), _Launch(tag, dims, dev, n_kernels):
-            status = L_.msda_snippet_backward(
-                value_or_vsum.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-                proj.data_ptr(), proj.data_ptr() + 4 * 2 * mlp, ref_ptr, grad_output.data_ptr(),
-                gsum.data_ptr(), grad_proj.data_ptr(), grad_proj.data_ptr() + 4 * 2 * mlp,
-                N, T2, T1, int(n_frame), S, M, D, L, Lq, P, 0, 0, rsn, rst, 3 * mlp, 3 * mlp,
-                _ptr(offsets_bias), _ptr(logits_bias), vr_ptr, None, 0, 0, _DTYPES[dt], flags, ws_ptr, ws_bytes,
-                _stream(dev))
-        capi.check(status, "msda_snippet_backward")
-        grad_value = torch.empty((N, T2, S, M, D), dtype=dt, device=dev)
-        with torch.cuda.device(dev), _Launch("frame_unsum", (N, T2, T1, S, M * D), dev):
-            status = L_.msda_frame_unsum(gsum.data_ptr(), _ptr(mask), grad_value.data_ptr(), N, T2, T1, int(n_frame), S,
-                                         M * D, mrs, mcs, _DTYPES[dt], _stream(dev))
-        capi.check(status, "msda_frame_unsum")
-        return grad_value, grad_proj
-    sn, st = _value_strides5(value_or_vsum)
-    grad_value = torch.empty((N, T2, S, M, D), dtype=torch.float32, device=dev)  # fp32 accumulation
-    with torch.cuda.device(dev), _Launch("snippet_backward", dims, dev, 2):
-        status = L_.msda_snippet_backward(
-            value_or_vsum.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
-            proj.data_ptr(), proj.data_ptr() + 4 * 2 * mlp, ref_ptr, grad_output.data_ptr(),
-            grad_value.data_ptr(), grad_proj.data_ptr(), grad_proj.data_ptr() + 4 * 2 * mlp,
-            N, T2, T1, int(n_frame), S, M, D, L, Lq, P, sn, st, rsn, rst, 3 * mlp, 3 * mlp,
-            _ptr(offsets_bias), _ptr(logits_bias), vr_ptr, _ptr(mask), mrs, mcs, _DTYPES[dt], 0, None, 0, _stream(dev))
-    capi.check(status, "msda_snippet_backward")
-    if dt != torch.float32:
-        grad_value = grad_value.to(dt)
-    return grad_value, grad_proj
+    else:
+        grad_src = torch.empty((N, T2, S, M, D), dtype=torch.float32, device=dev)  # fp32 accumulation
+        flags, tag, n_kernels = 0, "snippet_backward", 2
+    offsets, logits = _proj_columns(proj, M * L * P)
+    grad_offsets, grad_logits = _proj_columns(grad_proj, M * L * P)
+    _issue_snippet_backward(tag, n_kernels, dims, n_frame, value_or_vsum, spatial_shapes, level_start_index,
+                            grad_output, grad_src, offsets=offsets, logits=logits, grad_offsets=grad_offsets[0],
+                            grad_logits=grad_logits[0], value_strides=(0, 0) if presum else _value_strides5(value_or_vsum),
+                            reference_points=reference_points, valid_ratios=valid_ratios,
+                            biases=(offsets_bias, logits_bias), mask=(None, 0, 0) if presum else mask, flags=flags,
+                            workspace=workspace)
+    if presum:
+        return _frame_unsum(grad_src, mask, dims, n_frame, dt, planar), grad_proj
+    return (grad_src if dt == torch.float32 else grad_src.to(dt)), grad_proj
 
 
 @snippet_attn_backward.register_fake
@@ -702,19 +665,14 @@ def _attn_setup_context(ctx, inputs, output):
     out, carry = output
     ctx.n_frame, ctx.presum, ctx.T2 = n_frame, bool(presum), value.shape[1]
     ctx.value_dims = list(value.shape[2:]) if planar else None    # the 3-d planar carry does not say
-    ctx.flags = (reference_points is not None, valid_ratios is not None, ob is not None, lb is not None,
-                 value_mask is not None)
     # the presummed value replaces value itself: the backward reads nothing else of it
-    ctx.save_for_backward(*[t for t in (carry if presum else value, spatial_shapes, level_start_index, proj,
-                                        reference_points, valid_ratios, ob, lb, value_mask) if t is not None])
+    ctx.save_for_backward(carry if presum else value, spatial_shapes, level_start_index, proj, reference_points,
+                          valid_ratios, ob, lb, value_mask)
     ctx.set_materialize_grads(False)
 
 
 def _attn_backward_formula(ctx, grad_output, grad_carry):
-    saved = list(ctx.saved_tensors)
-    value, spatial_shapes, level_start_index, proj = saved[:4]
-    rest = saved[4:]
-    ref, vr, ob, lb, value_mask = [rest.pop(0) if f else None for f in ctx.flags]
+    value, spatial_shapes, level_start_index, proj, ref, vr, ob, lb, value_mask = ctx.saved_tensors
     if grad_output is None:
         return (None,) * 12
     if _deterministic and ctx.value_dims is not None:
@@ -733,9 +691,8 @@ def _attn_backward_formula(ctx, grad_output, grad_carry):
         gob = col[:2 * mlp] if ctx.needs_input_grad[5] else None
         glb = col[2 * mlp:] if ctx.needs_input_grad[6] else None
     if ref is not None and ctx.needs_input_grad[7]:
-        goff = gproj[..., :2 * mlp].view(proj.shape[0], proj.shape[1], proj.shape[2], M, L, P, 2)
-        wh = torch.stack([spatial_shapes[:, 1], spatial_shapes[:, 0]], -1).to(goff.dtype)
-        gref = (goff * wh[None, None, None, None, :, None, :]).sum(dim=(3, 5))
+        gref = _grad_ref(gproj[..., :2 * mlp].view(proj.shape[0], proj.shape[1], proj.shape[2], M, L, P, 2),
+                         spatial_shapes)
     return gv, None, None, None, gproj, gob, glb, gref, None, None, None, None
 
 
@@ -793,12 +750,9 @@ def layer_tail(y: Tensor, bias: Optional[Tensor], residual: Tensor, gamma: Tenso
         out_pos = torch.empty_like(y)
     else:
         out_pos = y.new_empty((0,))
-    with torch.cuda.device(y.device), _Launch("layer_tail", (rows, C, int(pos is not None)), y.device):
-        status = capi.lib().msda_layer_tail(y.data_ptr(), _ptr(bias), residual.data_ptr(), gamma.data_ptr(),
-                                            beta.data_ptr(), _ptr(pos), out.data_ptr(),
-                                            out_pos.data_ptr() if pos is not None else None, rows, C, float(eps),
-                                            capi.MSDA_DTYPE_F32, _stream(y.device))
-    capi.check(status, "msda_layer_tail")
+    _launch("msda_layer_tail", "layer_tail", (rows, C, int(pos is not None)), y.device,
+            y.data_ptr(), _ptr(bias), residual.data_ptr(), gamma.data_ptr(), beta.data_ptr(), _ptr(pos),
+            out.data_ptr(), out_pos.data_ptr() if pos is not None else None, rows, C, float(eps), capi.MSDA_DTYPE_F32)
     return out, out_pos
 
 
