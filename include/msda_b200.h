@@ -34,9 +34,11 @@
  *   - every function returns an msda_status_t (0 = ok).  Launch failures are returned, not
  *     printed (the reference only printf()s them, ms_deform_im2col_cuda.cuh:948-952).
  *   - re-entrant and stateless: no entry point writes process state.  (Benchmark knobs are READ from the
- *     environment once, at the first launch, and never change results: MSDA_PAIRS_D48 / MSDA_SNIP_PAIRS_D48 =
- *     8|16|32 and MSDA_PLANAR_PAIRS = 16|32|64, queries per CTA tile; MSDA_FWD_SPLIT=0 keeps the tile kernels for
- *     few-queries launches; MSDA_PLANAR_TILE2D=0 keeps row-segment tiles in the planar kernels.)
+ *     environment once, at the first launch; they change speed, not results beyond rounding: MSDA_PAIRS_D48 /
+ *     MSDA_SNIP_PAIRS_D48 = 8|16|32 and MSDA_PLANAR_PAIRS = 16|32|64, queries per CTA tile, and
+ *     MSDA_PLANAR_TILE2D=0, row-segment tiles in the planar kernels, keep each output's summation order, so
+ *     forwards are bit-identical; MSDA_FWD_SPLIT=0 keeps the tile kernels for few-queries launches, which sum in
+ *     another order than the split kernels.)
  *   - padding masks: one byte per element, != 0 = padding; element (n,t,s,c) of a mask over value
  *     (N,T2,S,M*D) lives at mask[((n*T2+t)*S+s)*mask_row_stride + c*mask_col_stride] with
  *     mask_col_stride 1 (the reference's materialised (N,T,S,C) bool tensor, models/model.py:156-157;

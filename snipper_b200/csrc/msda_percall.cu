@@ -324,7 +324,7 @@ bool fast_path_ok(const OpDims &d, int esize)
 bool fast_path_ok(const OpDims &d) { return fast_path_ok(d, 4); }
 
 // queries per CTA tile for LANES == 12: 16 unless MSDA_PAIRS_D48 = 8 | 16 | 32 is set in the environment
-// (benchmark knob; read once, results never depend on it)
+// (benchmark knob, read once; every tile length sums each output in the same order)
 static int pairs_d48()
 {
     static const int v = env_tile_pairs("MSDA_PAIRS_D48");

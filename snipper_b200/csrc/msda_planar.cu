@@ -637,8 +637,11 @@ cudaError_t launch_fwd(const void *vsum, const int64_t *shapes, const int64_t *l
     const PlanarGeom g = make_geom(d.S, d.M);
     const dim3 grid(d.M, (d.Lq + PAIRS - 1) / PAIRS, d.N * d.T1);
     const size_t smem = (2 * sizeof(float4) + sizeof(float)) * PAIRS * d.L * d.P;
-    if (smem > kSmemOptIn)
-        cudaFuncSetAttribute(msda_planar_fwd_kernel<PAIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (smem > kSmemOptIn) {
+        const cudaError_t e =
+            cudaFuncSetAttribute(msda_planar_fwd_kernel<PAIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
     msda_planar_fwd_kernel<PAIRS><<<grid, PlanarCfg<PAIRS>::THREADS, smem, stream>>>(
         static_cast<const char *>(vsum), shapes, lsi, offsets, logits, ref, out, a, g);
     return cudaGetLastError();
@@ -653,8 +656,11 @@ cudaError_t launch_bwd(const void *vsum, const int64_t *shapes, const int64_t *l
     const PlanarGeom g = make_geom(d.S, d.M);
     const dim3 grid(d.M, (d.Lq + PAIRS - 1) / PAIRS, d.N * d.T1);
     const size_t smem = (2 * sizeof(float4) + 4 * sizeof(float)) * PAIRS * d.L * d.P;
-    if (smem > kSmemOptIn)
-        cudaFuncSetAttribute(msda_planar_bwd_kernel<PAIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (smem > kSmemOptIn) {
+        const cudaError_t e =
+            cudaFuncSetAttribute(msda_planar_bwd_kernel<PAIRS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
     msda_planar_bwd_kernel<PAIRS><<<grid, PlanarCfg<PAIRS>::THREADS, smem, stream>>>(
         static_cast<const char *>(vsum), shapes, lsi, offsets, logits, ref, grad_out, static_cast<char *>(gsum),
         grad_offsets, grad_logits, a, g);

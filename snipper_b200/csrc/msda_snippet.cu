@@ -500,7 +500,7 @@ bool snippet_ok(const SnippetDims &d, int esize)
 bool snippet_ok(const SnippetDims &d) { return snippet_ok(d, 4); }
 
 // queries per CTA tile for D = 48: 16 unless MSDA_SNIP_PAIRS_D48 = 8 | 16 | 32 is set in the environment
-// (benchmark knob; read once, results never depend on it)
+// (benchmark knob, read once; every tile length sums each output in the same order)
 int snip_pairs_d48()
 {
     static const int v = env_tile_pairs("MSDA_SNIP_PAIRS_D48");
@@ -552,9 +552,11 @@ static cudaError_t launch_snip_bwd_impl(const typename Chunk<VT>::elem *value, c
     const SnipArgs a = make_snip_args<VT>(d);
     const dim3 grid(d.M, (d.Lq + PAIRS - 1) / PAIRS, d.N * d.T1);
     const size_t smem = sizeof(float4) * Cfg::PAIRS * (d.L * d.P + 1) + sizeof(float) * 3 * Cfg::SUBS * Cfg::PAIRS * d.L * d.P;
-    if (smem > kSmemOptIn)
-        cudaFuncSetAttribute(msda_snippet_bwd_kernel<VT, LANES, PAIRS, CSB, MODE>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (smem > kSmemOptIn) {
+        const cudaError_t e = cudaFuncSetAttribute(msda_snippet_bwd_kernel<VT, LANES, PAIRS, CSB, MODE>,
+                                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
     msda_snippet_bwd_kernel<VT, LANES, PAIRS, CSB, MODE><<<grid, Cfg::THREADS, smem, stream>>>(
         value, shapes, lsi, offsets, logits, ref, grad_out, grad_value, grad_offsets, grad_logits, a);
     return cudaGetLastError();
@@ -591,7 +593,10 @@ static cudaError_t launch_snip_bwd_noscatter(const typename Chunk<VT>::elem *val
     const dim3 grid(d.M, (d.Lq + PAIRS - 1) / PAIRS, d.N * d.T1);
     const size_t smem = sizeof(float4) * Cfg::PAIRS * (d.L * d.P + 1) + sizeof(float) * 3 * Cfg::SUBS * Cfg::PAIRS * d.L * d.P;
     auto kernel = msda_snippet_bwd_kernel<VT, LANES, PAIRS, 0, kPresummed, false>;
-    if (smem > kSmemOptIn) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (smem > kSmemOptIn) {
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
     kernel<<<grid, Cfg::THREADS, smem, stream>>>(value, shapes, lsi, offsets, logits, ref, grad_out, nullptr,
                                                 grad_offsets, grad_logits, a);
     return cudaGetLastError();
