@@ -15,8 +15,19 @@ loads) to a version that
     (get_reference_points, :219-232), so the fused kernels compute the reference points from the query index
     (SURVEY.md section 8f rank 2).
 
-It applies in inference (autograd off or nothing requiring grad), fp32, dropout inactive; in every other
-situation the layer's ORIGINAL forward runs, so training behaviour is exactly the stock one.
+``_eligible`` alone decides, per call, whether the fused forward runs.  It runs only when all of these hold:
+
+  * the residual stream is fp32 on CUDA with C = 128*k <= 1024 channels (what the kernel covers);
+  * autocast is off for CUDA (under autocast the GEMMs return bf16 / fp16, which the fp32 kernel does not take);
+  * nothing would need a gradient: grad mode is off, or no parameter of the layer and no tensor argument of its
+    forward (src / tgt, pos / query_pos, reference points, the decoder's src, masks) requires grad -- the tail
+    op has no autograd formula;
+  * every dropout of the layer is inactive (p = 0 or eval mode);
+  * the FFN activation is ReLU (``layer.activation is F.relu`` where the layer has one, as the reference's do);
+  * every norm is an ``nn.LayerNorm`` with both weight and bias, and ``linear1`` has a bias.
+
+In every other situation the layer's ORIGINAL forward runs, so training, autocast and any layer variant keep
+exactly the stock behaviour.
 Works on the reference's own layer classes (after ``install_module()``) and on the bench harness' layers: both
 expose the reference's attribute names (self_attn / cross_attn, norm1..3, linear1/2, dropout1..4).
 """
@@ -36,9 +47,21 @@ def _dropout_off(layer):
     return not any(isinstance(m, nn.Dropout) and m.p > 0 and m.training for m in layer.children())
 
 
-def _eligible(layer, x):
-    return (ops.layer_tail_supported(x, x) and _dropout_off(layer) and
-            not (torch.is_grad_enabled() and any(p.requires_grad for p in layer.parameters())))
+def _affine_layer_norm(norm):
+    return isinstance(norm, nn.LayerNorm) and norm.weight is not None and norm.bias is not None
+
+
+def _eligible(layer, x, *inputs):
+    """Whether the fused forward computes what ``layer``'s own forward would (the module docstring lists the
+    conditions).  ``x`` is the residual stream, ``inputs`` every other argument of the layer's forward."""
+    if torch.is_autocast_enabled("cuda") or not ops.layer_tail_supported(x, x) or not _dropout_off(layer):
+        return False
+    if torch.is_grad_enabled() and (any(p.requires_grad for p in layer.parameters()) or
+                                    any(torch.is_tensor(t) and t.requires_grad for t in inputs)):
+        return False
+    norms = [getattr(layer, n) for n in ("norm1", "norm2", "norm3") if hasattr(layer, n)]
+    return (getattr(layer, "activation", F.relu) is F.relu and all(_affine_layer_norm(n) for n in norms) and
+            layer.linear1.bias is not None)
 
 
 def _tail(y, bias, residual, norm, pos=None):
@@ -64,7 +87,7 @@ def _with_pos(x, pos):
 
 def _encoder_forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask=None):
     """reference deformable_transformer.py:200-210 (forward) and :192-198 (forward_ffn)"""
-    if not _eligible(self, src):
+    if not _eligible(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask):
         return self._stock_forward(src, pos, reference_points, spatial_shapes, level_start_index, padding_mask)
     attn = self.self_attn
     core, _ = attn._attend(_with_pos(src, pos), reference_points, src, spatial_shapes, level_start_index, padding_mask)
@@ -81,7 +104,8 @@ def _encoder_forward(self, src, pos, reference_points, spatial_shapes, level_sta
 def _decoder_forward(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
                      src_padding_mask=None):
     """reference deformable_transformer.py:279-300 (forward) and :268-274 (forward_ffn)"""
-    if not _eligible(self, tgt):
+    if not _eligible(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
+                     src_padding_mask):
         return self._stock_forward(tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
                                    src_padding_mask)
     bs, t, lq, c = tgt.shape
@@ -105,7 +129,8 @@ def _reference_encoder_forward(self, src, spatial_shapes, level_start_index, val
                                n_frame=1):
     """reference DeformableTransformerEncoder.forward (deformable_transformer.py:234-241) without building the
     (N,T,S,L,2) reference-point tensor: the layers receive its closed form (``EncoderGrid``)."""
-    if not (torch.is_tensor(spatial_shapes) and _eligible(self.layers[0], src)):
+    if not (torch.is_tensor(spatial_shapes) and
+            _eligible(self.layers[0], src, pos, valid_ratios, spatial_shapes, level_start_index, padding_mask)):
         return self._stock_forward(src, spatial_shapes, level_start_index, valid_ratios, pos, padding_mask, n_frame)
     grid = EncoderGrid(valid_ratios, _sizes_of(self, spatial_shapes), n_frame)
     output = src
