@@ -1,6 +1,9 @@
 """Build libmsda_b200.so in-tree with nvcc for sm_100a (replaces the reference's
 models/ops/setup.py + make.sh torch CUDAExtension build).  No torch headers are involved:
-the library is plain CUDA behind a C ABI (include/msda_b200.h)."""
+the library is plain CUDA behind a C ABI (include/msda_b200.h).
+
+``build_all`` also builds the companion library libmsda_b200_amp.so (csrc_amp/, include/msda_b200_amp.h), the
+mixed-precision layer tail used under bf16 autocast, with the same flags."""
 import os
 import shutil
 import subprocess
@@ -12,6 +15,10 @@ LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200.so")
 SOURCES = ["msda_capi.cu", "msda_percall.cu", "msda_snippet.cu", "msda_deterministic.cu", "msda_mask.cu", "msda_frames.cu", "msda_tail.cu", "msda_planar.cu"]
 HEADERS = ["msda_common.cuh", "msda_fast.cuh", "msda_snippet_common.cuh", "msda_internal.h", os.path.join("..", "..", "include", "msda_b200.h")]
 OBJ_DIR = os.path.join(PKG, "lib", "obj")
+AMP_CSRC = os.path.join(PKG, "csrc_amp")
+AMP_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_amp.so")
+AMP_SOURCES = ["msda_amp_tail.cu"]
+AMP_HEADERS = [os.path.join("..", "..", "include", "msda_b200_amp.h"), os.path.join("..", "..", "include", "msda_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -26,40 +33,54 @@ def _nvcc():
     return exe
 
 
-def is_stale():
-    if not os.path.exists(LIB_PATH):
+def is_stale(lib_path=LIB_PATH, csrc=CSRC, files=SOURCES + HEADERS):
+    if not os.path.exists(lib_path):
         return True
-    t = os.path.getmtime(LIB_PATH)
-    return any(os.path.getmtime(os.path.join(CSRC, f)) > t for f in SOURCES + HEADERS)
+    t = os.path.getmtime(lib_path)
+    return any(os.path.getmtime(os.path.join(csrc, f)) > t for f in files)
 
 
-def build_library(force=False, verbose=False, extra_flags=()):
-    """Compile every .cu of the package into snipper_b200/lib/libmsda_b200.so."""
-    if not force and not is_stale():
-        return LIB_PATH
+def _build(lib_path, csrc, sources, headers, force, verbose, extra_flags):
+    if not force and not is_stale(lib_path, csrc, sources + headers):
+        return lib_path
     os.makedirs(OBJ_DIR, exist_ok=True)
     nvcc = _nvcc()
 
     def compile_one(src):
         obj = os.path.join(OBJ_DIR, src.replace(".cu", ".o"))
         cmd = [nvcc] + NVCC_FLAGS + list(extra_flags) + os.environ.get("MSDA_NVCC_EXTRA", "").split() + (["-Xptxas=-v"] if verbose else []) + ["-c", src, "-o", obj]
-        res = subprocess.run(cmd, cwd=CSRC, capture_output=True, text=True)
+        res = subprocess.run(cmd, cwd=csrc, capture_output=True, text=True)
         return src, obj, res
 
     from concurrent.futures import ThreadPoolExecutor
-    with ThreadPoolExecutor(max_workers=len(SOURCES)) as pool:  # the translation units compile side by side
-        results = list(pool.map(compile_one, SOURCES))
+    with ThreadPoolExecutor(max_workers=len(sources)) as pool:  # the translation units compile side by side
+        results = list(pool.map(compile_one, sources))
     for src, obj, res in results:
         if verbose:
             print(res.stdout + res.stderr)
         if res.returncode != 0:
             raise RuntimeError("nvcc failed on %s:\n%s" % (src, res.stdout + res.stderr))
-    link = [nvcc, "-shared", "-Xcompiler", "-fPIC", "-o", LIB_PATH] + [obj for _, obj, _ in results]
-    res = subprocess.run(link, cwd=CSRC, capture_output=True, text=True)
+    link = [nvcc, "-shared", "-Xcompiler", "-fPIC", "-o", lib_path] + [obj for _, obj, _ in results]
+    res = subprocess.run(link, cwd=csrc, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError("link failed:\n" + res.stdout + res.stderr)
-    return LIB_PATH
+    return lib_path
+
+
+def build_library(force=False, verbose=False, extra_flags=()):
+    """Compile every .cu of the package into snipper_b200/lib/libmsda_b200.so."""
+    return _build(LIB_PATH, CSRC, SOURCES, HEADERS, force, verbose, extra_flags)
+
+
+def build_amp_library(force=False, verbose=False, extra_flags=()):
+    """Compile csrc_amp/ into snipper_b200/lib/libmsda_b200_amp.so."""
+    return _build(AMP_LIB_PATH, AMP_CSRC, AMP_SOURCES, AMP_HEADERS, force, verbose, extra_flags)
+
+
+def build_all(force=False, verbose=False):
+    """-> (LIB_PATH, AMP_LIB_PATH), both built."""
+    return build_library(force, verbose), build_amp_library(force, verbose)
 
 
 if __name__ == "__main__":
-    print(build_library(force=True, verbose=True))
+    print(*build_all(force=True, verbose=True), sep="\n")

@@ -1,14 +1,16 @@
-"""ctypes binding of libmsda_b200.so (include/msda_b200.h).
+"""ctypes binding of libmsda_b200.so (include/msda_b200.h) and of its mixed-precision companion
+libmsda_b200_amp.so (include/msda_b200_amp.h).
 
 This is the ONLY way the package reaches compute: there is no CPU fallback and no alternate
-backend.  If the library is missing, importing callers fail loudly.
+backend.  If a library is missing, its callers fail loudly.
 """
 import ctypes
 import os
 
-from .build import LIB_PATH
+from .build import AMP_LIB_PATH, LIB_PATH
 
 MSDA_ABI_VERSION = 4
+MSDA_AMP_ABI_VERSION = 1
 
 MSDA_OK = 0
 MSDA_ERR_INVALID_ARGUMENT = 1
@@ -34,8 +36,11 @@ EXPORTS = (
     "msda_snippet_backward", "msda_snippet_backward_workspace_bytes", "msda_snippet_num_slots", "msda_snippet_prefers_presum", "msda_frame_sum",
     "msda_frame_unsum", "msda_layer_tail", "msda_planar_slot_bytes", "msda_frame_sum_planar", "msda_frame_unsum_planar",
 )
+# every symbol include/msda_b200_amp.h declares
+AMP_EXPORTS = ("msda_amp_abi_version", "msda_amp_last_cuda_error", "msda_amp_layer_tail")
 
 _lib = None
+_amp_lib = None
 
 
 class MsdaError(RuntimeError):
@@ -99,8 +104,34 @@ def lib():
     return L
 
 
-def check(status, what, batch=None, im2col_step=None):
-    """Turn a status code into the exception the reference would have raised."""
+def amp_lib():
+    """Load (once) and return the ctypes handle of libmsda_b200_amp.so; raise if it was not built."""
+    global _amp_lib
+    if _amp_lib is not None:
+        return _amp_lib
+    if not os.path.exists(AMP_LIB_PATH):
+        raise RuntimeError(
+            "libmsda_b200_amp.so is not built (%s). Build it with "
+            "`python -c 'import __graft_entry__ as g; g.build()'` or `python -m snipper_b200.build`. "
+            "There is no CPU / PyTorch fallback for this op." % AMP_LIB_PATH)
+    L = ctypes.CDLL(AMP_LIB_PATH)
+    vp, i32, i64 = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64
+    L.msda_amp_abi_version.restype = i32
+    L.msda_amp_abi_version.argtypes = []
+    L.msda_amp_last_cuda_error.restype = i32
+    L.msda_amp_last_cuda_error.argtypes = []
+    L.msda_amp_layer_tail.restype = i32
+    L.msda_amp_layer_tail.argtypes = [vp, vp, vp, i32] + [vp] * 6 + [i64, i32, ctypes.c_float, vp]
+    if L.msda_amp_abi_version() != MSDA_AMP_ABI_VERSION:
+        raise RuntimeError("libmsda_b200_amp.so ABI %d != binding ABI %d; rebuild" %
+                           (L.msda_amp_abi_version(), MSDA_AMP_ABI_VERSION))
+    _amp_lib = L
+    return L
+
+
+def check(status, what, batch=None, im2col_step=None, last_cuda_error=None):
+    """Turn a status code into the exception the reference would have raised.  ``last_cuda_error``: the
+    ``*_last_cuda_error`` function of the library that returned ``status`` (default: libmsda_b200.so's)."""
     if status == MSDA_OK:
         return
     L = lib()
@@ -109,5 +140,5 @@ def check(status, what, batch=None, im2col_step=None):
         # reference message: ms_deform_attn_cuda.cu:52
         msg = "batch(%d) must divide im2col_step(%d)" % (batch, min(batch, im2col_step) if im2col_step > 0 else im2col_step)
     if status == MSDA_ERR_CUDA:
-        msg += " [cudaError %d]" % L.msda_last_cuda_error()
+        msg += " [cudaError %d]" % (last_cuda_error or L.msda_last_cuda_error)()
     raise MsdaError(status, "%s: %s" % (what, msg))

@@ -15,18 +15,32 @@ loads) to a version that
     (get_reference_points, :219-232), so the fused kernels compute the reference points from the query index
     (SURVEY.md section 8f rank 2).
 
-``_eligible`` alone decides, per call, whether the fused forward runs.  It runs only when all of these hold:
+``_eligible`` alone decides, per call, which of three forwards runs:
 
-  * the residual stream is fp32 on CUDA with C = 128*k <= 1024 channels (what the kernel covers);
-  * autocast is off for CUDA (under autocast the GEMMs return bf16 / fp16, which the fp32 kernel does not take);
+  * the layer's ORIGINAL forward (stock);
+  * the fp32 tails (``layer_tail``), when autocast is off for CUDA and the residual stream is fp32 on CUDA with
+    C = 128*k <= 1024 channels (what the kernel covers);
+  * the bf16 autocast tails (``layer_tail_amp``, libmsda_b200_amp.so), when the layer was switched with
+    ``enable_fused_layer_tails(model, autocast=True)``, autocast is on for CUDA with dtype bfloat16, the residual
+    stream is fp32 or bf16 on CUDA with C = 128*k <= 1024, and ``pos`` / ``query_pos`` is absent or fp32.  The GEMM
+    in front of each tail returns bf16 there; the tail reads it, writes the fp32 residual stream (what autocast's
+    fp32 LayerNorm gives) and, in the same pass, the bf16 copies the next GEMMs take -- ``linear1``'s input, and the
+    next encoder layer's ``value_proj`` input and query (the decoder's cross-attention query) -- with exactly the
+    bits autocast's own cast would give them.  The FFN's first GEMM then runs in bf16 with its bias + ReLU
+    epilogue.  The result is not bit-identical to the stock autocast network (the output_proj / linear2 bias is
+    added in fp32 rather than in a bf16 GEMM epilogue, and the LayerNorm sums in another order), which is why it
+    is opt-in per model.  Autocast to float16 keeps the stock layers.
+
+Both fused forwards further need all of these:
+
   * nothing would need a gradient: grad mode is off, or no parameter of the layer and no tensor argument of its
     forward (src / tgt, pos / query_pos, reference points, the decoder's src, masks) requires grad -- the tail
-    op has no autograd formula;
+    ops have no autograd formula;
   * every dropout of the layer is inactive (p = 0 or eval mode);
   * the FFN activation is ReLU (``layer.activation is F.relu`` where the layer has one, as the reference's do);
   * every norm is an ``nn.LayerNorm`` with both weight and bias, and ``linear1`` has a bias.
 
-In every other situation the layer's ORIGINAL forward runs, so training, autocast and any layer variant keep
+In every other situation the layer's ORIGINAL forward runs, so training, fp16 autocast and any layer variant keep
 exactly the stock behaviour.
 Works on the reference's own layer classes (after ``install_module()``) and on the bench harness' layers: both
 expose the reference's attribute names (self_attn / cross_attn, norm1..3, linear1/2, dropout1..4).
@@ -41,6 +55,7 @@ from . import ops
 from .modules import EncoderGrid, MSDeformAttn
 
 _PLUS_POS = "_snipper_b200_plus_pos"   # attribute on a layer's output tensor: (pos tensor, output + pos)
+_AS_BF16 = "_snipper_b200_as_bf16"     # attribute on an amp layer's output tensor: the output rounded to bf16
 
 
 def _dropout_off(layer):
@@ -51,77 +66,110 @@ def _affine_layer_norm(norm):
     return isinstance(norm, nn.LayerNorm) and norm.weight is not None and norm.bias is not None
 
 
-def _eligible(layer, x, *inputs):
-    """Whether the fused forward computes what ``layer``'s own forward would (the module docstring lists the
-    conditions).  ``x`` is the residual stream, ``inputs`` every other argument of the layer's forward."""
-    if torch.is_autocast_enabled("cuda") or not ops.layer_tail_supported(x, x) or not _dropout_off(layer):
-        return False
+def _eligible(layer, x, pos, *inputs):
+    """Which forward computes what ``layer``'s own forward would (the module docstring lists the conditions):
+    None (the layer's own), "fp32" or "amp".  ``x`` is the residual stream, ``pos`` the positional embedding
+    (``pos`` / ``query_pos``), ``inputs`` every other argument of the layer's forward."""
+    if torch.is_autocast_enabled("cuda"):
+        if not (getattr(layer, "_amp_tails", False) and torch.get_autocast_dtype("cuda") == torch.bfloat16 and
+                ops.layer_tail_amp_supported(x, pos)):
+            return None
+        path = "amp"
+    elif ops.layer_tail_supported(x, x):
+        path = "fp32"
+    else:
+        return None
+    if not _dropout_off(layer):
+        return None
     if torch.is_grad_enabled() and (any(p.requires_grad for p in layer.parameters()) or
-                                    any(torch.is_tensor(t) and t.requires_grad for t in inputs)):
-        return False
+                                    any(torch.is_tensor(t) and t.requires_grad for t in (pos,) + inputs)):
+        return None
     norms = [getattr(layer, n) for n in ("norm1", "norm2", "norm3") if hasattr(layer, n)]
-    return (getattr(layer, "activation", F.relu) is F.relu and all(_affine_layer_norm(n) for n in norms) and
-            layer.linear1.bias is not None)
+    if (getattr(layer, "activation", F.relu) is F.relu and all(_affine_layer_norm(n) for n in norms) and
+            layer.linear1.bias is not None):
+        return path
+    return None
 
 
-def _tail(y, bias, residual, norm, pos=None):
+def _tail(y, bias, residual, norm, pos=None, amp=False, emit_bf16=False):
+    """-> (out fp32, out in bf16 or None, out + pos or None).  ``amp``: y is a bf16 GEMM output; out + pos is then
+    returned in bf16 and ``emit_bf16`` asks for the bf16 copy of out."""
+    if amp:
+        out, out16, out_pos = torch.ops.snipper_b200.layer_tail_amp(y, bias, residual, norm.weight, norm.bias, pos,
+                                                                    norm.eps, emit_bf16)
+        return out, (out16 if emit_bf16 else None), (out_pos if pos is not None else None)
     out, out_pos = torch.ops.snipper_b200.layer_tail(y, bias, residual, norm.weight, norm.bias, pos, norm.eps)
-    return out, (out_pos if pos is not None else None)
+    return out, None, (out_pos if pos is not None else None)
 
 
 def _ffn_hidden(layer, x):
-    """relu(linear1(x)) with the bias + ReLU applied in the GEMM epilogue."""
+    """relu(linear1(x)) with the bias + ReLU applied in the GEMM epilogue.  A bf16 ``x`` (an amp tail's copy) makes
+    it a bf16 GEMM: ``_addmm_activation`` is not on autocast's cast list, so the weight and bias are rounded here as
+    autocast would round them."""
     c = x.shape[-1]
-    return torch._addmm_activation(layer.linear1.bias, x.reshape(-1, c), layer.linear1.weight.t())
+    w, b = layer.linear1.weight, layer.linear1.bias
+    if x.dtype != w.dtype:
+        w, b = w.to(x.dtype), b.to(x.dtype)
+    return torch._addmm_activation(b, x.reshape(-1, c), w.t())
 
 
-def _with_pos(x, pos):
-    """x + pos, taken from the previous layer's tail when it already produced it for this very ``pos``."""
+def _with_pos(x, pos, amp):
+    """x + pos, taken from the previous layer's tail when it already produced it for this very ``pos`` (in bf16 on
+    the ``amp`` path, where the query only feeds a bf16 GEMM; else in fp32)."""
     if pos is None:
         return x
     cached = getattr(x, _PLUS_POS, None)
-    if cached is not None and cached[0] is pos:
+    if cached is not None and cached[0] is pos and (cached[1].dtype == torch.bfloat16) == amp:
         return cached[1]
     return x + pos
 
 
 def _encoder_forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask=None):
     """reference deformable_transformer.py:200-210 (forward) and :192-198 (forward_ffn)"""
-    if not _eligible(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask):
+    path = _eligible(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask)
+    if path is None:
         return self._stock_forward(src, pos, reference_points, spatial_shapes, level_start_index, padding_mask)
+    amp = path == "amp"
     attn = self.self_attn
-    core, _ = attn._attend(_with_pos(src, pos), reference_points, src, spatial_shapes, level_start_index, padding_mask)
+    value_in = getattr(src, _AS_BF16, src) if amp else src                   # the previous amp tail's bf16 copy
+    core, _ = attn._attend(_with_pos(src, pos, amp), reference_points, value_in, spatial_shapes, level_start_index,
+                           padding_mask)
     y = F.linear(core, attn.output_proj.weight)                              # bias joins the tail
-    x, _ = _tail(y, attn.output_proj.bias, src, self.norm1)                  # :204-205
-    ff = F.linear(_ffn_hidden(self, x), self.linear2.weight).view_as(x)      # :194
+    x, x16, _ = _tail(y, attn.output_proj.bias, src, self.norm1, amp=amp, emit_bf16=amp)   # :204-205
+    ff = F.linear(_ffn_hidden(self, x16 if amp else x), self.linear2.weight).view_as(x)  # :194
     emit = pos if (self._emit_next_query and pos is not None) else None
-    out, out_pos = _tail(ff, self.linear2.bias, x, self.norm2, emit)         # :195-197 (+ the next layer's :202)
+    out, out16, out_pos = _tail(ff, self.linear2.bias, x, self.norm2, emit,  # :195-197 (+ the next layer's :202)
+                                amp=amp, emit_bf16=amp and self._emit_next_query)
     if out_pos is not None:
         setattr(out, _PLUS_POS, (pos, out_pos))
+    if out16 is not None:
+        setattr(out, _AS_BF16, out16)
     return out
 
 
 def _decoder_forward(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
                      src_padding_mask=None):
     """reference deformable_transformer.py:279-300 (forward) and :268-274 (forward_ffn)"""
-    if not _eligible(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
-                     src_padding_mask):
+    path = _eligible(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
+                     src_padding_mask)
+    if path is None:
         return self._stock_forward(tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
                                    src_padding_mask)
+    amp = path == "amp"
     bs, t, lq, c = tgt.shape
     x = tgt.reshape(bs, t * lq, c)
     qp = None if query_pos is None else query_pos.reshape(bs, t * lq, c)
     qk = (x if qp is None else x + qp).transpose(0, 1)
     sa = self.self_attn(qk, qk, x.transpose(0, 1))[0].transpose(0, 1)        # :285 (nn.MultiheadAttention, stock)
-    x, xq = _tail(sa, None, x, self.norm2, qp)                               # :286-287 (+ with_pos_embed of :292)
+    x, _, xq = _tail(sa, None, x, self.norm2, qp, amp=amp)                   # :286-287 (+ with_pos_embed of :292)
     q = (x if xq is None else xq).view(bs, t, lq, c)
     x = x.view(bs, t, lq, c)
     attn = self.cross_attn
     core, vis = attn._attend(q, reference_points, src, src_spatial_shapes, level_start_index, src_padding_mask)
     y = F.linear(core, attn.output_proj.weight)
-    x, _ = _tail(y, attn.output_proj.bias, x, self.norm1)                    # :294-295
-    ff = F.linear(_ffn_hidden(self, x), self.linear2.weight).view_as(x)      # :270
-    out, _ = _tail(ff, self.linear2.bias, x, self.norm3)                     # :271-273
+    x, x16, _ = _tail(y, attn.output_proj.bias, x, self.norm1, amp=amp, emit_bf16=amp)   # :294-295
+    ff = F.linear(_ffn_hidden(self, x16 if amp else x), self.linear2.weight).view_as(x)  # :270
+    out, _, _ = _tail(ff, self.linear2.bias, x, self.norm3, amp=amp)         # :271-273
     return out, vis
 
 
@@ -161,9 +209,11 @@ def _is_decoder_layer(m):
             all(hasattr(m, a) for a in ("norm1", "norm2", "norm3", "linear1", "linear2")))
 
 
-def enable_fused_layer_tails(model):
+def enable_fused_layer_tails(model, autocast=False):
     """Rebind ``forward`` of every deformable encoder / decoder layer under ``model`` (idempotent).
-    Returns the number of layers switched.  ``disable_fused_layer_tails`` undoes it."""
+    ``autocast=True`` also lets the layers run their tails under bf16 autocast (the module docstring says what that
+    changes); calling again with another value updates every switched layer.  Returns the number of layers newly
+    switched.  ``disable_fused_layer_tails`` undoes it."""
     n = 0
     for parent in model.modules():
         layers = getattr(parent, "layers", None)
@@ -171,7 +221,10 @@ def enable_fused_layer_tails(model):
             continue
         for i, layer in enumerate(layers):
             enc, dec = _is_encoder_layer(layer), _is_decoder_layer(layer)
-            if not (enc or dec) or hasattr(layer, "_stock_forward"):
+            if not (enc or dec):
+                continue
+            layer._amp_tails = bool(autocast)
+            if hasattr(layer, "_stock_forward"):
                 continue
             layer._stock_forward = layer.forward
             layer._emit_next_query = enc and i + 1 < len(layers) and _is_encoder_layer(layers[i + 1])
@@ -196,4 +249,6 @@ def disable_fused_layer_tails(model):
             del m.__dict__["forward"]
             del m.__dict__["_stock_forward"]
             n += _is_encoder_layer(m) or _is_decoder_layer(m)
+        for a in ("_amp_tails", "_emit_next_query"):
+            m.__dict__.pop(a, None)
     return n

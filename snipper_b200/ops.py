@@ -11,6 +11,8 @@ in the hand-written kernels.  Ops (namespace ``snipper_b200``):
                                         biases, padding mask and encoder reference points; what the module runs
   masked_zero_                          in-place masked zero-fill of value (ms_deform_attn.py:116-117)
   layer_tail                            bias + residual + LayerNorm (+ pos) after a block, inference only
+  layer_tail_amp                        the same on a bf16 GEMM output, also writing the next GEMMs' bf16 inputs
+                                        (libmsda_b200_amp.so, for bf16 autocast)
 
 The three forwards (msda_forward, snippet_forward, snippet_attn) carry ``register_autograd`` formulas, so they
 compose with autograd / DDP as plain nodes (no host sync, no unused parameters).
@@ -75,20 +77,22 @@ class LaunchStats:
 STATS = LaunchStats()
 
 
-def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None, im2col_step=None):
-    """Call the C entry point ``entry`` with ``args`` and ``device``'s current stream (every launching entry point takes
-    the stream last), count its ``n_kernels`` kernels in STATS under ``tag`` / ``dims`` and raise on a failed status."""
+def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None, im2col_step=None, amp=False):
+    """Call the C entry point ``entry`` (of libmsda_b200_amp.so when ``amp``) with ``args`` and ``device``'s current
+    stream (every launching entry point takes the stream last), count its ``n_kernels`` kernels in STATS under ``tag`` /
+    ``dims`` and raise on a failed status."""
+    lib = capi.amp_lib() if amp else capi.lib()
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device)
         if STATS.timing:
             start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             start.record(stream)
-        status = getattr(capi.lib(), entry)(*args, stream.cuda_stream)
+        status = getattr(lib, entry)(*args, stream.cuda_stream)
         STATS.launches += n_kernels
         if STATS.timing:
             end.record(stream)
             STATS.events.append((tag, dims, start, end))
-    capi.check(status, what or entry, batch, im2col_step)
+    capi.check(status, what or entry, batch, im2col_step, lib.msda_amp_last_cuda_error if amp else None)
 
 
 def _workspace(nbytes, device):
@@ -759,3 +763,58 @@ def layer_tail(y: Tensor, bias: Optional[Tensor], residual: Tensor, gamma: Tenso
 @layer_tail.register_fake
 def _(y, bias, residual, gamma, beta, pos, eps):
     return torch.empty_like(y), (torch.empty_like(y) if pos is not None else y.new_empty((0,)))
+
+
+# ------------------------------------------------------------------------------------------
+# layer tail under bf16 autocast (libmsda_b200_amp.so): the block's Linear returned bf16, the residual stream stays
+# fp32, and the next GEMMs want bf16 copies of the result -- written by the same pass
+# ------------------------------------------------------------------------------------------
+def layer_tail_amp_supported(residual: Tensor, pos: Optional[Tensor] = None) -> bool:
+    """fp32 or bf16 CUDA residual rows of 128*k <= 1024 channels, ``pos`` absent or fp32 shaped like them, inference
+    (no autograd formula exists for this op).  The GEMM output the op adds is bf16 rows of the same shape."""
+    C = residual.shape[-1]
+    return (residual.is_cuda and residual.dtype in (torch.float32, torch.bfloat16) and C % 128 == 0 and C <= 1024 and
+            (pos is None or (pos.dtype == torch.float32 and pos.shape == residual.shape)) and
+            not (torch.is_grad_enabled() and (residual.requires_grad or (pos is not None and pos.requires_grad))))
+
+
+@torch.library.custom_op("snipper_b200::layer_tail_amp", mutates_args=())
+def layer_tail_amp(y: Tensor, bias: Optional[Tensor], residual: Tensor, gamma: Tensor, beta: Tensor,
+                   pos: Optional[Tensor], eps: float, emit_bf16: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """(out, out_bf16, out_pos_bf16) with out = LayerNorm(residual + (y + bias)) in fp32 -- the bits ``layer_tail``
+    gives for y.float(), residual.float() -- out_bf16 = out rounded to bf16 (empty unless ``emit_bf16``) and
+    out_pos_bf16 = (out + pos) rounded to bf16 (empty when ``pos`` is None).  y is bf16, residual fp32 or bf16,
+    bias / gamma / beta / pos fp32."""
+    _require_cuda(y, "y")
+    C = y.shape[-1]
+    if (y.dtype != torch.bfloat16 or residual.dtype not in (torch.float32, torch.bfloat16) or C % 128 != 0 or
+            C > 1024 or residual.shape != y.shape):
+        raise RuntimeError("layer_tail_amp: bfloat16 rows of 128*k <= 1024 channels, residual float32 / bfloat16 "
+                           "shaped like y")
+    y, residual = y.contiguous(), residual.contiguous()
+    for t, n in ((bias, C), (gamma, C), (beta, C)):
+        if t is not None and (t.numel() != n or t.dtype != torch.float32 or not t.is_contiguous()):
+            raise RuntimeError("layer_tail_amp: bias / gamma / beta must be contiguous float32 vectors of C elements")
+    rows = y.numel() // C
+    out = torch.empty(y.shape, dtype=torch.float32, device=y.device)
+    out_bf16 = torch.empty_like(y) if emit_bf16 else y.new_empty((0,))
+    if pos is not None:
+        if pos.shape != y.shape or pos.dtype != torch.float32:
+            raise RuntimeError("layer_tail_amp: pos must be float32 shaped like y")
+        pos = pos.contiguous()
+        out_pos = torch.empty_like(y)
+    else:
+        out_pos = y.new_empty((0,))
+    _launch("msda_amp_layer_tail", "layer_tail_amp", (rows, C, residual.element_size(), int(emit_bf16), int(pos is not None)),
+            y.device,
+            y.data_ptr(), _ptr(bias), residual.data_ptr(), _DTYPES[residual.dtype], gamma.data_ptr(), beta.data_ptr(),
+            _ptr(pos), out.data_ptr(), out_bf16.data_ptr() if emit_bf16 else None,
+            out_pos.data_ptr() if pos is not None else None, rows, C, float(eps), amp=True)
+    return out, out_bf16, out_pos
+
+
+@layer_tail_amp.register_fake
+def _(y, bias, residual, gamma, beta, pos, eps, emit_bf16):
+    return (torch.empty(y.shape, dtype=torch.float32, device=y.device),
+            torch.empty_like(y) if emit_bf16 else y.new_empty((0,)),
+            torch.empty_like(y) if pos is not None else y.new_empty((0,)))
