@@ -2,8 +2,9 @@
 models/ops/setup.py + make.sh torch CUDAExtension build).  No torch headers are involved:
 the library is plain CUDA behind a C ABI (include/msda_b200.h).
 
-``build_all`` also builds the companion library libmsda_b200_amp.so (csrc_amp/, include/msda_b200_amp.h), the
-mixed-precision layer tail used under bf16 autocast, with the same flags."""
+``build_all`` also builds, with the same flags, the two companion libraries: libmsda_b200_amp.so (csrc_amp/,
+include/msda_b200_amp.h), the mixed-precision layer tail used under bf16 autocast, and libmsda_b200_train.so
+(csrc_train/, include/msda_b200_train.h), the layer tail with dropout and its backward used in training."""
 import os
 import shutil
 import subprocess
@@ -19,6 +20,10 @@ AMP_CSRC = os.path.join(PKG, "csrc_amp")
 AMP_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_amp.so")
 AMP_SOURCES = ["msda_amp_tail.cu"]
 AMP_HEADERS = [os.path.join("..", "..", "include", "msda_b200_amp.h"), os.path.join("..", "..", "include", "msda_b200.h")]
+TRAIN_CSRC = os.path.join(PKG, "csrc_train")
+TRAIN_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_train.so")
+TRAIN_SOURCES = ["msda_train_tail.cu"]
+TRAIN_HEADERS = [os.path.join("..", "..", "include", "msda_b200_train.h"), os.path.join("..", "..", "include", "msda_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -77,9 +82,14 @@ def build_amp_library(force=False, verbose=False, extra_flags=()):
     return _build(AMP_LIB_PATH, AMP_CSRC, AMP_SOURCES, AMP_HEADERS, force, verbose, extra_flags)
 
 
+def build_train_library(force=False, verbose=False, extra_flags=()):
+    """Compile csrc_train/ into snipper_b200/lib/libmsda_b200_train.so."""
+    return _build(TRAIN_LIB_PATH, TRAIN_CSRC, TRAIN_SOURCES, TRAIN_HEADERS, force, verbose, extra_flags)
+
+
 def build_all(force=False, verbose=False):
-    """-> (LIB_PATH, AMP_LIB_PATH), both built."""
-    return build_library(force, verbose), build_amp_library(force, verbose)
+    """-> (LIB_PATH, AMP_LIB_PATH, TRAIN_LIB_PATH), all three built."""
+    return build_library(force, verbose), build_amp_library(force, verbose), build_train_library(force, verbose)
 
 
 if __name__ == "__main__":

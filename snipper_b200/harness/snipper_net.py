@@ -135,6 +135,7 @@ class Encoder(nn.Module):
         super().__init__()
         self.layers, self.num_layers = _clones(layer, n), n
         self.analytic_reference_points = False   # snipper_b200.enable_fused_layer_tails: closed form, computed in-kernel
+        self.analytic_reference_points_with_grad = False   # ... also while autograd records (training=True)
 
     @staticmethod
     def reference_points(sizes, valid_ratios, device):
@@ -150,7 +151,7 @@ class Encoder(nn.Module):
         return torch.cat(pts, 1)[:, :, None] * valid_ratios[:, None]  # (b, S, L, 2)
 
     def forward(self, src, sizes, shapes, lsi, valid_ratios, pos, mask, n_frame):
-        if self.analytic_reference_points and not torch.is_grad_enabled():
+        if self.analytic_reference_points and (self.analytic_reference_points_with_grad or not torch.is_grad_enabled()):
             from ..modules import EncoderGrid
             ref = EncoderGrid(valid_ratios, sizes, n_frame)
         else:

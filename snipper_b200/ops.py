@@ -13,12 +13,15 @@ in the hand-written kernels.  Ops (namespace ``snipper_b200``):
   layer_tail                            bias + residual + LayerNorm (+ pos) after a block, inference only
   layer_tail_amp                        the same on a bf16 GEMM output, also writing the next GEMMs' bf16 inputs
                                         (libmsda_b200_amp.so, for bf16 autocast)
+  layer_tail_train / _backward          bias + dropout (by a given keep-mask) + residual + LayerNorm (+ pos) and its
+                                        backward, for training (libmsda_b200_train.so)
 
-The three forwards (msda_forward, snippet_forward, snippet_attn) carry ``register_autograd`` formulas, so they
+The four forwards (msda_forward, snippet_forward, snippet_attn, layer_tail_train) carry ``register_autograd`` formulas, so they
 compose with autograd / DDP as plain nodes (no host sync, no unused parameters).
 """
 from typing import Optional, Tuple
 
+import numpy as np
 import torch
 from torch import Tensor
 
@@ -77,11 +80,12 @@ class LaunchStats:
 STATS = LaunchStats()
 
 
-def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None, im2col_step=None, amp=False):
-    """Call the C entry point ``entry`` (of libmsda_b200_amp.so when ``amp``) with ``args`` and ``device``'s current
-    stream (every launching entry point takes the stream last), count its ``n_kernels`` kernels in STATS under ``tag`` /
-    ``dims`` and raise on a failed status."""
-    lib = capi.amp_lib() if amp else capi.lib()
+def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None, im2col_step=None, amp=False,
+            train=False):
+    """Call the C entry point ``entry`` (of libmsda_b200_amp.so when ``amp``, of libmsda_b200_train.so when ``train``)
+    with ``args`` and ``device``'s current stream (every launching entry point takes the stream last), count its
+    ``n_kernels`` kernels in STATS under ``tag`` / ``dims`` and raise on a failed status."""
+    lib = capi.amp_lib() if amp else capi.train_lib() if train else capi.lib()
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device)
         if STATS.timing:
@@ -92,7 +96,8 @@ def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None,
         if STATS.timing:
             end.record(stream)
             STATS.events.append((tag, dims, start, end))
-    capi.check(status, what or entry, batch, im2col_step, lib.msda_amp_last_cuda_error if amp else None)
+    last_error = lib.msda_amp_last_cuda_error if amp else lib.msda_train_last_cuda_error if train else None
+    capi.check(status, what or entry, batch, im2col_step, last_error)
 
 
 def _workspace(nbytes, device):
@@ -818,3 +823,145 @@ def _(y, bias, residual, gamma, beta, pos, eps, emit_bf16):
     return (torch.empty(y.shape, dtype=torch.float32, device=y.device),
             torch.empty_like(y) if emit_bf16 else y.new_empty((0,)),
             torch.empty_like(y) if pos is not None else y.new_empty((0,)))
+
+
+# ------------------------------------------------------------------------------------------
+# layer tail for training (libmsda_b200_train.so): the dropout in front of the norm applies a keep-mask the caller drew
+# (snipper_b200/layers.py draws it with torch's generator), and the op has a backward of its own
+# ------------------------------------------------------------------------------------------
+def layer_tail_train_supported(residual: Tensor, pos: Optional[Tensor] = None) -> bool:
+    """fp32 CUDA residual rows of 128*k <= 1024 channels, ``pos`` absent or fp32 shaped like them.  Autograd may record
+    (the op has a gradient formula); the GEMM output the op adds is fp32 rows of the same shape."""
+    C = residual.shape[-1]
+    return (residual.is_cuda and residual.dtype == torch.float32 and C % 128 == 0 and C <= 1024 and
+            (pos is None or (pos.dtype == torch.float32 and pos.shape == residual.shape)))
+
+
+def keep_scale(p: float) -> float:
+    """1 / (1 - p) rounded to float, as torch's dropout scales the kept elements."""
+    return float(np.float32(1.0) / np.float32(1.0 - p))
+
+
+def _dense16(t: Tensor) -> Tensor:
+    """``t`` with dense rows at a 16-byte aligned address (the C ABI's layout), copied only when it is not."""
+    t = t.contiguous()
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+def _check_train_mask(keep_mask, y, p):
+    if not (0.0 <= p < 1.0):
+        raise RuntimeError("layer_tail_train: dropout probability must be in [0, 1)")
+    if keep_mask is None:
+        return None
+    if keep_mask.shape != y.shape or keep_mask.dtype not in (torch.uint8, torch.bool) or not keep_mask.is_cuda:
+        raise RuntimeError("layer_tail_train: keep_mask must be a uint8 / bool CUDA tensor shaped like y")
+    return _dense16(keep_mask.view(torch.uint8) if keep_mask.dtype == torch.bool else keep_mask)
+
+
+@torch.library.custom_op("snipper_b200::layer_tail_train", mutates_args=())
+def layer_tail_train(y: Tensor, bias: Optional[Tensor], residual: Tensor, keep_mask: Optional[Tensor], p: float,
+                     gamma: Tensor, beta: Tensor, pos: Optional[Tensor], eps: float
+                     ) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """(out, out_pos, h, mean_rstd): h = residual + d with d = ((y + bias) * keep_scale(p)) * keep_mask, or y + bias
+    without a mask; out = LayerNorm(h) * gamma + beta; out_pos = out + pos (empty when ``pos`` is None); mean_rstd the
+    (mean, rstd) of every row, shaped (..., 2).  h and mean_rstd are what the backward reads.  Without a mask ``out``
+    has the bits of ``layer_tail``; with one, the bits ``layer_tail`` gives for the pre-dropped input and no bias."""
+    _require_cuda(y, "y")
+    C = y.shape[-1]
+    if (y.dtype != torch.float32 or residual.dtype != torch.float32 or C % 128 != 0 or C > 1024 or
+            residual.shape != y.shape):
+        raise RuntimeError("layer_tail_train: float32 rows of 128*k <= 1024 channels, residual shaped like y")
+    keep_mask = _check_train_mask(keep_mask, y, p)
+    y, residual = _dense16(y), _dense16(residual)
+    for t in (bias, gamma, beta):
+        if t is not None and (t.numel() != C or t.dtype != torch.float32 or not t.is_contiguous()):
+            raise RuntimeError("layer_tail_train: bias / gamma / beta must be contiguous float32 vectors of C elements")
+    # locals: an aligned copy must stay alive until the kernel that reads it has run
+    bias = _dense16(bias) if bias is not None else None
+    gamma, beta = _dense16(gamma), _dense16(beta)
+    rows = y.numel() // C
+    out, h = torch.empty_like(y), torch.empty_like(y)
+    mean_rstd = y.new_empty((*y.shape[:-1], 2))
+    if pos is not None:
+        if pos.shape != y.shape or pos.dtype != torch.float32:
+            raise RuntimeError("layer_tail_train: pos must be float32 shaped like y")
+        pos = _dense16(pos)
+        out_pos = torch.empty_like(y)
+    else:
+        out_pos = y.new_empty((0,))
+    _launch("msda_train_layer_tail_forward", "layer_tail_train", (rows, C, int(keep_mask is not None), int(pos is not None)),
+            y.device, y.data_ptr(), _ptr(bias), residual.data_ptr(), _ptr(keep_mask),
+            keep_scale(p) if keep_mask is not None else 1.0, gamma.data_ptr(), beta.data_ptr(),
+            _ptr(pos), out.data_ptr(), out_pos.data_ptr() if pos is not None else None, h.data_ptr(),
+            mean_rstd.data_ptr(), rows, C, float(eps), train=True)
+    return out, out_pos, h, mean_rstd
+
+
+@layer_tail_train.register_fake
+def _(y, bias, residual, keep_mask, p, gamma, beta, pos, eps):
+    return (torch.empty_like(y), torch.empty_like(y) if pos is not None else y.new_empty((0,)), torch.empty_like(y),
+            y.new_empty((*y.shape[:-1], 2)))
+
+
+@torch.library.custom_op("snipper_b200::layer_tail_train_backward", mutates_args=())
+def layer_tail_train_backward(grad_out: Tensor, grad_out_pos: Optional[Tensor], h: Tensor, mean_rstd: Tensor,
+                              keep_mask: Optional[Tensor], p: float, gamma: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
+    """(grad_residual, grad_y, param_grads): param_grads is (3, C) = (grad_gamma, grad_beta, grad_bias), reduced in a
+    fixed order without atomics, so two calls on the same inputs give the same bits.  grad_y is also the gradient of
+    y + bias; with no mask it equals grad_residual."""
+    _require_cuda(h, "h")
+    C = h.shape[-1]
+    if (h.dtype != torch.float32 or C % 128 != 0 or C > 1024 or grad_out.shape != h.shape or
+            grad_out.dtype != torch.float32 or mean_rstd.shape != (*h.shape[:-1], 2) or
+            (grad_out_pos is not None and (grad_out_pos.shape != h.shape or grad_out_pos.dtype != torch.float32))):
+        raise RuntimeError("layer_tail_train_backward: float32 rows of 128*k <= 1024 channels, gradients shaped like h, "
+                           "mean_rstd (..., 2)")
+    if gamma.numel() != C or gamma.dtype != torch.float32:
+        raise RuntimeError("layer_tail_train_backward: gamma must be a float32 vector of C elements")
+    keep_mask = _check_train_mask(keep_mask, h, p)
+    rows = h.numel() // C
+    grad_out, h, mean_rstd, gamma = _dense16(grad_out), _dense16(h), _dense16(mean_rstd), _dense16(gamma)
+    if grad_out_pos is not None:
+        grad_out_pos = _dense16(grad_out_pos)
+    grad_residual, grad_y = torch.empty_like(h), torch.empty_like(h)
+    # the parameter gradients get a tensor of their own: autograd may keep them as .grad, the partials go with the call
+    param_grads = torch.zeros((3, C), dtype=torch.float32, device=h.device) if rows == 0 else \
+        torch.empty((3, C), dtype=torch.float32, device=h.device)
+    ws_bytes = capi.train_lib().msda_train_layer_tail_workspace_bytes(rows, C)
+    ws = torch.empty(max(ws_bytes // 4, 1), dtype=torch.float32, device=h.device)
+    _launch("msda_train_layer_tail_backward", "layer_tail_train_backward",
+            (rows, C, int(keep_mask is not None), int(grad_out_pos is not None)), h.device,
+            grad_out.data_ptr(), _ptr(grad_out_pos), h.data_ptr(), mean_rstd.data_ptr(), _ptr(keep_mask),
+            keep_scale(p) if keep_mask is not None else 1.0, gamma.data_ptr(), grad_residual.data_ptr(),
+            grad_y.data_ptr(), param_grads.data_ptr(), ws.data_ptr(), rows, C, n_kernels=2, train=True)
+    return grad_residual, grad_y, param_grads
+
+
+@layer_tail_train_backward.register_fake
+def _(grad_out, grad_out_pos, h, mean_rstd, keep_mask, p, gamma):
+    return torch.empty_like(h), torch.empty_like(h), h.new_empty((3, h.shape[-1]))
+
+
+def _tail_train_setup_context(ctx, inputs, output):
+    y, bias, residual, keep_mask, p, gamma, beta, pos, eps = inputs
+    out, out_pos, h, mean_rstd = output
+    ctx.p, ctx.has_bias, ctx.has_pos = p, bias is not None, pos is not None
+    # what stock saves for the same block: dropout its mask, layer_norm its input and (mean, rstd)
+    ctx.save_for_backward(h, mean_rstd, keep_mask, gamma)
+    ctx.set_materialize_grads(False)
+
+
+def _tail_train_backward_formula(ctx, grad_out, grad_out_pos, grad_h, grad_mean_rstd):
+    h, mean_rstd, keep_mask, gamma = ctx.saved_tensors
+    if not ctx.has_pos:
+        grad_out_pos = None
+    if grad_out is None and grad_out_pos is None:
+        return (None,) * 9
+    if grad_out is None:
+        grad_out = torch.zeros_like(h)
+    grad_residual, grad_y, pg = torch.ops.snipper_b200.layer_tail_train_backward(
+        grad_out, grad_out_pos, h, mean_rstd, keep_mask, ctx.p, gamma)
+    return (grad_y, pg[2] if ctx.has_bias else None, grad_residual, None, None, pg[0], pg[1], grad_out_pos, None)
+
+
+layer_tail_train.register_autograd(_tail_train_backward_formula, setup_context=_tail_train_setup_context)
