@@ -2,9 +2,11 @@
 models/ops/setup.py + make.sh torch CUDAExtension build).  No torch headers are involved:
 the library is plain CUDA behind a C ABI (include/msda_b200.h).
 
-``build_all`` also builds, with the same flags, the two companion libraries: libmsda_b200_amp.so (csrc_amp/,
-include/msda_b200_amp.h), the mixed-precision layer tail used under bf16 autocast, and libmsda_b200_train.so
-(csrc_train/, include/msda_b200_train.h), the layer tail with dropout and its backward used in training."""
+``build_all`` also builds, with the same flags, the three companion libraries: libmsda_b200_amp.so (csrc_amp/,
+include/msda_b200_amp.h), the mixed-precision layer tail used under bf16 autocast; libmsda_b200_train.so
+(csrc_train/, include/msda_b200_train.h), the layer tail with dropout and its backward used in training; and
+libmsda_b200_amp_train.so (csrc_amp_train/, include/msda_b200_amp_train.h), the same pair for training under bf16
+autocast."""
 import os
 import shutil
 import subprocess
@@ -19,11 +21,16 @@ OBJ_DIR = os.path.join(PKG, "lib", "obj")
 AMP_CSRC = os.path.join(PKG, "csrc_amp")
 AMP_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_amp.so")
 AMP_SOURCES = ["msda_amp_tail.cu"]
-AMP_HEADERS = [os.path.join("..", "..", "include", "msda_b200_amp.h"), os.path.join("..", "..", "include", "msda_b200.h")]
+AMP_HEADERS = ["msda_bf16_io.cuh", os.path.join("..", "..", "include", "msda_b200_amp.h"), os.path.join("..", "..", "include", "msda_b200.h")]
 TRAIN_CSRC = os.path.join(PKG, "csrc_train")
 TRAIN_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_train.so")
 TRAIN_SOURCES = ["msda_train_tail.cu"]
-TRAIN_HEADERS = [os.path.join("..", "..", "include", "msda_b200_train.h"), os.path.join("..", "..", "include", "msda_b200.h")]
+TRAIN_HEADERS = ["msda_train_common.cuh", os.path.join("..", "..", "include", "msda_b200_train.h"), os.path.join("..", "..", "include", "msda_b200.h")]
+AMP_TRAIN_CSRC = os.path.join(PKG, "csrc_amp_train")
+AMP_TRAIN_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_amp_train.so")
+AMP_TRAIN_SOURCES = ["msda_amp_train_tail.cu"]
+AMP_TRAIN_HEADERS = [os.path.join("..", "csrc_train", "msda_train_common.cuh"), os.path.join("..", "csrc_amp", "msda_bf16_io.cuh"),
+                     os.path.join("..", "..", "include", "msda_b200_amp_train.h"), os.path.join("..", "..", "include", "msda_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -87,9 +94,15 @@ def build_train_library(force=False, verbose=False, extra_flags=()):
     return _build(TRAIN_LIB_PATH, TRAIN_CSRC, TRAIN_SOURCES, TRAIN_HEADERS, force, verbose, extra_flags)
 
 
+def build_amp_train_library(force=False, verbose=False, extra_flags=()):
+    """Compile csrc_amp_train/ into snipper_b200/lib/libmsda_b200_amp_train.so."""
+    return _build(AMP_TRAIN_LIB_PATH, AMP_TRAIN_CSRC, AMP_TRAIN_SOURCES, AMP_TRAIN_HEADERS, force, verbose, extra_flags)
+
+
 def build_all(force=False, verbose=False):
-    """-> (LIB_PATH, AMP_LIB_PATH, TRAIN_LIB_PATH), all three built."""
-    return build_library(force, verbose), build_amp_library(force, verbose), build_train_library(force, verbose)
+    """-> (LIB_PATH, AMP_LIB_PATH, TRAIN_LIB_PATH, AMP_TRAIN_LIB_PATH), all four built."""
+    return (build_library(force, verbose), build_amp_library(force, verbose), build_train_library(force, verbose),
+            build_amp_train_library(force, verbose))
 
 
 if __name__ == "__main__":

@@ -1,6 +1,7 @@
 """ctypes binding of libmsda_b200.so (include/msda_b200.h) and of its companions: the mixed-precision
-libmsda_b200_amp.so (include/msda_b200_amp.h) and the training library libmsda_b200_train.so
-(include/msda_b200_train.h).
+libmsda_b200_amp.so (include/msda_b200_amp.h), the training library libmsda_b200_train.so
+(include/msda_b200_train.h) and the bf16-autocast training library libmsda_b200_amp_train.so
+(include/msda_b200_amp_train.h).
 
 This is the ONLY way the package reaches compute: there is no CPU fallback and no alternate
 backend.  If a library is missing, its callers fail loudly.
@@ -8,11 +9,12 @@ backend.  If a library is missing, its callers fail loudly.
 import ctypes
 import os
 
-from .build import AMP_LIB_PATH, LIB_PATH, TRAIN_LIB_PATH
+from .build import AMP_LIB_PATH, AMP_TRAIN_LIB_PATH, LIB_PATH, TRAIN_LIB_PATH
 
 MSDA_ABI_VERSION = 4
 MSDA_AMP_ABI_VERSION = 1
 MSDA_TRAIN_ABI_VERSION = 1
+MSDA_AMP_TRAIN_ABI_VERSION = 1
 
 MSDA_OK = 0
 MSDA_ERR_INVALID_ARGUMENT = 1
@@ -43,10 +45,15 @@ AMP_EXPORTS = ("msda_amp_abi_version", "msda_amp_last_cuda_error", "msda_amp_lay
 # every symbol include/msda_b200_train.h declares
 TRAIN_EXPORTS = ("msda_train_abi_version", "msda_train_last_cuda_error", "msda_train_layer_tail_forward",
                  "msda_train_layer_tail_workspace_bytes", "msda_train_layer_tail_backward")
+# every symbol include/msda_b200_amp_train.h declares
+AMP_TRAIN_EXPORTS = ("msda_amp_train_abi_version", "msda_amp_train_last_cuda_error",
+                     "msda_amp_train_layer_tail_forward", "msda_amp_train_layer_tail_workspace_bytes",
+                     "msda_amp_train_layer_tail_backward")
 
 _lib = None
 _amp_lib = None
 _train_lib = None
+_amp_train_lib = None
 
 
 class MsdaError(RuntimeError):
@@ -161,6 +168,35 @@ def train_lib():
         raise RuntimeError("libmsda_b200_train.so ABI %d != binding ABI %d; rebuild" %
                            (L.msda_train_abi_version(), MSDA_TRAIN_ABI_VERSION))
     _train_lib = L
+    return L
+
+
+def amp_train_lib():
+    """Load (once) and return the ctypes handle of libmsda_b200_amp_train.so; raise if it was not built."""
+    global _amp_train_lib
+    if _amp_train_lib is not None:
+        return _amp_train_lib
+    if not os.path.exists(AMP_TRAIN_LIB_PATH):
+        raise RuntimeError(
+            "libmsda_b200_amp_train.so is not built (%s). Build it with "
+            "`python -c 'import __graft_entry__ as g; g.build()'` or `python -m snipper_b200.build`. "
+            "There is no CPU / PyTorch fallback for this op." % AMP_TRAIN_LIB_PATH)
+    L = ctypes.CDLL(AMP_TRAIN_LIB_PATH)
+    vp, i32, i64, f32 = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_float
+    L.msda_amp_train_abi_version.restype = i32
+    L.msda_amp_train_abi_version.argtypes = []
+    L.msda_amp_train_last_cuda_error.restype = i32
+    L.msda_amp_train_last_cuda_error.argtypes = []
+    L.msda_amp_train_layer_tail_forward.restype = i32
+    L.msda_amp_train_layer_tail_forward.argtypes = [vp] * 3 + [i32, vp, f32] + [vp] * 8 + [i64, i32, f32, vp]
+    L.msda_amp_train_layer_tail_workspace_bytes.restype = ctypes.c_size_t
+    L.msda_amp_train_layer_tail_workspace_bytes.argtypes = [i64, i32]
+    L.msda_amp_train_layer_tail_backward.restype = i32
+    L.msda_amp_train_layer_tail_backward.argtypes = [vp] * 6 + [f32] + [vp] * 2 + [i32] + [vp] * 3 + [i64, i32, vp]
+    if L.msda_amp_train_abi_version() != MSDA_AMP_TRAIN_ABI_VERSION:
+        raise RuntimeError("libmsda_b200_amp_train.so ABI %d != binding ABI %d; rebuild" %
+                           (L.msda_amp_train_abi_version(), MSDA_AMP_TRAIN_ABI_VERSION))
+    _amp_train_lib = L
     return L
 
 

@@ -19,6 +19,7 @@
 #include <stdint.h>
 
 #include "../../include/msda_b200_amp.h"
+#include "msda_bf16_io.cuh"
 
 namespace msda {
 
@@ -34,23 +35,6 @@ __device__ __forceinline__ float warp_sum(float v)
 }
 
 __device__ __forceinline__ float4 load4(const float *p, int c4) { return __ldg(reinterpret_cast<const float4 *>(p) + c4); }
-
-__device__ __forceinline__ float4 load4(const __nv_bfloat16 *p, int c4)
-{
-    const uint2 u = __ldg(reinterpret_cast<const uint2 *>(p) + c4);
-    const float2 lo = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162 *>(&u.x));
-    const float2 hi = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162 *>(&u.y));
-    return make_float4(lo.x, lo.y, hi.x, hi.y);
-}
-
-__device__ __forceinline__ void store4_bf16(__nv_bfloat16 *p, int c4, float4 v)
-{
-    const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
-    uint2 u;
-    u.x = *reinterpret_cast<const uint32_t *>(&lo);
-    u.y = *reinterpret_cast<const uint32_t *>(&hi);
-    reinterpret_cast<uint2 *>(p)[c4] = u;
-}
 
 template <int VPL, typename Residual>
 __global__ void __launch_bounds__(256)

@@ -135,7 +135,7 @@ class Encoder(nn.Module):
         super().__init__()
         self.layers, self.num_layers = _clones(layer, n), n
         self.analytic_reference_points = False   # snipper_b200.enable_fused_layer_tails: closed form, computed in-kernel
-        self.analytic_reference_points_with_grad = False   # ... also while autograd records (training=True)
+        self.analytic_reference_points_with_grad = False   # ... also while autograd records (training / amp_training)
 
     @staticmethod
     def reference_points(sizes, valid_ratios, device):

@@ -15,7 +15,7 @@ loads) to a version that
     (get_reference_points, :219-232), so the fused kernels compute the reference points from the query index
     (SURVEY.md section 8f rank 2).
 
-``_eligible`` alone decides, per call, which of four forwards runs:
+``_eligible`` alone decides, per call, which of five forwards runs:
 
   * the layer's ORIGINAL forward (stock);
   * the fp32 tails (``layer_tail``), when autocast is off for CUDA and the residual stream is fp32 on CUDA with
@@ -31,7 +31,9 @@ loads) to a version that
     added in fp32 rather than in a bf16 GEMM epilogue, and the LayerNorm sums in another order), which is why it
     is opt-in per model.  Autocast to float16 keeps the stock layers.
   * the training tails (``layer_tail_train``, libmsda_b200_train.so), when the layer was switched with
-    ``enable_fused_layer_tails(model, training=True)`` and neither inference forward applies -- see below.
+    ``enable_fused_layer_tails(model, training=True)`` and neither inference forward applies -- see below;
+  * the bf16 autocast training tails (``layer_tail_amp_train``, libmsda_b200_amp_train.so), when the layer was switched
+    with ``enable_fused_layer_tails(model, amp_training=True)`` and neither inference forward applies -- see below.
 
 Both inference forwards further need all of these:
 
@@ -53,6 +55,15 @@ mask is drawn in eval mode or at p = 0.  The FFN's inner dropout and the decoder
 stock, and the FFN's first GEMM is ``relu(linear(x, w, b))`` (``_addmm_activation`` has no derivative).  The stock
 layers draw their masks from the same generator in another order and another dtype, so a step is not bit-identical
 to the stock one; it computes the same function of its masks (tests/test_layer_tails_train_gpu.py).
+
+The bf16 autocast training tails follow the same rules under ``torch.autocast("cuda", dtype=torch.bfloat16)``, with
+the amp tails' I/O: the residual stream is fp32 or bf16, the GEMM in front of each tail returns bf16, and each tail
+also writes, with exactly autocast's rounding, the bf16 copies the next GEMMs take (``linear1``'s input, the next
+encoder layer's ``value_proj`` input and query, the decoder's cross-attention query).  ``linear1`` runs as
+``relu(linear(x16, w, b))``, autocast casting w and b.  The gradient of the GEMM output is bf16, rounded once from
+fp32; the output_proj / linear2 bias gradient is summed from the fp32 values before that rounding, where stock autocast
+sums the bf16 GEMM-output gradient (tests/test_layer_tails_amp_train_gpu.py).  The new keyword is needed because
+``autocast=True, training=True`` keeps the stock layers in autocast training.  fp16 autocast keeps the stock layers.
 Works on the reference's own layer classes (after ``install_module()``) and on the bench harness' layers: both
 expose the reference's attribute names (self_attn / cross_attn, norm1..3, linear1/2, dropout1..4).
 """
@@ -79,12 +90,10 @@ def _affine_layer_norm(norm):
 
 def _eligible(layer, x, pos, *inputs):
     """Which forward computes what ``layer``'s own forward would (the module docstring lists the conditions):
-    None (the layer's own), "fp32", "amp" or "train".  ``x`` is the residual stream, ``pos`` the positional embedding
-    (``pos`` / ``query_pos``), ``inputs`` every other argument of the layer's forward."""
+    None (the layer's own), "fp32", "amp", "train" or "amp_train".  ``x`` is the residual stream, ``pos`` the positional
+    embedding (``pos`` / ``query_pos``), ``inputs`` every other argument of the layer's forward."""
     path = _inference_path(layer, x, pos, *inputs)
-    if path is None and _train_eligible(layer, x, pos):
-        return "train"
-    return path
+    return path if path is not None else _train_path(layer, x, pos)
 
 
 def _inference_path(layer, x, pos, *inputs):
@@ -117,13 +126,21 @@ def _fusable_structure(layer):
 _TAIL_DROPOUTS = {"encoder": ("dropout1", "dropout3"), "decoder": ("dropout2", "dropout1", "dropout4")}
 
 
-def _train_eligible(layer, x, pos):
-    if not getattr(layer, "_train_tails", False) or torch.is_autocast_enabled("cuda"):
-        return False
-    if not ops.layer_tail_train_supported(x, pos):
-        return False
+def _train_path(layer, x, pos):
+    """None, "train" or "amp_train": the training forwards' conditions."""
+    if torch.is_autocast_enabled("cuda"):
+        if not (getattr(layer, "_amp_train_tails", False) and torch.get_autocast_dtype("cuda") == torch.bfloat16 and
+                ops.layer_tail_amp_train_supported(x, pos)):
+            return None
+        path = "amp_train"
+    elif getattr(layer, "_train_tails", False) and ops.layer_tail_train_supported(x, pos):
+        path = "train"
+    else:
+        return None
     drops = [getattr(layer, n, None) for n in _TAIL_DROPOUTS["decoder" if hasattr(layer, "cross_attn") else "encoder"]]
-    return all(isinstance(d, nn.Dropout) and _dropout_p(d) < 1 for d in drops) and _fusable_structure(layer)
+    if not all(isinstance(d, nn.Dropout) and _dropout_p(d) < 1 for d in drops):
+        return None
+    return path if _fusable_structure(layer) else None
 
 
 def _dropout_p(dropout):
@@ -137,13 +154,19 @@ def draw_keep_mask(shape, p, device):
     return torch.empty(shape, dtype=torch.uint8, device=device).bernoulli_(1 - p)
 
 
-def _train_tail(y, bias, residual, dropout, norm, pos=None):
-    """norm(residual + dropout(y + bias)) and that + pos (None without ``pos``), both differentiable."""
+def _train_tail(y, bias, residual, dropout, norm, pos=None, amp=False, emit_bf16=False):
+    """_tail with ``dropout`` before the residual add, differentiable: -> (norm(residual + dropout(y + bias)) in fp32,
+    that in bf16 or None, that + pos or None).  ``amp``: y is a bf16 GEMM output; out + pos is then returned in bf16
+    and ``emit_bf16`` asks for the bf16 copy of out."""
     p = _dropout_p(dropout)
     mask = draw_keep_mask(y.shape, p, y.device) if p > 0 else None
+    if amp:
+        out, out16, out_pos, _, _ = torch.ops.snipper_b200.layer_tail_amp_train(
+            y, bias, residual, mask, float(p), norm.weight, norm.bias, pos, norm.eps, emit_bf16)
+        return out, (out16 if emit_bf16 else None), (out_pos if pos is not None else None)
     out, out_pos, _, _ = torch.ops.snipper_b200.layer_tail_train(y, bias, residual, mask, float(p), norm.weight,
                                                                  norm.bias, pos, norm.eps)
-    return out, (out_pos if pos is not None else None)
+    return out, None, (out_pos if pos is not None else None)
 
 
 def _tail(y, bias, residual, norm, pos=None, amp=False, emit_bf16=False):
@@ -184,8 +207,9 @@ def _encoder_forward(self, src, pos, reference_points, spatial_shapes, level_sta
     path = _eligible(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask)
     if path is None:
         return self._stock_forward(src, pos, reference_points, spatial_shapes, level_start_index, padding_mask)
-    if path == "train":
-        return _encoder_train_forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask)
+    if path in ("train", "amp_train"):
+        return _encoder_train_forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask,
+                                      amp=path == "amp_train")
     amp = path == "amp"
     attn = self.self_attn
     value_in = getattr(src, _AS_BF16, src) if amp else src                   # the previous amp tail's bf16 copy
@@ -212,9 +236,9 @@ def _decoder_forward(self, tgt, query_pos, reference_points, src, src_spatial_sh
     if path is None:
         return self._stock_forward(tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
                                    src_padding_mask)
-    if path == "train":
+    if path in ("train", "amp_train"):
         return _decoder_train_forward(self, tgt, query_pos, reference_points, src, src_spatial_shapes,
-                                      level_start_index, src_padding_mask)
+                                      level_start_index, src_padding_mask, amp=path == "amp_train")
     amp = path == "amp"
     bs, t, lq, c = tgt.shape
     x = tgt.reshape(bs, t * lq, c)
@@ -233,40 +257,49 @@ def _decoder_forward(self, tgt, query_pos, reference_points, src, src_spatial_sh
     return out, vis
 
 
-def _encoder_train_forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask):
-    """_encoder_forward's fp32 path with dropout and autograd: the tails apply dropout1 / dropout3."""
+def _encoder_train_forward(self, src, pos, reference_points, spatial_shapes, level_start_index, padding_mask,
+                           amp=False):
+    """_encoder_forward with dropout and autograd: the tails apply dropout1 / dropout3.  ``amp``: under bf16 autocast,
+    the tails hand their bf16 copies to linear1 and to the next layer, as on the amp inference path."""
     attn = self.self_attn
-    core, _ = attn._attend(_with_pos(src, pos, False), reference_points, src, spatial_shapes, level_start_index,
+    value_in = getattr(src, _AS_BF16, src) if amp else src                   # the previous amp tail's bf16 copy
+    core, _ = attn._attend(_with_pos(src, pos, amp), reference_points, value_in, spatial_shapes, level_start_index,
                            padding_mask)
     y = F.linear(core, attn.output_proj.weight)
-    x, _ = _train_tail(y, attn.output_proj.bias, src, self.dropout1, self.norm1)            # :204-205
-    hidden = F.relu(F.linear(x, self.linear1.weight, self.linear1.bias))
+    x, x16, _ = _train_tail(y, attn.output_proj.bias, src, self.dropout1, self.norm1, amp=amp,
+                            emit_bf16=amp)                                                    # :204-205
+    hidden = F.relu(F.linear(x16 if amp else x, self.linear1.weight, self.linear1.bias))
     ff = F.linear(self.dropout2(hidden), self.linear2.weight)                                 # :194
     emit = pos if (self._emit_next_query and pos is not None) else None
-    out, out_pos = _train_tail(ff, self.linear2.bias, x, self.dropout3, self.norm2, emit)   # :195-197 (+ :202)
+    out, out16, out_pos = _train_tail(ff, self.linear2.bias, x, self.dropout3, self.norm2, emit, amp=amp,
+                                      emit_bf16=amp and self._emit_next_query)              # :195-197 (+ :202)
     if out_pos is not None:
         setattr(out, _PLUS_POS, (pos, out_pos))
+    if out16 is not None:
+        setattr(out, _AS_BF16, out16)
     return out
 
 
 def _decoder_train_forward(self, tgt, query_pos, reference_points, src, src_spatial_shapes, level_start_index,
-                           src_padding_mask):
-    """_decoder_forward's fp32 path with dropout and autograd: the tails apply dropout2 / dropout1 / dropout4."""
+                           src_padding_mask, amp=False):
+    """_decoder_forward with dropout and autograd: the tails apply dropout2 / dropout1 / dropout4.  ``amp``: under bf16
+    autocast, the cross-attention query and linear1's input are the tails' bf16 copies."""
     bs, t, lq, c = tgt.shape
     x = tgt.reshape(bs, t * lq, c)
     qp = None if query_pos is None else query_pos.reshape(bs, t * lq, c)
     qk = (x if qp is None else x + qp).transpose(0, 1)
     sa = self.self_attn(qk, qk, x.transpose(0, 1))[0].transpose(0, 1)        # :285 (nn.MultiheadAttention, stock)
-    x, xq = _train_tail(sa, None, x, self.dropout2, self.norm2, qp)          # :286-287 (+ with_pos_embed of :292)
+    x, _, xq = _train_tail(sa, None, x, self.dropout2, self.norm2, qp, amp=amp)  # :286-287 (+ with_pos_embed of :292)
     q = (x if xq is None else xq).view(bs, t, lq, c)
     x = x.view(bs, t, lq, c)
     attn = self.cross_attn
     core, vis = attn._attend(q, reference_points, src, src_spatial_shapes, level_start_index, src_padding_mask)
     y = F.linear(core, attn.output_proj.weight)
-    x, _ = _train_tail(y, attn.output_proj.bias, x, self.dropout1, self.norm1)              # :294-295
-    hidden = F.relu(F.linear(x, self.linear1.weight, self.linear1.bias))
+    x, x16, _ = _train_tail(y, attn.output_proj.bias, x, self.dropout1, self.norm1, amp=amp,
+                            emit_bf16=amp)                                                    # :294-295
+    hidden = F.relu(F.linear(x16 if amp else x, self.linear1.weight, self.linear1.bias))
     ff = F.linear(self.dropout3(hidden), self.linear2.weight)                                 # :270
-    out, _ = _train_tail(ff, self.linear2.bias, x, self.dropout4, self.norm3)               # :271-273
+    out, _, _ = _train_tail(ff, self.linear2.bias, x, self.dropout4, self.norm3, amp=amp)    # :271-273
     return out, vis
 
 
@@ -306,11 +339,12 @@ def _is_decoder_layer(m):
             all(hasattr(m, a) for a in ("norm1", "norm2", "norm3", "linear1", "linear2")))
 
 
-def enable_fused_layer_tails(model, autocast=False, training=False):
+def enable_fused_layer_tails(model, autocast=False, training=False, amp_training=False):
     """Rebind ``forward`` of every deformable encoder / decoder layer under ``model`` (idempotent).
     ``autocast=True`` also lets the layers run their tails under bf16 autocast, ``training=True`` lets them run the
-    training tails while autograd records and dropouts are active (the module docstring says what each changes);
-    calling again with other values updates every switched layer.  Returns the number of layers newly switched.
+    training tails while autograd records and dropouts are active, ``amp_training=True`` the training tails under bf16
+    autocast (the module docstring says what each changes); calling again with other values updates every switched
+    layer.  Returns the number of layers newly switched.
     ``disable_fused_layer_tails`` undoes it."""
     n = 0
     for parent in model.modules():
@@ -323,6 +357,7 @@ def enable_fused_layer_tails(model, autocast=False, training=False):
                 continue
             layer._amp_tails = bool(autocast)
             layer._train_tails = bool(training)
+            layer._amp_train_tails = bool(amp_training)
             if hasattr(layer, "_stock_forward"):
                 continue
             layer._stock_forward = layer.forward
@@ -333,7 +368,7 @@ def enable_fused_layer_tails(model, autocast=False, training=False):
         if len(layers) and all(_is_encoder_layer(l) for l in layers) and not hasattr(parent, "_stock_forward"):
             if hasattr(parent, "analytic_reference_points"):          # the bench harness' encoder has a switch
                 parent.analytic_reference_points = True
-                parent.analytic_reference_points_with_grad = bool(training)
+                parent.analytic_reference_points_with_grad = bool(training or amp_training)
             elif hasattr(parent, "get_reference_points"):             # the reference's DeformableTransformerEncoder
                 parent._stock_forward = parent.forward
                 parent.forward = types.MethodType(_reference_encoder_forward, parent)
@@ -350,6 +385,6 @@ def disable_fused_layer_tails(model):
             del m.__dict__["forward"]
             del m.__dict__["_stock_forward"]
             n += _is_encoder_layer(m) or _is_decoder_layer(m)
-        for a in ("_amp_tails", "_train_tails", "_emit_next_query"):
+        for a in ("_amp_tails", "_train_tails", "_amp_train_tails", "_emit_next_query"):
             m.__dict__.pop(a, None)
     return n

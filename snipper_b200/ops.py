@@ -15,9 +15,11 @@ in the hand-written kernels.  Ops (namespace ``snipper_b200``):
                                         (libmsda_b200_amp.so, for bf16 autocast)
   layer_tail_train / _backward          bias + dropout (by a given keep-mask) + residual + LayerNorm (+ pos) and its
                                         backward, for training (libmsda_b200_train.so)
+  layer_tail_amp_train / _backward      the same on a bf16 GEMM output, also writing the next GEMMs' bf16 inputs, for
+                                        training under bf16 autocast (libmsda_b200_amp_train.so)
 
-The four forwards (msda_forward, snippet_forward, snippet_attn, layer_tail_train) carry ``register_autograd`` formulas, so they
-compose with autograd / DDP as plain nodes (no host sync, no unused parameters).
+The five forwards (msda_forward, snippet_forward, snippet_attn, layer_tail_train, layer_tail_amp_train) carry
+``register_autograd`` formulas, so they compose with autograd / DDP as plain nodes (no host sync, no unused parameters).
 """
 from typing import Optional, Tuple
 
@@ -82,10 +84,12 @@ STATS = LaunchStats()
 
 def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None, im2col_step=None, amp=False,
             train=False):
-    """Call the C entry point ``entry`` (of libmsda_b200_amp.so when ``amp``, of libmsda_b200_train.so when ``train``)
-    with ``args`` and ``device``'s current stream (every launching entry point takes the stream last), count its
-    ``n_kernels`` kernels in STATS under ``tag`` / ``dims`` and raise on a failed status."""
-    lib = capi.amp_lib() if amp else capi.train_lib() if train else capi.lib()
+    """Call the C entry point ``entry`` (of libmsda_b200_amp.so when ``amp``, of libmsda_b200_train.so when ``train``,
+    of libmsda_b200_amp_train.so when both) with ``args`` and ``device``'s current stream (every launching entry point
+    takes the stream last), count its ``n_kernels`` kernels in STATS under ``tag`` / ``dims`` and raise on a failed
+    status."""
+    lib = (capi.amp_train_lib() if amp and train else capi.amp_lib() if amp else capi.train_lib() if train
+           else capi.lib())
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device)
         if STATS.timing:
@@ -96,7 +100,8 @@ def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None,
         if STATS.timing:
             end.record(stream)
             STATS.events.append((tag, dims, start, end))
-    last_error = lib.msda_amp_last_cuda_error if amp else lib.msda_train_last_cuda_error if train else None
+    last_error = (lib.msda_amp_train_last_cuda_error if amp and train else lib.msda_amp_last_cuda_error if amp
+                  else lib.msda_train_last_cuda_error if train else None)
     capi.check(status, what or entry, batch, im2col_step, last_error)
 
 
@@ -965,3 +970,145 @@ def _tail_train_backward_formula(ctx, grad_out, grad_out_pos, grad_h, grad_mean_
 
 
 layer_tail_train.register_autograd(_tail_train_backward_formula, setup_context=_tail_train_setup_context)
+
+
+# ------------------------------------------------------------------------------------------
+# layer tail for training under bf16 autocast (libmsda_b200_amp_train.so): layer_tail_train's dropout, saved h and
+# (mean, rstd) and ordered parameter-gradient sum, with layer_tail_amp's bf16 GEMM output in and bf16 copies out
+# ------------------------------------------------------------------------------------------
+def layer_tail_amp_train_supported(residual: Tensor, pos: Optional[Tensor] = None) -> bool:
+    """fp32 or bf16 CUDA residual rows of 128*k <= 1024 channels, ``pos`` absent or fp32 shaped like them.  Autograd
+    may record (the op has a gradient formula); the GEMM output the op adds is bf16 rows of the same shape."""
+    C = residual.shape[-1]
+    return (residual.is_cuda and residual.dtype in (torch.float32, torch.bfloat16) and C % 128 == 0 and C <= 1024 and
+            (pos is None or (pos.dtype == torch.float32 and pos.shape == residual.shape)))
+
+
+@torch.library.custom_op("snipper_b200::layer_tail_amp_train", mutates_args=())
+def layer_tail_amp_train(y: Tensor, bias: Optional[Tensor], residual: Tensor, keep_mask: Optional[Tensor], p: float,
+                         gamma: Tensor, beta: Tensor, pos: Optional[Tensor], eps: float, emit_bf16: bool
+                         ) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """(out, out_bf16, out_pos_bf16, h, mean_rstd): ``layer_tail_train`` on y.float(), residual.float() -- out, h and
+    mean_rstd have its bits -- with out_bf16 = out rounded to bf16 (empty unless ``emit_bf16``) and out_pos_bf16 =
+    (out + pos) rounded to bf16 (empty when ``pos`` is None).  y is bf16, residual fp32 or bf16, bias / gamma / beta /
+    pos fp32."""
+    _require_cuda(y, "y")
+    C = y.shape[-1]
+    if (y.dtype != torch.bfloat16 or residual.dtype not in (torch.float32, torch.bfloat16) or C % 128 != 0 or
+            C > 1024 or residual.shape != y.shape):
+        raise RuntimeError("layer_tail_amp_train: bfloat16 rows of 128*k <= 1024 channels, residual float32 / "
+                           "bfloat16 shaped like y")
+    keep_mask = _check_train_mask(keep_mask, y, p)
+    y, residual = _dense16(y), _dense16(residual)
+    for t in (bias, gamma, beta):
+        if t is not None and (t.numel() != C or t.dtype != torch.float32 or not t.is_contiguous()):
+            raise RuntimeError("layer_tail_amp_train: bias / gamma / beta must be contiguous float32 vectors of C "
+                               "elements")
+    # locals: an aligned copy must stay alive until the kernel that reads it has been enqueued
+    bias = _dense16(bias) if bias is not None else None
+    gamma, beta = _dense16(gamma), _dense16(beta)
+    rows = y.numel() // C
+    out = torch.empty(y.shape, dtype=torch.float32, device=y.device)
+    h = torch.empty_like(out)
+    mean_rstd = out.new_empty((*y.shape[:-1], 2))
+    out_bf16 = torch.empty_like(y) if emit_bf16 else y.new_empty((0,))
+    if pos is not None:
+        if pos.shape != y.shape or pos.dtype != torch.float32:
+            raise RuntimeError("layer_tail_amp_train: pos must be float32 shaped like y")
+        pos = _dense16(pos)
+        out_pos = torch.empty_like(y)
+    else:
+        out_pos = y.new_empty((0,))
+    _launch("msda_amp_train_layer_tail_forward", "layer_tail_amp_train",
+            (rows, C, residual.element_size(), int(keep_mask is not None), int(emit_bf16), int(pos is not None)),
+            y.device, y.data_ptr(), _ptr(bias), residual.data_ptr(), _DTYPES[residual.dtype], _ptr(keep_mask),
+            keep_scale(p) if keep_mask is not None else 1.0, gamma.data_ptr(), beta.data_ptr(), _ptr(pos),
+            out.data_ptr(), out_bf16.data_ptr() if emit_bf16 else None,
+            out_pos.data_ptr() if pos is not None else None, h.data_ptr(), mean_rstd.data_ptr(), rows, C, float(eps),
+            amp=True, train=True)
+    return out, out_bf16, out_pos, h, mean_rstd
+
+
+@layer_tail_amp_train.register_fake
+def _(y, bias, residual, keep_mask, p, gamma, beta, pos, eps, emit_bf16):
+    out = torch.empty(y.shape, dtype=torch.float32, device=y.device)
+    return (out, torch.empty_like(y) if emit_bf16 else y.new_empty((0,)),
+            torch.empty_like(y) if pos is not None else y.new_empty((0,)), torch.empty_like(out),
+            out.new_empty((*y.shape[:-1], 2)))
+
+
+@torch.library.custom_op("snipper_b200::layer_tail_amp_train_backward", mutates_args=())
+def layer_tail_amp_train_backward(grad_out: Tensor, grad_out_bf16: Optional[Tensor], grad_out_pos_bf16: Optional[Tensor],
+                                  h: Tensor, mean_rstd: Tensor, keep_mask: Optional[Tensor], p: float, gamma: Tensor,
+                                  residual_bf16: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """(grad_residual, grad_y, param_grads) of ``layer_tail_amp_train`` for the incoming gradients grad_out (fp32) and
+    the optional bf16 grad_out_bf16 / grad_out_pos_bf16 of its bf16 copies, added as (grad_out + grad_out_bf16) +
+    grad_out_pos_bf16 in fp32.  grad_residual is bf16 when ``residual_bf16`` (else fp32) and grad_y bf16, each rounded
+    once from fp32; param_grads is (3, C) fp32 = (grad_gamma, grad_beta, grad_bias), with grad_bias summed from the fp32
+    grad_y, reduced in a fixed order without atomics."""
+    _require_cuda(h, "h")
+    C = h.shape[-1]
+    if (h.dtype != torch.float32 or C % 128 != 0 or C > 1024 or grad_out.shape != h.shape or
+            grad_out.dtype != torch.float32 or mean_rstd.shape != (*h.shape[:-1], 2) or
+            any(g is not None and (g.shape != h.shape or g.dtype != torch.bfloat16)
+                for g in (grad_out_bf16, grad_out_pos_bf16))):
+        raise RuntimeError("layer_tail_amp_train_backward: float32 rows of 128*k <= 1024 channels, grad_out float32 "
+                           "and the optional bf16 gradients shaped like h, mean_rstd (..., 2)")
+    if gamma.numel() != C or gamma.dtype != torch.float32:
+        raise RuntimeError("layer_tail_amp_train_backward: gamma must be a float32 vector of C elements")
+    keep_mask = _check_train_mask(keep_mask, h, p)
+    rows = h.numel() // C
+    grad_out, h, mean_rstd, gamma = _dense16(grad_out), _dense16(h), _dense16(mean_rstd), _dense16(gamma)
+    grad_out_bf16 = _dense16(grad_out_bf16) if grad_out_bf16 is not None else None
+    grad_out_pos_bf16 = _dense16(grad_out_pos_bf16) if grad_out_pos_bf16 is not None else None
+    rdt = torch.bfloat16 if residual_bf16 else torch.float32
+    grad_residual = torch.empty(h.shape, dtype=rdt, device=h.device)
+    grad_y = torch.empty(h.shape, dtype=torch.bfloat16, device=h.device)
+    param_grads = torch.zeros((3, C), dtype=torch.float32, device=h.device) if rows == 0 else \
+        torch.empty((3, C), dtype=torch.float32, device=h.device)
+    ws_bytes = capi.amp_train_lib().msda_amp_train_layer_tail_workspace_bytes(rows, C)
+    ws = torch.empty(max(ws_bytes // 4, 1), dtype=torch.float32, device=h.device)
+    _launch("msda_amp_train_layer_tail_backward", "layer_tail_amp_train_backward",
+            (rows, C, grad_residual.element_size(), int(keep_mask is not None), int(grad_out_bf16 is not None),
+             int(grad_out_pos_bf16 is not None)), h.device,
+            grad_out.data_ptr(), _ptr(grad_out_bf16), _ptr(grad_out_pos_bf16), h.data_ptr(), mean_rstd.data_ptr(),
+            _ptr(keep_mask), keep_scale(p) if keep_mask is not None else 1.0, gamma.data_ptr(),
+            grad_residual.data_ptr(), _DTYPES[rdt], grad_y.data_ptr(), param_grads.data_ptr(), ws.data_ptr(), rows, C,
+            n_kernels=2, amp=True, train=True)
+    return grad_residual, grad_y, param_grads
+
+
+@layer_tail_amp_train_backward.register_fake
+def _(grad_out, grad_out_bf16, grad_out_pos_bf16, h, mean_rstd, keep_mask, p, gamma, residual_bf16):
+    return (torch.empty(h.shape, dtype=torch.bfloat16 if residual_bf16 else torch.float32, device=h.device),
+            torch.empty(h.shape, dtype=torch.bfloat16, device=h.device), h.new_empty((3, h.shape[-1])))
+
+
+def _tail_amp_train_setup_context(ctx, inputs, output):
+    y, bias, residual, keep_mask, p, gamma, beta, pos, eps, emit_bf16 = inputs
+    out, out_bf16, out_pos, h, mean_rstd = output
+    ctx.p, ctx.has_bias, ctx.has_pos, ctx.emit_bf16 = p, bias is not None, pos is not None, emit_bf16
+    ctx.residual_bf16 = residual.dtype == torch.bfloat16
+    # what stock autocast saves for the same block: dropout its mask, layer_norm its fp32 input and (mean, rstd)
+    ctx.save_for_backward(h, mean_rstd, keep_mask, gamma)
+    ctx.set_materialize_grads(False)
+
+
+def _tail_amp_train_backward_formula(ctx, grad_out, grad_out_bf16, grad_out_pos, grad_h, grad_mean_rstd):
+    h, mean_rstd, keep_mask, gamma = ctx.saved_tensors
+    if not ctx.emit_bf16:
+        grad_out_bf16 = None
+    if not ctx.has_pos:
+        grad_out_pos = None
+    if grad_out is None and grad_out_bf16 is None and grad_out_pos is None:
+        return (None,) * 10
+    if grad_out is None:
+        grad_out = torch.zeros_like(h)
+    grad_residual, grad_y, pg = torch.ops.snipper_b200.layer_tail_amp_train_backward(
+        grad_out, grad_out_bf16, grad_out_pos, h, mean_rstd, keep_mask, ctx.p, gamma, ctx.residual_bf16)
+    # out_pos_bf16 = bf16(out + pos): pos gets the gradient of that copy, in pos's dtype
+    grad_pos = grad_out_pos.float() if (grad_out_pos is not None and ctx.needs_input_grad[7]) else None
+    return (grad_y, pg[2] if ctx.has_bias else None, grad_residual, None, None, pg[0], pg[1], grad_pos, None, None)
+
+
+layer_tail_amp_train.register_autograd(_tail_amp_train_backward_formula, setup_context=_tail_amp_train_setup_context)

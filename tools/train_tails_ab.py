@@ -1,12 +1,14 @@
 """A/B of the layer tails in training: the tools/trainbench.py step with the stock layers against
-``enable_fused_layer_tails(model, training=True)`` (``layer_tail_train``), eager, one process.
+``enable_fused_layer_tails(model, training=True)`` (``layer_tail_train``), eager, one process.  With ``--bf16`` both
+arms run under torch.autocast("cuda", dtype=torch.bfloat16) and the fused arm is
+``enable_fused_layer_tails(model, amp_training=True)`` (``layer_tail_amp_train``).
 
-    python tools/train_tails_ab.py --out DIR [--rounds 6] [--steps 5] [--warmup 3] [--profile-steps 2]
+    python tools/train_tails_ab.py --out DIR [--bf16] [--rounds 6] [--steps 5] [--warmup 3] [--profile-steps 2]
 
 The step is trainbench.py's: forward, synthetic loss over every head, backward, clip_grad_norm_(0.1), AdamW; batch 2,
 T = 4, 600x800, dropout 0.1, fp32.  Both arms are ONE model whose tails are switched on and off; they are timed
 alternately (``--rounds`` blocks of ``--steps`` steps each, the arm order flipped every round).  Writes
-DIR/train_tails_ab.json:
+DIR/train_tails_ab.json (DIR/train_tails_ab_bf16.json with ``--bf16``):
 
   * ms per step of each arm: median over the rounds, min, max, and the median / min / max of the per-round
     fused - stock differences;
@@ -45,6 +47,20 @@ def bwd_bytes(dims):
     return rows * C * (4 + 4 * pos + 4 + mask + 4 + 4) + 8 * rows + 4 * C
 
 
+def amp_fwd_bytes(dims):
+    """bf16 forward launch: read y (bf16), residual (fp32 or bf16) (+ mask) (+ pos, fp32), write out, h, (mean, rstd)
+    (+ the bf16 copy of out) (+ the bf16 out + pos), plus bias / gamma / beta."""
+    rows, C, res_bytes, mask, emit, pos = dims
+    return rows * C * (2 + res_bytes + mask + 4 + 4 + 2 * emit + 6 * pos) + 8 * rows + 3 * 4 * C
+
+
+def amp_bwd_bytes(dims):
+    """bf16 backward launch pair: read grad_out (+ the bf16 gradients of the copies), h (+ mask), (mean, rstd); write
+    grad_residual (fp32 or bf16), grad_y (bf16).  The CTA partials are left out."""
+    rows, C, res_bytes, mask, b16, pos = dims
+    return rows * C * (4 + 2 * b16 + 2 * pos + 4 + mask + res_bytes + 2) + 8 * rows + 4 * C
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True, help="output directory for train_tails_ab.json")
@@ -53,6 +69,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=3, help="untimed steps per arm before the first round")
     ap.add_argument("--profile-steps", type=int, default=2)
     ap.add_argument("--batch", type=int, default=2)
+    ap.add_argument("--bf16", action="store_true", help="both arms under bf16 autocast, the fused arm amp_training=True")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "train_tails_ab.py needs a CUDA device"
     dev = torch.device("cuda", 0)
@@ -68,8 +85,9 @@ def main():
     xs = [torch.rand(args.batch, 12, 600, 800, generator=g).to(dev) for _ in range(2)]
 
     def step(i):
-        out, _ = model(xs[i % len(xs)])
-        loss = synthetic_loss(out)
+        with torch.autocast("cuda", dtype=torch.bfloat16, enabled=args.bf16):
+            out, _ = model(xs[i % len(xs)])
+            loss = synthetic_loss(out)
         opt.zero_grad(set_to_none=True)
         loss.backward()
         torch.nn.utils.clip_grad_norm_(params, 0.1)
@@ -77,10 +95,13 @@ def main():
 
     def set_arm(fused):
         if fused:
-            return snipper_b200.enable_fused_layer_tails(model, training=True)
+            return snipper_b200.enable_fused_layer_tails(model, **({"amp_training": True} if args.bf16 else
+                                                                   {"training": True}))
         return snipper_b200.disable_fused_layer_tails(model)
 
-    arms = {"stock": dict(fused=False, ms=[]), "train_tails": dict(fused=True, ms=[])}
+    fused_arm = "amp_train_tails" if args.bf16 else "train_tails"
+    fwd_tag = "layer_tail_amp_train" if args.bf16 else "layer_tail_train"
+    arms = {"stock": dict(fused=False, ms=[]), fused_arm: dict(fused=True, ms=[])}
     order = list(arms)
     for name in order:                                           # warm-up, launch counts and peak memory per arm
         set_arm(arms[name]["fused"])
@@ -125,10 +146,10 @@ def main():
             step(i)
         torch.cuda.synchronize()
     ops.STATS.timing = False
-    fwd_dims = [e[1] for e in ops.STATS.events if e[0] == "layer_tail_train"]
-    bwd_dims = [e[1] for e in ops.STATS.events if e[0] == "layer_tail_train_backward"]
+    fwd_dims = [e[1] for e in ops.STATS.events if e[0] == fwd_tag]
+    bwd_dims = [e[1] for e in ops.STATS.events if e[0] == fwd_tag + "_backward"]
     evs = sorted((ev for ev in prof.events() if ev.device_type.name == "CUDA" and
-                  ("layer_tail_train_fwd_kernel" in ev.name or "layer_tail_train_bwd_kernel" in ev.name or
+                  (fwd_tag + "_fwd_kernel" in ev.name or fwd_tag + "_bwd_kernel" in ev.name or
                    "layer_tail_param_sum_kernel" in ev.name)), key=lambda ev: ev.time_range.start)
     fwd_us = [ev.time_range.elapsed_us() for ev in evs if "fwd_kernel" in ev.name]
     bwd_us = [ev.time_range.elapsed_us() for ev in evs if "bwd_kernel" in ev.name]
@@ -144,16 +165,24 @@ def main():
         rows = []
         for d, ts in sorted(per.items()):
             med = statistics.median(ts)
-            rows.append({"rows": d[0], "C": d[1], "mask": d[2], "pos": d[3], "launches": len(ts), "us_median": med,
-                         "us_min": min(ts), "bytes": nbytes(d), "GB_per_s": nbytes(d) / med / 1e3, "kernel": what})
+            rows.append({**dict(zip(dim_names, d)), "launches": len(ts), "us_median": med, "us_min": min(ts),
+                         "bytes": nbytes(d), "GB_per_s": nbytes(d) / med / 1e3, "kernel": what})
         return rows
 
-    forward = by_dims(fwd_dims, fwd_us, fwd_bytes, "layer_tail_train_fwd_kernel")
-    backward = by_dims(bwd_dims, bwd_us, bwd_bytes, "layer_tail_train_bwd_kernel (without the parameter sum)")
+    if args.bf16:
+        dim_names = ("rows", "C", "residual_bytes", "mask", "bf16_copy", "pos")
+        forward = by_dims(fwd_dims, fwd_us, amp_fwd_bytes, fwd_tag + "_fwd_kernel")
+        dim_names = ("rows", "C", "grad_residual_bytes", "mask", "bf16_grad", "pos_grad")
+        backward = by_dims(bwd_dims, bwd_us, amp_bwd_bytes, fwd_tag + "_bwd_kernel (without the parameter sum)")
+    else:
+        dim_names = ("rows", "C", "mask", "pos")
+        forward = by_dims(fwd_dims, fwd_us, fwd_bytes, "layer_tail_train_fwd_kernel")
+        backward = by_dims(bwd_dims, bwd_us, bwd_bytes, "layer_tail_train_bwd_kernel (without the parameter sum)")
 
     result = {"gpu": gpu_info(0), "torch": torch.__version__,
               "step": "tools/trainbench.py step: forward, synthetic loss, backward, clip_grad_norm_(0.1), AdamW; "
-                      "batch %d, T = 4, 600x800, dropout 0.1, fp32 (torch default TF32 settings)" % args.batch,
+                      "batch %d, T = 4, 600x800, dropout 0.1, %s" % (
+                          args.batch, "bf16 autocast" if args.bf16 else "fp32 (torch default TF32 settings)"),
               "rounds": args.rounds, "steps_per_round": args.steps, "warmup": args.warmup, "arms": {},
               "train_tail_profile": {"forward_launches_per_step": len(fwd_dims) // args.profile_steps,
                                      "backward_launches_per_step": len(bwd_dims) // args.profile_steps,
@@ -168,14 +197,14 @@ def main():
                                 "ms_max": max(a["ms"]), "ms_per_round": a["ms"],
                                 "snippets_per_s": args.batch * 1e3 / statistics.median(a["ms"]),
                                 "peak_memory_bytes": a["peak_bytes"], "launches_per_step": a["launches_per_step"]}
-    diffs = [b - a for a, b in zip(arms["stock"]["ms"], arms["train_tails"]["ms"])]
-    result["train_tails_minus_stock_ms"] = {"median": statistics.median(diffs), "min": min(diffs), "max": max(diffs)}
+    diffs = [b - a for a, b in zip(arms["stock"]["ms"], arms[fused_arm]["ms"])]
+    result[fused_arm + "_minus_stock_ms"] = {"median": statistics.median(diffs), "min": min(diffs), "max": max(diffs)}
     os.makedirs(args.out, exist_ok=True)
-    path = os.path.join(args.out, "train_tails_ab.json")
+    path = os.path.join(args.out, "train_tails_ab_bf16.json" if args.bf16 else "train_tails_ab.json")
     with open(path, "w") as f:
         json.dump(result, f, indent=1)
     summary = {k: result["arms"][k]["ms_per_step_median"] for k in order}
-    print(json.dumps({"ms_per_step": summary, "train_tails_minus_stock_ms": result["train_tails_minus_stock_ms"],
+    print(json.dumps({"ms_per_step": summary, fused_arm + "_minus_stock_ms": result[fused_arm + "_minus_stock_ms"],
                       "peak_bytes": {k: result["arms"][k]["peak_memory_bytes"] for k in order},
                       "gpu": result["gpu"], "json": path}))
 
