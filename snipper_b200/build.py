@@ -2,11 +2,12 @@
 models/ops/setup.py + make.sh torch CUDAExtension build).  No torch headers are involved:
 the library is plain CUDA behind a C ABI (include/msda_b200.h).
 
-``build_all`` also builds, with the same flags, the three companion libraries: libmsda_b200_amp.so (csrc_amp/,
+``build_all`` also builds, with the same flags, the companion libraries: libmsda_b200_amp.so (csrc_amp/,
 include/msda_b200_amp.h), the mixed-precision layer tail used under bf16 autocast; libmsda_b200_train.so
 (csrc_train/, include/msda_b200_train.h), the layer tail with dropout and its backward used in training; and
 libmsda_b200_amp_train.so (csrc_amp_train/, include/msda_b200_amp_train.h), the same pair for training under bf16
-autocast."""
+autocast.  A fifth, libmsda_b200_f16.so (csrc_f16/, include/msda_b200_f16.h), is the attention op with float16 storage
+for torch.autocast's default dtype; it instantiates the kernel templates of csrc/ for fp16 lanes."""
 import os
 import shutil
 import subprocess
@@ -16,7 +17,8 @@ CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.path.join(PKG, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200.so")
 SOURCES = ["msda_capi.cu", "msda_percall.cu", "msda_snippet.cu", "msda_deterministic.cu", "msda_mask.cu", "msda_frames.cu", "msda_tail.cu", "msda_planar.cu"]
-HEADERS = ["msda_common.cuh", "msda_fast.cuh", "msda_snippet_common.cuh", "msda_internal.h", os.path.join("..", "..", "include", "msda_b200.h")]
+HEADERS = ["msda_common.cuh", "msda_fast.cuh", "msda_snippet_common.cuh", "msda_internal.h", "msda_percall.cuh",
+           "msda_snippet.cuh", "msda_frames.cuh", "msda_validate.h", os.path.join("..", "..", "include", "msda_b200.h")]
 OBJ_DIR = os.path.join(PKG, "lib", "obj")
 AMP_CSRC = os.path.join(PKG, "csrc_amp")
 AMP_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_amp.so")
@@ -31,6 +33,11 @@ AMP_TRAIN_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_amp_train.so")
 AMP_TRAIN_SOURCES = ["msda_amp_train_tail.cu"]
 AMP_TRAIN_HEADERS = [os.path.join("..", "csrc_train", "msda_train_common.cuh"), os.path.join("..", "csrc_amp", "msda_bf16_io.cuh"),
                      os.path.join("..", "..", "include", "msda_b200_amp_train.h"), os.path.join("..", "..", "include", "msda_b200.h")]
+F16_CSRC = os.path.join(PKG, "csrc_f16")
+F16_LIB_PATH = os.path.join(LIB_DIR, "libmsda_b200_f16.so")
+F16_SOURCES = ["msda_f16_capi.cu", "msda_f16_percall.cu", "msda_f16_snippet.cu", "msda_f16_frames.cu"]
+F16_HEADERS = [os.path.join("..", "csrc", h) for h in HEADERS[:-1]] + [
+    os.path.join("..", "..", "include", "msda_b200_f16.h"), os.path.join("..", "..", "include", "msda_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
@@ -99,10 +106,15 @@ def build_amp_train_library(force=False, verbose=False, extra_flags=()):
     return _build(AMP_TRAIN_LIB_PATH, AMP_TRAIN_CSRC, AMP_TRAIN_SOURCES, AMP_TRAIN_HEADERS, force, verbose, extra_flags)
 
 
+def build_f16_library(force=False, verbose=False, extra_flags=()):
+    """Compile csrc_f16/ into snipper_b200/lib/libmsda_b200_f16.so."""
+    return _build(F16_LIB_PATH, F16_CSRC, F16_SOURCES, F16_HEADERS, force, verbose, extra_flags)
+
+
 def build_all(force=False, verbose=False):
-    """-> (LIB_PATH, AMP_LIB_PATH, TRAIN_LIB_PATH, AMP_TRAIN_LIB_PATH), all four built."""
+    """-> (LIB_PATH, AMP_LIB_PATH, TRAIN_LIB_PATH, AMP_TRAIN_LIB_PATH, F16_LIB_PATH), all five built."""
     return (build_library(force, verbose), build_amp_library(force, verbose), build_train_library(force, verbose),
-            build_amp_train_library(force, verbose))
+            build_amp_train_library(force, verbose), build_f16_library(force, verbose))
 
 
 if __name__ == "__main__":

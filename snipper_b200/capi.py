@@ -1,7 +1,8 @@
 """ctypes binding of libmsda_b200.so (include/msda_b200.h) and of its companions: the mixed-precision
 libmsda_b200_amp.so (include/msda_b200_amp.h), the training library libmsda_b200_train.so
-(include/msda_b200_train.h) and the bf16-autocast training library libmsda_b200_amp_train.so
-(include/msda_b200_amp_train.h).
+(include/msda_b200_train.h), the bf16-autocast training library libmsda_b200_amp_train.so
+(include/msda_b200_amp_train.h) and the float16-storage attention library libmsda_b200_f16.so
+(include/msda_b200_f16.h).
 
 This is the ONLY way the package reaches compute: there is no CPU fallback and no alternate
 backend.  If a library is missing, its callers fail loudly.
@@ -9,12 +10,13 @@ backend.  If a library is missing, its callers fail loudly.
 import ctypes
 import os
 
-from .build import AMP_LIB_PATH, AMP_TRAIN_LIB_PATH, LIB_PATH, TRAIN_LIB_PATH
+from .build import AMP_LIB_PATH, AMP_TRAIN_LIB_PATH, F16_LIB_PATH, LIB_PATH, TRAIN_LIB_PATH
 
 MSDA_ABI_VERSION = 4
 MSDA_AMP_ABI_VERSION = 1
 MSDA_TRAIN_ABI_VERSION = 1
 MSDA_AMP_TRAIN_ABI_VERSION = 1
+MSDA_F16_ABI_VERSION = 1
 
 MSDA_OK = 0
 MSDA_ERR_INVALID_ARGUMENT = 1
@@ -49,11 +51,15 @@ TRAIN_EXPORTS = ("msda_train_abi_version", "msda_train_last_cuda_error", "msda_t
 AMP_TRAIN_EXPORTS = ("msda_amp_train_abi_version", "msda_amp_train_last_cuda_error",
                      "msda_amp_train_layer_tail_forward", "msda_amp_train_layer_tail_workspace_bytes",
                      "msda_amp_train_layer_tail_backward")
+# every symbol include/msda_b200_f16.h declares
+F16_EXPORTS = ("msda_f16_abi_version", "msda_f16_last_cuda_error", "msda_f16_forward", "msda_f16_backward",
+               "msda_f16_snippet_forward", "msda_f16_snippet_backward", "msda_f16_frame_sum", "msda_f16_frame_unsum")
 
 _lib = None
 _amp_lib = None
 _train_lib = None
 _amp_train_lib = None
+_f16_lib = None
 
 
 class MsdaError(RuntimeError):
@@ -197,6 +203,42 @@ def amp_train_lib():
         raise RuntimeError("libmsda_b200_amp_train.so ABI %d != binding ABI %d; rebuild" %
                            (L.msda_amp_train_abi_version(), MSDA_AMP_TRAIN_ABI_VERSION))
     _amp_train_lib = L
+    return L
+
+
+def f16_lib():
+    """Load (once) and return the ctypes handle of libmsda_b200_f16.so; raise if it was not built."""
+    global _f16_lib
+    if _f16_lib is not None:
+        return _f16_lib
+    if not os.path.exists(F16_LIB_PATH):
+        raise RuntimeError(
+            "libmsda_b200_f16.so is not built (%s). Build it with "
+            "`python -c 'import __graft_entry__ as g; g.build()'` or `python -m snipper_b200.build`. "
+            "There is no CPU / PyTorch fallback for this op." % F16_LIB_PATH)
+    L = ctypes.CDLL(F16_LIB_PATH)
+    vp, i32, i64, u32 = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_uint
+    L.msda_f16_abi_version.restype = i32
+    L.msda_f16_abi_version.argtypes = []
+    L.msda_f16_last_cuda_error.restype = i32
+    L.msda_f16_last_cuda_error.argtypes = []
+    # the argument lists of the msda_* twins without dtype (and without the deterministic workspace)
+    L.msda_f16_forward.restype = i32
+    L.msda_f16_forward.argtypes = [vp] * 6 + [i32] * 7 + [i64, i32, vp]
+    L.msda_f16_backward.restype = i32
+    L.msda_f16_backward.argtypes = [vp] * 9 + [i32] * 7 + [i64, i32, u32, vp]
+    L.msda_f16_snippet_forward.restype = i32
+    L.msda_f16_snippet_forward.argtypes = [vp] * 7 + [i32] * 10 + [i64] * 6 + [vp, vp, vp, vp, i64, i32, u32, vp]
+    L.msda_f16_snippet_backward.restype = i32
+    L.msda_f16_snippet_backward.argtypes = [vp] * 10 + [i32] * 10 + [i64] * 6 + [vp, vp, vp, vp, i64, i32, u32, vp]
+    L.msda_f16_frame_sum.restype = i32
+    L.msda_f16_frame_sum.argtypes = [vp, vp, vp] + [i32] * 6 + [i64, i64, i64, i32, vp]
+    L.msda_f16_frame_unsum.restype = i32
+    L.msda_f16_frame_unsum.argtypes = [vp, vp, vp] + [i32] * 6 + [i64, i32, vp]
+    if L.msda_f16_abi_version() != MSDA_F16_ABI_VERSION:
+        raise RuntimeError("libmsda_b200_f16.so ABI %d != binding ABI %d; rebuild" %
+                           (L.msda_f16_abi_version(), MSDA_F16_ABI_VERSION))
+    _f16_lib = L
     return L
 
 

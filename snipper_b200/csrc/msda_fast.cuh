@@ -22,6 +22,7 @@
 #pragma once
 
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "msda_common.cuh"
@@ -78,6 +79,7 @@ __device__ __forceinline__ int cell_stride_bytes(int runtime_csb) { return CSB >
 // 16-byte channel chunk of the value / output / grad_output element type VT, widened to fp32:
 //   float          4 channels  (LDG.E.128 -> 4 registers used as they are)
 //   __nv_bfloat16  8 channels  (LDG.E.128 -> 4 registers, each split with one shift / one mask)
+//   __half         8 channels  (LDG.E.128 -> 4 registers, each widened by two half -> float conversions)
 // All arithmetic is fp32 whatever VT is.
 // ------------------------------------------------------------------------------------------
 template <typename VT> struct Chunk;
@@ -156,6 +158,63 @@ template <> struct Chunk<bf16q> {
     }
 };
 
+// fp16 twins of the two bf16 lane types (libmsda_b200_f16.so): same lanes, same bytes, only the widening and the
+// rounding differ -- one conversion per channel on load (as the bf16 shift / mask), one packing conversion per two
+// channels on store, round to nearest even with overflow to +-inf.
+__device__ __forceinline__ float2 widen_half2(unsigned w) { return __half22float2(*reinterpret_cast<const __half2 *>(&w)); }
+
+__device__ __forceinline__ unsigned narrow_half2(float a, float b)
+{
+    const __half2 t = __floats2half2_rn(a, b);
+    return *reinterpret_cast<const unsigned *>(&t);
+}
+
+template <> struct Chunk<__half> {
+    using elem = __half;
+    static constexpr int N = 8;
+    static constexpr int BYTES = 16;
+    float x[8];
+    static __device__ __forceinline__ Chunk load(const char *p)
+    {
+        const uint4 v = __ldg(reinterpret_cast<const uint4 *>(p));
+        const unsigned w[4] = {v.x, v.y, v.z, v.w};
+        Chunk c;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const float2 f = widen_half2(w[i]);
+            c.x[2 * i] = f.x; c.x[2 * i + 1] = f.y;
+        }
+        return c;
+    }
+    __device__ __forceinline__ void store(char *p) const
+    {
+        *reinterpret_cast<uint4 *>(p) = make_uint4(narrow_half2(x[0], x[1]), narrow_half2(x[2], x[3]),
+                                                   narrow_half2(x[4], x[5]), narrow_half2(x[6], x[7]));
+    }
+};
+
+// 8-byte lane of 4 fp16 channels: the twin of bf16q
+struct halfq {};
+
+template <> struct Chunk<halfq> {
+    using elem = __half;
+    static constexpr int N = 4;
+    static constexpr int BYTES = 8;
+    float x[4];
+    static __device__ __forceinline__ Chunk load(const char *p)
+    {
+        const uint2 v = __ldg(reinterpret_cast<const uint2 *>(p));
+        const float2 lo = widen_half2(v.x), hi = widen_half2(v.y);
+        Chunk c;
+        c.x[0] = lo.x; c.x[1] = lo.y; c.x[2] = hi.x; c.x[3] = hi.y;
+        return c;
+    }
+    __device__ __forceinline__ void store(char *p) const
+    {
+        *reinterpret_cast<uint2 *>(p) = make_uint2(narrow_half2(x[0], x[1]), narrow_half2(x[2], x[3]));
+    }
+};
+
 template <typename C>
 __device__ __forceinline__ C zero_chunk()
 {
@@ -188,11 +247,12 @@ __device__ __forceinline__ float dot_chunk(const C &a, const C &b)
 // Instead lanes pair up (2j, 2j+1) over 64 bytes: instruction A writes bytes [0,32) of the pair
 // (16 each), instruction B bytes [32,64).  `RedView` holds G's channels in that arrangement
 // (swapped once per pair of lanes with four shuffles), `red_lane_offset` the matching address.
-template <typename VT> struct RedView;
+// Lanes of 4 channels (float, bf16q, halfq) and lanes of 8 (__nv_bfloat16, __half) each have one view.
+template <typename VT, int N = Chunk<VT>::N> struct RedView;
 
-template <> struct RedView<float> {
+template <typename VT> struct RedView<VT, 4> {
     float x[4];
-    static __device__ __forceinline__ RedView make(const Chunk<float> &g)
+    static __device__ __forceinline__ RedView make(const Chunk<VT> &g)
     {
         RedView r;
 #pragma unroll
@@ -206,27 +266,11 @@ template <> struct RedView<float> {
     }
 };
 
-template <> struct RedView<bf16q> {
-    float x[4];
-    static __device__ __forceinline__ RedView make(const Chunk<bf16q> &g)
-    {
-        RedView r;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) r.x[i] = g.x[i];
-        return r;
-    }
-    static __device__ __forceinline__ int lane_offset(int lane) { return lane * 16; }
-    __device__ __forceinline__ void red(char *gp, float a) const
-    {
-        red_add_v4(reinterpret_cast<float *>(gp), a * x[0], a * x[1], a * x[2], a * x[3]);
-    }
-};
-
-template <> struct RedView<__nv_bfloat16> {
+template <typename VT> struct RedView<VT, 8> {
     float x[8];  // [0,4): what instruction A writes, [4,8): instruction B
     // every lane of the warp must call this (full-mask shuffles); LANES is even, so (2j, 2j+1) never
     // straddles a query
-    static __device__ __forceinline__ RedView make(const Chunk<__nv_bfloat16> &g)
+    static __device__ __forceinline__ RedView make(const Chunk<VT> &g)
     {
         const bool odd = threadIdx.x & 1;
         RedView r;

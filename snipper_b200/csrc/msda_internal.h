@@ -8,6 +8,8 @@
 namespace msda {
 
 constexpr int kMaxLevels = 64;
+constexpr int kSnippetMaxLP = 32;   // L * P of the fused snippet kernels
+constexpr int kPlanarD = 48;        // fp32 head channels the planar slot layout is built for: 128-byte plane + 64-byte plane
 
 // Dynamic shared memory above which a launcher opts in with cudaFuncAttributeMaxDynamicSharedMemorySize: the 48 KB
 // default limit covers STATIC + dynamic shared memory, and every kernel here also holds a static level table (~1 KB).
@@ -56,8 +58,26 @@ struct FrameDims {
 
 // ---- per-call op (msda_percall.cu) ----
 // fast = vectorised fp32 path (D % 16 == 0, D <= 256); generic = any D, float or double.
-bool fast_path_ok(const OpDims &d);             // fp32
-bool fast_path_ok(const OpDims &d, int esize);  // esize = 4 (float) or 2 (bf16)
+// esize = sizeof(VT): 4 (float) or 2 (bf16 / fp16)
+inline bool fast_path_ok(const OpDims &d, int esize)
+{
+    const int epl = 16 / esize;                    // channels per 16-byte lane
+    if (d.D % epl != 0) return false;
+    const int lanes = d.D / epl;
+    if (lanes % 2 != 0 || lanes > 32) return false;
+    if (esize == 4 && lanes % 4 != 0) return false;  // fp32 instantiations: LANES in {4,8,...,32}
+    if (esize == 2 && lanes != 2 && lanes != 4 && lanes != 6 && lanes != 8 && lanes != 12 && lanes != 16) return false;
+    if (d.L > kMaxLevels) return false;
+    if ((d.value_batch_stride * esize) % 16 != 0) return false;
+    // 28-bit row stride / 31-bit cell offsets in bytes (SampleMeta)
+    if ((int64_t)d.S * d.M * d.D * esize >= ((int64_t)1 << 28)) return false;
+    // grid dimensions (y: query tiles, z: batch) and the 24-bit fast_div range
+    if (d.N > 65535 || (d.Lq + 7) / 8 > 65535) return false;
+    if ((int64_t)d.L * d.P >= 4096) return false;
+    return true;
+}
+
+inline bool fast_path_ok(const OpDims &d) { return fast_path_ok(d, 4); }
 
 // bf16 value / output / grad_output, fp32 everything else (grad_value accumulates in fp32)
 cudaError_t launch_forward_fast_bf16(const void *value, const int64_t *shapes, const int64_t *lsi,
@@ -111,8 +131,21 @@ cudaError_t launch_layer_tail(const float *y, const float *bias, const float *re
                               int cols, float eps, cudaStream_t stream);
 
 // ---- neighbour-frame pre-summation (msda_frames.cu) ----
-int snippet_num_slots(int T1, int n_frame);
-bool frame_dims_ok(const FrameDims &d, int esize);
+inline int snippet_num_slots(int T1, int n_frame) { return (T1 < n_frame ? T1 : n_frame) + (T1 > n_frame ? 1 : 0); }
+
+inline bool frame_dims_ok(const FrameDims &d, int esize)
+{
+    const int vec = 16 / esize;
+    if (d.N < 0 || d.T2 <= 0 || d.T1 <= 0 || d.n_frame <= 0 || d.n_frame > d.T2 || d.S <= 0 || d.C <= 0) return false;
+    if (d.C % vec != 0 || d.C % 4 != 0) return false;
+    if ((d.value_stride_n * esize) % 16 != 0 || (d.value_stride_t * esize) % 16 != 0) return false;
+    if (d.mask_col_stride != 0 && d.mask_col_stride != 1) return false;
+    // per-channel masks are read as 32-bit words: rows must start on a 4-byte boundary
+    if (d.mask_col_stride == 1 && d.mask_row_stride % 4 != 0) return false;
+    if ((int64_t)d.N * d.S * (d.C / 4) >= ((int64_t)1 << 40)) return false;
+    return true;
+}
+
 cudaError_t launch_frame_sum(const void *value, const uint8_t *mask, void *vsum, const FrameDims &d, int esize,
                              cudaStream_t stream);
 cudaError_t launch_frame_unsum(const float *grad_vsum, const uint8_t *mask, void *grad_value, const FrameDims &d,
@@ -120,7 +153,13 @@ cudaError_t launch_frame_unsum(const float *grad_vsum, const uint8_t *mask, void
 
 // ---- planar neighbour-frame slots (msda_planar.cu): fp32, D = 48 ----
 // bytes of one (n, slot) of the planar layout, 0 when it does not apply
-size_t planar_slot_bytes(int S, int M, int D, int esize);
+inline size_t planar_slot_bytes(int S, int M, int D, int esize)
+{
+    if (esize != 4 || D != kPlanarD || S <= 0 || M <= 0) return 0;
+    const int64_t bytes = (int64_t)M * (S * (int64_t)128 + (int64_t)((S + 3) & ~1) * 128);
+    if (bytes >= ((int64_t)1 << 31) - 256 || (int64_t)S * 16 >= ((int64_t)1 << 27)) return 0;
+    return (size_t)bytes;
+}
 cudaError_t launch_frame_sum_planar(const float *value, const uint8_t *mask, void *vsum, const FrameDims &d, int M,
                                     cudaStream_t stream);
 cudaError_t launch_frame_unsum_planar(const void *grad_vsum, const uint8_t *mask, float *grad_value, const FrameDims &d,
@@ -133,8 +172,21 @@ cudaError_t launch_planar_backward_f32(const void *vsum, const int64_t *shapes, 
                                        float *grad_offsets, float *grad_logits, const SnippetDims &d, cudaStream_t stream);
 
 // ---- fused snippet op (msda_snippet.cu) ----
-bool snippet_ok(const SnippetDims &d);             // fp32
-bool snippet_ok(const SnippetDims &d, int esize);
+inline bool snippet_ok(const SnippetDims &d, int esize)
+{
+    const int epl = 16 / esize;
+    if (d.D % epl != 0) return false;
+    const int lanes = d.D / epl;
+    if (esize == 4 && (lanes % 4 != 0 || lanes > 32)) return false;
+    if (esize == 2 && lanes != 2 && lanes != 4 && lanes != 6 && lanes != 8 && lanes != 12 && lanes != 16) return false;
+    if (d.L > kMaxLevels || d.L * d.P > kSnippetMaxLP) return false;
+    if ((d.value_stride_n * esize) % 16 != 0 || (d.value_stride_t * esize) % 16 != 0) return false;
+    if ((int64_t)d.S * d.M * d.D * esize >= ((int64_t)1 << 28)) return false;  // SampleMeta bit budget
+    if ((int64_t)d.N * d.T1 > 65535 || (d.Lq + 7) / 8 > 65535) return false;
+    return true;
+}
+
+inline bool snippet_ok(const SnippetDims &d) { return snippet_ok(d, 4); }
 cudaError_t launch_snippet_forward_bf16(const void *value, const int64_t *shapes,
                                         const int64_t *lsi, const float *offsets,
                                         const float *logits, const float *ref, void *out,

@@ -36,7 +36,6 @@ namespace msda {
 
 namespace {
 
-constexpr int kPlanarD = 48;        // fp32 head channels this layout is built for: 128-byte plane + 64-byte plane
 constexpr int kALanes = 8;          // 16-byte chunks of a cell in plane A
 constexpr int kBLanes = 4;          // 16-byte chunks of a cell in plane B
 
@@ -670,14 +669,6 @@ cudaError_t launch_bwd(const void *vsum, const int64_t *shapes, const int64_t *l
 }  // namespace
 
 // 0 when the planar layout does not apply (it is built for fp32 heads of 48 channels, 32-bit slot offsets)
-size_t planar_slot_bytes(int S, int M, int D, int esize)
-{
-    if (esize != 4 || D != kPlanarD || S <= 0 || M <= 0) return 0;
-    const int64_t bytes = (int64_t)M * (S * (int64_t)128 + (int64_t)((S + 3) & ~1) * 128);
-    if (bytes >= ((int64_t)1 << 31) - 256 || (int64_t)S * 16 >= ((int64_t)1 << 27)) return 0;
-    return (size_t)bytes;
-}
-
 cudaError_t launch_frame_sum_planar(const float *value, const uint8_t *mask, void *vsum, const FrameDims &d, int M,
                                     cudaStream_t stream)
 {

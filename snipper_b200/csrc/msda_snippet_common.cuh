@@ -8,8 +8,6 @@
 
 namespace msda {
 
-constexpr int kSnippetMaxLP = 32;
-
 struct SnipArgs {
     SnippetDims d;
     int cell_bytes;            // M * D * sizeof(VT)

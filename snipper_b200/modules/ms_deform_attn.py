@@ -233,7 +233,7 @@ class MSDeformAttn(nn.Module):
             # the biases are added inside the kernel (no GEMM epilogue pass over the projection output), and
             # the kernel reads its offsets / logits as column blocks of the one output.  The padding mask
             # (:116-117) is applied inside the kernels as well -- value is never re-written.
-            # value may be bf16 (autocast): the kernels gather bf16 and keep every location / weight
+            # value may be bf16 or fp16 (autocast): the kernels gather 16-bit values and keep every location / weight
             # computation in fp32, so the projection and the reference points go in as fp32.
             weight, off_bias, logit_bias = self._stacked_projection()
             proj = F.linear(query, weight)
@@ -296,13 +296,13 @@ class MSDeformAttn(nn.Module):
             q = query[:, t1]
             logits = torch.stack([self.attention_weights[t2](q).view(N, Lq, M, L, P) for t2 in frames], -1)
             att = F.softmax(logits.flatten(-3), -1).view(N, Lq, M, L, P, len(frames))
-            if value.dtype == torch.bfloat16:
+            if value.dtype in (torch.bfloat16, torch.float16):
                 att = att.float()
             acc, locs = None, []
             for j, t2 in enumerate(frames):
                 off = self.sampling_offsets[t2](q).view(N, Lq, M, L, P, 2)
                 loc = reference_points[:, t1, :, None, :, None, :] + off / wh[None, None, None, :, None, :]
-                if value.dtype == torch.bfloat16:
+                if value.dtype in (torch.bfloat16, torch.float16):
                     loc = loc.float()
                 if self.attention_vis:
                     locs.append(loc.detach())

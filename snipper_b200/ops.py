@@ -18,6 +18,9 @@ in the hand-written kernels.  Ops (namespace ``snipper_b200``):
   layer_tail_amp_train / _backward      the same on a bf16 GEMM output, also writing the next GEMMs' bf16 inputs, for
                                         training under bf16 autocast (libmsda_b200_amp_train.so)
 
+msda_forward / msda_backward, the snippet ops and the frame passes also take float16 value / output / grad_output: those
+calls go to libmsda_b200_f16.so, the same kernels with fp16 storage, under the rules of the bfloat16 mode.
+
 The five forwards (msda_forward, snippet_forward, snippet_attn, layer_tail_train, layer_tail_amp_train) carry
 ``register_autograd`` formulas, so they compose with autograd / DDP as plain nodes (no host sync, no unused parameters).
 """
@@ -31,6 +34,14 @@ from . import capi
 
 _DTYPES = {torch.float32: capi.MSDA_DTYPE_F32, torch.float64: capi.MSDA_DTYPE_F64,
            torch.bfloat16: capi.MSDA_DTYPE_BF16}
+# 16-bit storage: value / output / grad_output in the dtype, everything else float32.  float16 runs in
+# libmsda_b200_f16.so, whose entry points take no dtype argument.
+_HALF = (torch.bfloat16, torch.float16)
+
+
+def _dt(dtype):
+    """The dtype argument of a C entry point: none for float16 (libmsda_b200_f16.so)"""
+    return () if dtype == torch.float16 else (_DTYPES[dtype],)
 
 # process-wide switch for the deterministic (atomics-free) grad_value path
 _deterministic = False
@@ -83,13 +94,16 @@ STATS = LaunchStats()
 
 
 def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None, im2col_step=None, amp=False,
-            train=False):
+            train=False, f16=False):
     """Call the C entry point ``entry`` (of libmsda_b200_amp.so when ``amp``, of libmsda_b200_train.so when ``train``,
-    of libmsda_b200_amp_train.so when both) with ``args`` and ``device``'s current stream (every launching entry point
-    takes the stream last), count its ``n_kernels`` kernels in STATS under ``tag`` / ``dims`` and raise on a failed
-    status."""
-    lib = (capi.amp_train_lib() if amp and train else capi.amp_lib() if amp else capi.train_lib() if train
-           else capi.lib())
+    of libmsda_b200_amp_train.so when both; when ``f16``, its ``msda_f16_*`` twin of libmsda_b200_f16.so) with ``args``
+    and ``device``'s current stream (every launching entry point takes the stream last), count its ``n_kernels`` kernels
+    in STATS under ``tag`` / ``dims`` and raise on a failed status."""
+    if f16:
+        lib, entry = capi.f16_lib(), "msda_f16_" + entry[len("msda_"):]
+    else:
+        lib = (capi.amp_train_lib() if amp and train else capi.amp_lib() if amp else capi.train_lib() if train
+               else capi.lib())
     with torch.cuda.device(device):
         stream = torch.cuda.current_stream(device)
         if STATS.timing:
@@ -100,8 +114,8 @@ def _launch(entry, tag, dims, device, *args, n_kernels=1, what=None, batch=None,
         if STATS.timing:
             end.record(stream)
             STATS.events.append((tag, dims, start, end))
-    last_error = (lib.msda_amp_train_last_cuda_error if amp and train else lib.msda_amp_last_cuda_error if amp
-                  else lib.msda_train_last_cuda_error if train else None)
+    last_error = (lib.msda_f16_last_cuda_error if f16 else lib.msda_amp_train_last_cuda_error if amp and train
+                  else lib.msda_amp_last_cuda_error if amp else lib.msda_train_last_cuda_error if train else None)
     capi.check(status, what or entry, batch, im2col_step, last_error)
 
 
@@ -143,14 +157,14 @@ def _check_percall(value, spatial_shapes, level_start_index, sampling_loc, attn_
         _require_contiguous(t, name)
     if value.dim() != 4 or sampling_loc.dim() != 6 or attn_weight.dim() != 5:
         raise RuntimeError("expected value (N,S,M,D), sampling_loc (N,Lq,M,L,P,2), attn_weight (N,Lq,M,L,P)")
-    if value.dtype not in _DTYPES:
-        raise RuntimeError("ms_deform_attn: unsupported dtype %s (float32 / float64 / bfloat16)" % value.dtype)
-    if value.dtype == torch.bfloat16:
-        # bf16 mode: value / output / grad_output are bf16; locations and weights are computed in fp32
+    if value.dtype not in _DTYPES and value.dtype != torch.float16:
+        raise RuntimeError("ms_deform_attn: unsupported dtype %s (float32 / float64 / bfloat16 / float16)" % value.dtype)
+    if value.dtype in _HALF:
+        # bf16 / fp16 mode: value / output / grad_output are 16-bit; locations and weights are computed in fp32
         if sampling_loc.dtype != torch.float32 or attn_weight.dtype != torch.float32:
-            raise RuntimeError("bfloat16 value needs float32 sampling_loc and attn_weight")
+            raise RuntimeError("%s value needs float32 sampling_loc and attn_weight" % str(value.dtype)[6:])
         if value.shape[3] % 16 != 0 or value.shape[3] > 128:
-            raise RuntimeError("bfloat16 ms_deform_attn needs head channels D % 16 == 0 and D <= 128")
+            raise RuntimeError("%s ms_deform_attn needs head channels D %% 16 == 0 and D <= 128" % str(value.dtype)[6:])
     elif sampling_loc.dtype != value.dtype or attn_weight.dtype != value.dtype:
         raise RuntimeError("value, sampling_loc and attn_weight must share one dtype")
     if spatial_shapes.dtype != torch.int64 or level_start_index.dtype != torch.int64:
@@ -173,8 +187,8 @@ def msda_forward(value: Tensor, spatial_shapes: Tensor, level_start_index: Tenso
     _launch("msda_forward", "msda_forward", (N, S, M, D, L, Lq, P), value.device,
             value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
             sampling_loc.data_ptr(), attn_weight.data_ptr(), out.data_ptr(),
-            N, S, M, D, L, Lq, P, vbs, int(im2col_step), _DTYPES[value.dtype],
-            what="ms_deform_attn_forward", batch=N, im2col_step=im2col_step)
+            N, S, M, D, L, Lq, P, vbs, int(im2col_step), *_dt(value.dtype),
+            what="ms_deform_attn_forward", batch=N, im2col_step=im2col_step, f16=value.dtype == torch.float16)
     return out
 
 
@@ -194,18 +208,17 @@ def msda_backward(value: Tensor, spatial_shapes: Tensor, level_start_index: Tens
     if grad_output.dtype != value.dtype or grad_output.numel() != N * Lq * M * D:
         raise RuntimeError("grad_output must be (N,Lq,M*D) in value's dtype")
     vbs = _value_batch_stride(value)
-    bf16 = value.dtype == torch.bfloat16
-    if bf16 and deterministic:
+    half, f16 = value.dtype in _HALF, value.dtype == torch.float16
+    if half and deterministic:
         raise RuntimeError("the deterministic backward is float32 only")
-    # bf16 mode accumulates grad_value in fp32 (include/msda_b200.h) and rounds once at the end
-    grad_value = torch.empty((N, S, M, D), dtype=torch.float32 if bf16 else value.dtype, device=value.device)
+    # bf16 / fp16 modes accumulate grad_value in fp32 (include/msda_b200.h) and round once at the end
+    grad_value = torch.empty((N, S, M, D), dtype=torch.float32 if half else value.dtype, device=value.device)
     grad_loc = torch.empty_like(sampling_loc)
     grad_attn = torch.empty_like(attn_weight)
     flags = capi.MSDA_FLAG_DETERMINISTIC if deterministic else 0
-    dt = _DTYPES[value.dtype]
     ws, ws_ptr, ws_bytes = None, 0, 0
     if deterministic:
-        ws_bytes = capi.lib().msda_backward_workspace_bytes(N, S, M, D, L, Lq, P, dt, flags)
+        ws_bytes = capi.lib().msda_backward_workspace_bytes(N, S, M, D, L, Lq, P, _DTYPES[value.dtype], flags)
         ws, ws_ptr = _workspace(ws_bytes, value.device)
     # deterministic: no-scatter kernel, memset, count, 3 scan kernels, fill, reduce, long-list reduce
     _launch("msda_backward", "msda_backward_deterministic" if deterministic else "msda_backward",
@@ -213,10 +226,11 @@ def msda_backward(value: Tensor, spatial_shapes: Tensor, level_start_index: Tens
             value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(),
             sampling_loc.data_ptr(), attn_weight.data_ptr(), grad_output.data_ptr(),
             grad_value.data_ptr(), grad_loc.data_ptr(), grad_attn.data_ptr(),
-            N, S, M, D, L, Lq, P, vbs, int(im2col_step), dt, flags, ws_ptr, ws_bytes,
-            n_kernels=9 if deterministic else 2, what="ms_deform_attn_backward", batch=N, im2col_step=im2col_step)
-    if bf16:
-        grad_value = grad_value.to(torch.bfloat16)
+            N, S, M, D, L, Lq, P, vbs, int(im2col_step), *_dt(value.dtype), flags,
+            *(() if f16 else (ws_ptr, ws_bytes)), n_kernels=9 if deterministic else 2, what="ms_deform_attn_backward",
+            batch=N, im2col_step=im2col_step, f16=f16)
+    if half:
+        grad_value = grad_value.to(value.dtype)
     return grad_value, grad_loc, grad_attn
 
 
@@ -272,8 +286,8 @@ def snippet_supported(n_heads: int, d_head: int, n_levels: int, n_points: int, d
     """Shapes the fused kernels cover -- every constraint the C ABI enforces for the packed call
     (include/msda_b200.h msda_snippet_forward; msda_snippet.cu snippet_ok), so that a caller can fall back
     to the per-call loop instead of getting MSDA_ERR_INVALID_ARGUMENT."""
-    esize = 2 if dtype == torch.bfloat16 else 4
-    return (dtype in (torch.float32, torch.bfloat16) and d_head % 16 == 0 and d_head <= 128 and
+    esize = 2 if dtype in _HALF else 4
+    return (dtype in (torch.float32, torch.bfloat16, torch.float16) and d_head % 16 == 0 and d_head <= 128 and
             n_levels * n_points <= 32 and n_levels <= 64 and
             (n_heads * n_levels * n_points) % 2 == 0 and                     # float2 loads of a packed projection row
             spatial_size * n_heads * d_head * esize < (1 << 28) and          # cell byte offsets are 28-bit
@@ -327,7 +341,7 @@ def _check_fused(value, spatial_shapes, level_start_index, reference_points, n_f
                 or not valid_ratios.is_contiguous() or Lq != S):
             raise RuntimeError("valid_ratios must be contiguous float32 (N,L,2) and the queries the S pixels of the pyramid")
     if not snippet_supported(M, D, L, P, value.dtype, S, N * T1):
-        raise RuntimeError("fused snippet attention needs float32 / bfloat16 value, D % 16 == 0, D <= 128, L*P <= 32")
+        raise RuntimeError("fused snippet attention needs float32 / bfloat16 / float16 value, D % 16 == 0, D <= 128, L*P <= 32")
     if any(t.dtype != torch.float32 for _, t in rows):
         raise RuntimeError("offsets and logits (or proj) must be float32")
     for b, n in zip(biases, (2 * M * L * P, M * L * P)):
@@ -380,7 +394,7 @@ def _issue_snippet_forward(tag, dims, n_frame, value, spatial_shapes, level_star
             value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(), offsets[0], logits[0], _ptr(ref),
             out.data_ptr(), N, T2, T1, int(n_frame), S, M, D, L, Lq, P, *value_strides, rsn, rst, offsets[1], logits[1],
             _ptr(biases[0]), _ptr(biases[1]), _ptr(valid_ratios), _ptr(mask[0]), mask[1], mask[2],
-            _DTYPES[value.dtype], flags)
+            *_dt(value.dtype), flags, f16=value.dtype == torch.float16)
 
 
 def _issue_snippet_backward(tag, n_kernels, dims, n_frame, value, spatial_shapes, level_start_index, grad_output,
@@ -388,15 +402,16 @@ def _issue_snippet_backward(tag, n_kernels, dims, n_frame, value, spatial_shapes
                             reference_points=None, valid_ratios=None, biases=(None, None), mask=(None, 0, 0), flags=0,
                             workspace=(None, 0)):
     """``grad_offsets`` / ``grad_logits`` are pointers with the row strides of ``offsets`` / ``logits``; ``workspace``
-    is (pointer, bytes)."""
+    is (pointer, bytes) and not passed for float16 (no deterministic mode there)."""
     N, T2, T1, S, M, D, L, Lq, P = dims
+    f16 = value.dtype == torch.float16
     ref, rsn, rst = _ref_strides(reference_points) if reference_points is not None else (None, 0, 0)
     _launch("msda_snippet_backward", tag, dims, value.device,
             value.data_ptr(), spatial_shapes.data_ptr(), level_start_index.data_ptr(), offsets[0], logits[0], _ptr(ref),
             grad_output.data_ptr(), grad_value.data_ptr(), grad_offsets, grad_logits,
             N, T2, T1, int(n_frame), S, M, D, L, Lq, P, *value_strides, rsn, rst, offsets[1], logits[1],
             _ptr(biases[0]), _ptr(biases[1]), _ptr(valid_ratios), _ptr(mask[0]), mask[1], mask[2],
-            _DTYPES[value.dtype], flags, *workspace, n_kernels=n_kernels)
+            *_dt(value.dtype), flags, *(() if f16 else workspace), n_kernels=n_kernels, f16=f16)
 
 
 def _grad_ref(grad_offsets, spatial_shapes):
@@ -527,7 +542,7 @@ def _frame_sum(value, mask, T1, n_frame, planar):
         vsum = torch.empty((N, slots, S, M, D), dtype=value.dtype, device=value.device)
         entry, tag, row = "msda_frame_sum", "frame_sum", (S, M * D)
     _launch(entry, tag, (N, T2, T1, S, M * D), value.device, value.data_ptr(), _ptr(mask[0]), vsum.data_ptr(),
-            N, T2, T1, int(n_frame), *row, sn, st, mask[1], mask[2], _DTYPES[value.dtype])
+            N, T2, T1, int(n_frame), *row, sn, st, mask[1], mask[2], *_dt(value.dtype), f16=value.dtype == torch.float16)
     return vsum
 
 
@@ -540,7 +555,7 @@ def _frame_unsum(grad_slots, mask, dims, n_frame, dtype, planar):
     else:
         entry, tag, row = "msda_frame_unsum", "frame_unsum", (S, M * D)
     _launch(entry, tag, (N, T2, T1, S, M * D), grad_slots.device, grad_slots.data_ptr(), _ptr(mask[0]),
-            grad_value.data_ptr(), N, T2, T1, int(n_frame), *row, mask[1], mask[2], _DTYPES[dtype])
+            grad_value.data_ptr(), N, T2, T1, int(n_frame), *row, mask[1], mask[2], *_dt(dtype), f16=dtype == torch.float16)
     return grad_value
 
 
